@@ -2,6 +2,7 @@
 """bench.py — PPO env-steps/s on B200 (BASELINE.json metric), with roofline, CPU baseline and clocks.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload auto|c1|c2|c3|c5]
+                    [--dump-outputs DIR]
 
 A "step" is one PPO iteration of the hot path: a rollout of `horizon` vector steps over the env batch, the batched GAE,
 and n_epoch x n_minibatch fused updates.  Observation / reward normalisation is ON (the reference yaml default,
@@ -28,6 +29,8 @@ Printed keys (one JSON line, rank 0):
 `--impl reference` times the reference's own CPU implementation: the unmodified `PPOCLIP_Agent.train` of the copy
 pip-installed into oracle/_ref (oracle/build_ref.py; kind "reference"), else its restatement oracle/ref_port.py (kind
 "port"), on a fixed 1024-env sample of the same config with a fixed thread policy.
+`--dump-outputs DIR` writes what the headline's last timed step computed (see dump_outputs); every input is seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -531,6 +534,38 @@ def measure(wl, world, steps, warmup, flush, shuffle, sync_info, norm=True):
     return agent, agent.n_envs * agent.n_steps * steps * world / secs, secs / steps * 1e3
 
 
+DUMP_BYTES = 64 << 20          # --dump-outputs writes at most this much
+
+
+def dump_outputs(agent, out_dir):
+    """--dump-outputs: what the timed path's last PPO iteration computed, one DIR/<name>.npy each (float32 or float64): the
+    log scalars train() returned, the policy parameters and running statistics it left, and the rollout it trained on
+    (time-major [T, envs, ...]).  Rollouts larger than the budget keep a fixed, seeded sample of the envs.  With --gpus N > 1
+    only rank 0 dumps, so the rollout is rank 0's env shard (envs_per_gpu of the config, not envs_total).  Run to run,
+    everything is bit-identical except info_mean_episode_score (its fp64 episode totals are summed by atomics)."""
+    mem = agent.memory
+    out = {"info_" + k.replace("-", "_"): np.float64(v) for k, v in agent.last_info.items()}
+    out.update({"param_" + k: v.detach().float().cpu().numpy() for k, v in agent.policy.state_dict().items()})
+    out["obs_rms"] = agent._obs_rms[agent._rms_cur].cpu().numpy()        # fp64 mean[D], var[D], count
+    out["ret_rms"] = agent._ret_rms.cpu().numpy()                       # fp64 mean, var, count
+    rollout = {"obs": mem._obs[..., :mem.obs_dim], "act": mem._act, "rew": mem._rew, "val": mem._val, "term": mem._term,
+               "logp": mem._logp, "adv": mem._adv, "ret": mem._ret}
+    fixed = sum(a.nbytes for a in out.values())
+    per_env = sum(t[:, 0].numel() * 4 for t in rollout.values())
+    keep = min(mem.n_envs, (DUMP_BYTES - fixed) // per_env)
+    envs = None
+    if keep < mem.n_envs:
+        envs = np.sort(np.random.default_rng(0).choice(mem.n_envs, keep, replace=False))
+        envs = torch.as_tensor(envs, device=mem._rew.device)
+    for k, t in rollout.items():
+        out[k] = (t if envs is None else t.index_select(1, envs)).float().cpu().numpy()
+    assert sum(a.nbytes for a in out.values()) <= DUMP_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    return sorted(out)
+
+
 def value_and_e2e(wl, world, steps, warmup, flush, norm=True, with_e2e=True):
     """{"value", "ms_per_step", "e2e": {...}} for a secondary workload (no kernel table)."""
     agent, value, ms = measure(wl, world, steps, warmup, flush, "device", False, norm)
@@ -654,6 +689,7 @@ def run_ours(args):
 
     # value: device-resident (permutations drawn on the GPU, one host sync at the end of train())
     agent, value, ms_step = measure(wl, world, args.steps, args.warmup, flush, "device", False, True)
+    dumped = dump_outputs(agent, args.dump_outputs) if (args.dump_outputs and rank == 0) else None
     launches = count_launches(agent)
     phases = time_phases(agent, flush) if world == 1 else None
     launches_per_step = {"updates": agent.n_epoch * agent.n_updates_per_epoch}
@@ -727,6 +763,8 @@ def run_ours(args):
     }
     if parity is not None:
         line["rank_parity"] = parity
+    if dumped is not None:
+        line["dumped_outputs"] = dumped
     line.update(side)
     print(json.dumps(line))
 
@@ -811,9 +849,7 @@ def run_reference(args):
     wl = WORKLOADS[key]
     n = min(REF_SAMPLE_ENVS, wl["envs"])
     threads = cpu_threads(n)
-    steps = max(3, args.steps)
-    # bound the run: ~2-7 s per step on 16-32 host cores; more than 12 timed steps add nothing but minutes
-    steps = min(steps, 12)
+    steps = args.steps          # ~2-7 s per step on 16-32 host cores
     res = time_reference_cpu(wl, n, threads, warmup=max(1, min(args.warmup, 2)), steps=steps)
     print(json.dumps({
         "impl": "reference", "metric": "PPO env-steps/s", "value": res["value"], "unit": "env-steps/s",
@@ -836,7 +872,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--headline-only", action="store_true", help="only the headline workload (no norm_off / c1 / c3 / weak_c2 / c5 / c4 keys)")
     ap.add_argument("--tf32", action="store_true", help="allow TF32 tensor-core GEMMs in the torch MLP (not the headline)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the headline's last timed step computed to DIR/<name>.npy "
+                    "(rank 0 only: with --gpus N > 1 the rollout is rank 0's env shard); bench_outputs/ is git-ignored")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the native arm (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -1,5 +1,16 @@
 """bench.roofline_of: the `roofline` object of the JSON line names the roof that bounds the dominant kernel (CPU only)."""
+import pytest
+
 import bench
+
+# The kernel fractions below were taken against this TF32 ceiling (1/2 x the measured bf16 burst of a B200, DESIGN.md);
+# pinned so the test does not depend on which peaks file, if any, the machine running it has.
+TF32_PEAK = 832.0
+
+
+@pytest.fixture(autouse=True)
+def _pinned_tf32_peak(monkeypatch):
+    monkeypatch.setattr(bench, "measured_tf32_peak", lambda: TF32_PEAK)
 
 
 def _kd(**kw):

@@ -1,5 +1,6 @@
-"""CPU, build container only (needs the reference SOURCE tree at /root/reference; skipped elsewhere): the oracle's
-restatements run side by side with the LIVE reference objects on fresh seeded inputs — not via stored goldens.
+"""CPU, wherever the reference is importable (installed into oracle/_ref by `python -m oracle.build_ref`, or a source tree
+named by XB200_REFERENCE_ROOT; skipped elsewhere): the oracle's restatements run side by side with the LIVE reference
+objects on fresh seeded inputs — not via stored goldens.
 
     RunningMeanStdPort   vs  xuance.common.RunningMeanStd                     statistic_tools.py:35-112
     PPOAgentPort.train   vs  PPOCLIP_Agent.train (built by xuance.get_runner)  ppoclip_agent.py:59-111
@@ -12,7 +13,7 @@ import torch
 from oracle import ref_loader, ref_port
 
 pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not ref_loader.source_tree_available(), reason="reference source tree not present")]
+              pytest.mark.skipif(not ref_loader.available(), reason="the reference is not importable (python -m oracle.build_ref)")]
 
 
 def test_running_mean_std_port_equals_live_reference_bit_for_bit():
