@@ -252,8 +252,10 @@ int xb_clip_adam_step(float* param, const float* grad, float* exp_avg, float* ex
  * Agent._process_observation/_process_reward (xuance/torch/agents/agent.py:104-123) and the per-env discounted
  * return tracker (ppoclip_agent.py:87,91-92).
  *   obs normaliser state: fp64 [9] = mean[4], var[4], count (mean/var hold float32-rounded values)
- *   xb_moments4      sums fp64 [9] = column sums (4), column sums of squares (4), N of x f32 [N][4]
- *                    (between the two calls the 9 sums may be all-reduced across ranks: the analogue of mpi_mean :6-17)
+ *   xb_moments4      sums fp64 [2D + 1] = column sums (D), column sums of squares (D), N of x f32 [N][D], D = row_floats
+ *                    (4, or 8 for wide rows: the first observations of an env-sharded agent, `obs_rms.update(obs)` of
+ *                    ppoclip_agent.py:62 with the sums exchanged across ranks in between: the analogue of mpi_mean :6-17);
+ *                    xb_rms_normalize takes the 4-float form
  *   xb_rms_normalize merges `sums` into state_in (Chan), writes the merged state to state_out (!= state_in) and
  *                    out = clip((x - mean) / (sqrt(var) + 1e-8), +-clip)     f32 [N][4]; lanes >= dim give 0.
  *                    Rows [0, n_merged_rows) use the merged statistics, rows beyond use state_in unchanged (the
@@ -266,7 +268,7 @@ int xb_clip_adam_step(float* param, const float* grad, float* exp_avg, float* ex
  *                    publishes rew_std = clip(sqrt(var), 0.1, 100), the divisor xb_store applies to rewards
  * workspace: fp64 [8 + 8*1184], word 0 ZERO-INITIALISED once by the caller (one workspace per call site).
  * ---------------------------------------------------------------------------------------------------------- */
-int xb_moments4(const float* x, double* sums, double* workspace, int64_t N, xb_stream_t stream);
+int xb_moments4(const float* x, int row_floats, double* sums, double* workspace, int64_t N, xb_stream_t stream);
 int xb_rms_normalize(const float* x, int dim, const double* sums, const double* state_in, double* state_out,
                      float clip, float* out, int64_t N, int64_t n_merged_rows, xb_stream_t stream);
 int xb_returns_track(double* returns, const float* rew, const uint8_t* term, const uint8_t* trunc, double gamma, int mask_terminal,
@@ -282,10 +284,11 @@ int xb_rms_apply(const float* x, int row_floats, int dim, const double* state_ne
                  float clip, float* out, int64_t N, xb_stream_t stream);
 int xb_rms_update_rows(const float* x, int row_floats, int dim, int64_t N, const double* state_in, double* state_out,
                        double* partials, uint32_t* ticket, xb_stream_t stream);
-/*   xb_rms_merge_sums   env-sharded form: sums fp64 [12] = the cross-rank totals of one step (layout of xb_moments4 + the three
- *                       return sums); obs_state_out = obs_state_in merged with them (nullable pair, 4-float rows), ret_state
- *                       merged in place and rew_std republished (nullable pair). */
-int xb_rms_merge_sums(const double* sums, const double* obs_state_in, double* obs_state_out, int dim, double* ret_state,
+/*   xb_rms_merge_sums   env-sharded form (mpi_moments + update_from_moments, statistic_tools.py:6-32,101-112): sums fp64 [n]
+ *                       = the cross-rank totals of one step, n = 2D + 4 = 12 or 20 for D = 4 or 8 floats per row (layout of
+ *                       xb_moments4 + the three return sums); obs_state_out = obs_state_in merged with them (nullable pair,
+ *                       state fp64 [2D + 1], dim <= D), ret_state merged in place and rew_std republished (nullable pair). */
+int xb_rms_merge_sums(const double* sums, int n, const double* obs_state_in, double* obs_state_out, int dim, double* ret_state,
                       float* rew_std, xb_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------------------
@@ -339,7 +342,7 @@ int xb_bias_act_fwd(float* y, const float* bias, float slope, int64_t B, int H, 
  *     last CTA (deterministic);
  *   stat_sums_out (nullable, fp64 [2D + 4], env-sharded form): this rank's totals (sum x[D], sum x^2[D], N, sum R, sum R^2,
  *     n finished) are written there INSTEAD of being merged (obs_state_out / ret_state unused); exchange them across ranks
- *     (xb_peer_allreduce_f64) and merge with xb_rms_merge_sums.
+ *     (xb_peer_allreduce_merge, or xb_peer_allreduce_f64 and xb_rms_merge_sums).
  * ---------------------------------------------------------------------------------------------------------- */
 int xb_rollout_step(int env_kind, const float* act_param, const float* logstd, const float* val, uint64_t seed,
                     const uint64_t* counter_dev, uint64_t offset, double* state, uint64_t* rng, int32_t* elapsed,
@@ -546,6 +549,11 @@ int xb_head3_unfold_grads(float* gw3, float* gb3, int H, xb_stream_t stream);
  *   rank) read from local memory; squared norm of grad_out * grad_scale; then exactly the scalars xb_clip_adam_step's
  *   first kernel derives (workspace layout identical), so xb_adam_apply can follow.  n must be a multiple of 4.
  * xb_adam_apply: the second kernel of xb_clip_adam_step alone (clip + Adam from the scalars in workspace).
+ * xb_peer_allreduce_mean: the push / barrier / rank-order sum of xb_peer_allreduce_grad_norm without the optimiser scalars:
+ *   grad_out = (sum_r grad_in_r) * (1 / W), written to local memory, bit-identical on every rank (W = 1: grad_out = grad_in bit
+ *   for bit).  The sharded form of the gradient a torch optimiser steps on (ppg_learner.py:44-46,59-63,80-84 `loss.backward();
+ *   optimizer.step()` over a minibatch split across ranks).  Shares the inbox, the per-CTA tickets and the grid of
+ *   xb_peer_allreduce_grad_norm: every launch on one comm block must pass the same n (a multiple of 4).
  * xb_peer_allreduce_f64: out[j] = sum_r stats_r[offset + j], j < n, offset + n <= xb_peer_stats_max().  Used once per epoch for
  *   the minibatch advantage statistics and, with use_obsnorm / use_rewnorm, once per vector step for the observation /
  *   return moments (the analogue of mpi_moments, xuance/common/statistic_tools.py:6-32).
@@ -574,14 +582,17 @@ int xb_adam_apply_split(float* param, const float* grad, float* exp_avg, float* 
                         float beta2, float eps, float grad_scale, const double* workspace, int64_t w_off0, float* hi0,
                         float* lo0, int64_t w_off1, float* hi1, float* lo1, int N, int K, float* thi, float* tlo,
                         xb_stream_t stream);
+int xb_peer_allreduce_mean(const void* const* peer_bases /* host [W] */, int rank, int W, int64_t n, const float* grad_in,
+                           float* grad_out, uint32_t* tickets, xb_stream_t stream);
 int xb_peer_allreduce_f64(const void* const* peer_bases /* host [W] */, int rank, int W, int offset, int n, double* out,
                           uint32_t* tickets, xb_stream_t stream);
 /*   xb_peer_allreduce_merge   the per-vector-step statistics exchange of the env-sharded normalisers as ONE kernel with ONE
- *                             cross-GPU barrier + the merge of xb_rms_merge_sums: every rank pushes src[0..n) (n <= 16) into a
- *                             parity double-buffered inbox at doubles [inbox_offset, inbox_offset + 256) of every peer's
+ *                             cross-GPU barrier + the merge of xb_rms_merge_sums: every rank pushes src[0..n) (n <= 20) into a
+ *                             parity double-buffered inbox at doubles [inbox_offset, inbox_offset + 320) of every peer's
  *                             statistics area, out[0..n) = the totals (rank order, bit-identical on every rank); with
- *                             obs_state_in / ret_state (n = 12: sum x[4], sum x^2[4], N, sum R, sum R^2, n finished) the
- *                             normaliser states are merged in the same launch (mpi_moments, statistic_tools.py:6-32). */
+ *                             obs_state_in / ret_state (n = 2D + 4 = 12 or 20: sum x[D], sum x^2[D], N, sum R, sum R^2,
+ *                             n finished, for D = 4 or 8 floats per observation row, dim <= D) the normaliser states are
+ *                             merged in the same launch (mpi_moments, statistic_tools.py:6-32). */
 int xb_peer_allreduce_merge(const void* const* peer_bases, int rank, int W, const double* src, int n, int inbox_offset,
                             double* out, uint32_t* tickets, const double* obs_state_in, double* obs_state_out, int dim,
                             double* ret_state, float* rew_std, xb_stream_t stream);

@@ -46,13 +46,13 @@ SIGNATURES = {
     "xb_host_permutation": [_vp, _i64, _u64],
     "xb_host_permutation32": [_vp, _i64, _u64],
     "xb_random_permutation": [_vp, _i64, _u64, _vp, _u64, _vp],
-    "xb_moments4": [_vp, _vp, _vp, _i64, _vp],
+    "xb_moments4": [_vp, _i32, _vp, _vp, _i64, _vp],
     "xb_rms_normalize": [_vp, _i32, _vp, _vp, _vp, _f32, _vp, _i64, _i64, _vp],
     "xb_returns_track": [_vp, _vp, _vp, _vp, _f64, _i32, _vp, _vp, _i64, _vp],
     "xb_rms_merge_scalar": [_vp, _vp, _vp, _vp],
     "xb_rms_apply": [_vp, _i32, _i32, _vp, _vp, _i64, _f32, _vp, _i64, _vp],
     "xb_rms_update_rows": [_vp, _i32, _i32, _i64, _vp, _vp, _vp, _vp, _vp],
-    "xb_rms_merge_sums": [_vp, _vp, _vp, _i32, _vp, _vp, _vp],
+    "xb_rms_merge_sums": [_vp, _i32, _vp, _vp, _i32, _vp, _vp, _vp],
     "xb_head_fwd": [_vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp],
     "xb_head_bwd_act": [_vp, _vp, _vp, _f32, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _vp],
     "xb_bias_act_fwd": [_vp, _vp, _f32, _i64, _i32, _vp],
@@ -100,6 +100,7 @@ SIGNATURES = {
     "xb_adam_apply": [_vp, _vp, _vp, _vp, _i64, _f32, _f32, _f32, _f32, _vp, _vp],
     "xb_adam_apply_split": [_vp, _vp, _vp, _vp, _i64, _f32, _f32, _f32, _f32, _vp, _i64, _vp, _vp, _i64, _vp, _vp, _i32, _i32,
                             _vp, _vp, _vp],
+    "xb_peer_allreduce_mean": [_vp, _i32, _i32, _i64, _vp, _vp, _vp, _vp],
     "xb_peer_allreduce_f64": [_vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp],
     "xb_peer_allreduce_merge": [_vp, _i32, _i32, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp],
     "xb_adv_stats_minibatches": [_vp, _i64, _i64, _i64, _i64, _vp, _i64, _vp, _vp],

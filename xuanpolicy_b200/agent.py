@@ -112,12 +112,12 @@ class PPOCLIP_Agent:
         self.learner = self._make_learner(config, policy, optimizer, scheduler)
         if self._graph_updates:
             self.learner.enable_fused_optimizer(process_group)
-        elif process_group is not None or (torch.distributed.is_available() and torch.distributed.is_initialized()
-                                           and torch.distributed.get_world_size() > 1):
-            raise NotImplementedError("%s trains on one GPU (its update phases are not env-sharded)" % type(self).__name__)
+        else:                 # eager update phases: the learner exchanges the gradients its torch optimiser steps on
+            self.learner.enable_sharding(process_group)
         self.world_size = self.learner.world_size
-        if self.world_size > 1 and self._graph_updates:   # replicated policy: every rank starts from rank 0's parameters
-            xdist.broadcast_parameters(self.learner._flat.flat_param, 0, process_group)
+        if self.world_size > 1:
+            if self._graph_updates:       # replicated policy: every rank starts from rank 0's parameters
+                xdist.broadcast_parameters(self.learner._flat.flat_param, 0, process_group)
             if self.buffer_size % self.batch_size:
                 raise ValueError("env-sharded training needs n_envs * n_steps (%d) divisible by n_minibatch (%d): the ranks' "
                                  "minibatches must be equal for the global-minibatch statistics" % (self.buffer_size, self.n_minibatch))
@@ -164,6 +164,7 @@ class PPOCLIP_Agent:
         init = torch.tensor([0.0] * D + [1.0] * D + [1e-4], **f64)
         self._obs_rms = [init.clone(), init.clone()]
         self._rms_cur = 0
+        self._norm_n = 2 * D + 4          # one step's sums: sum x[D], sum x^2[D], N, sum R, sum R^2, n finished
         self._obs_sums = torch.zeros(9, **f64)
         self._obs_ws = torch.zeros(8 + 8 * 1184, **f64)
         self._xn = torch.zeros((2 * N, D), dtype=torch.float32, device=dev)      # normalised policy input
@@ -172,7 +173,7 @@ class PPOCLIP_Agent:
         self._ret_ws = torch.zeros(8 + 8 * 1184, **f64)
         self._returns = torch.zeros(N, dtype=torch.float64, device=dev)
         self._rew_std = torch.ones(1, dtype=torch.float32, device=dev)
-        # env-sharded normalisers: the per-step observation moments [9] and finished-episode return sums [3] are exchanged
+        # env-sharded normalisers: the per-step observation moments [2D + 1] and finished-episode return sums [3] are exchanged
         # over peer memory (the analogue of mpi_moments, statistic_tools.py:6-32) so every rank keeps the GLOBAL statistics;
         # they live at the end of the comm block's statistics region (its start carries the per-epoch advantage sums)
         self._norm_peer = self.learner._peer if (self.use_obsnorm or self.use_rewnorm) else None
@@ -180,10 +181,10 @@ class PPOCLIP_Agent:
             raise NotImplementedError("use_obsnorm / use_rewnorm with env sharding need the peer-memory exchange "
                                       "(XB_PEER_COMM=1 and CUDA IPC available)")
         if self._norm_peer is not None:
-            self._norm_off = self._norm_peer.stats.numel() - 12
+            self._norm_off = self._norm_peer.stats.numel() - self._norm_n
             self._norm_local = self._norm_peer.stats[self._norm_off:]
             self._norm_local.zero_()
-            self._norm_global = torch.zeros(12, **f64)
+            self._norm_global = torch.zeros(self._norm_n, **f64)
         # one launch per vector step (sample + env step + store) for the two classic-control action shapes
         import os as _os
         self._fused_step = (_os.environ.get("XB_FUSED_STEP", "1") != "0" and
@@ -195,12 +196,12 @@ class PPOCLIP_Agent:
         # normalisers (xb_peer_allreduce_merge; every rank keeps the GLOBAL statistics, bit-identical).
         self._fused_norm = (self._fused_step and (self.use_obsnorm or self.use_rewnorm)
                             and _os.environ.get("XB_FUSED_NORM", "1") != "0"
-                            and (self.world_size == 1 or (self._norm_peer is not None and self.memory.obs_row == 4)))
+                            and (self.world_size == 1 or self._norm_peer is not None))
         self._shard_norm = self._fused_norm and self.world_size > 1
         self._norm_push = _os.environ.get("XB_NORM_PUSH", "1") != "0"      # one-barrier push exchange + merge in one launch
         if self.use_obsnorm and not self._fused_norm and self.memory.obs_row != 4:
             raise NotImplementedError("observations wider than 4 floats are normalised on the fused rollout path only "
-                                      "(single rank, XB_FUSED_STEP / XB_FUSED_NORM on)")
+                                      "(XB_FUSED_STEP / XB_FUSED_NORM on)")
         self._stat_partials = torch.zeros(20 * max(148, N // 32 + 2), **f64)
         self._stat_ticket = torch.zeros(1, dtype=torch.int32, device=dev)
         self._zero_v = None
@@ -218,8 +219,8 @@ class PPOCLIP_Agent:
             # `obs_rms.update(obs)` for the very first observations (ppoclip_agent.py:62); from here on every fused rollout
             # step merges the moments of the observations it produces
             if self._shard_norm:
-                ops.moments4(self._x[0][:N], self._norm_local[:9], self._obs_ws)
-                ops.peer_allreduce_f64(self._norm_peer, 12, self._norm_global, offset=self._norm_off)
+                ops.moments4(self._x[0][:N], self._norm_local[:2 * D + 1], self._obs_ws)
+                ops.peer_allreduce_f64(self._norm_peer, self._norm_n, self._norm_global, offset=self._norm_off)
                 ops.rms_merge_sums(self._norm_global, self._obs_rms[0], self._obs_rms[1], obs_dim, None, None)
                 self._norm_local.zero_()
             else:
@@ -327,13 +328,13 @@ class PPOCLIP_Agent:
                 c = self._rms_cur
                 if self._norm_push:
                     # one kernel, one cross-GPU barrier (push into a parity double-buffered inbox), merge included
-                    ops.peer_allreduce_merge(self._norm_peer, self._norm_local, 12, self._norm_global, self._NORM_INBOX,
+                    ops.peer_allreduce_merge(self._norm_peer, self._norm_local, self._norm_n, self._norm_global, self._NORM_INBOX,
                                              self._obs_rms[c] if self.use_obsnorm else None,
                                              self._obs_rms[c ^ 1] if self.use_obsnorm else None, self._obs_dim,
                                              self._ret_rms if self.use_rewnorm else None,
                                              self._rew_std if self.use_rewnorm else None)
                 else:                 # pull form: two barriers + a separate merge launch
-                    ops.peer_allreduce_f64(self._norm_peer, 12, self._norm_global, offset=self._norm_off)
+                    ops.peer_allreduce_f64(self._norm_peer, self._norm_n, self._norm_global, offset=self._norm_off)
                     ops.rms_merge_sums(self._norm_global, self._obs_rms[c] if self.use_obsnorm else None,
                                        self._obs_rms[c ^ 1] if self.use_obsnorm else None, self._obs_dim,
                                        self._ret_rms if self.use_rewnorm else None, self._rew_std if self.use_rewnorm else None)
@@ -345,11 +346,12 @@ class PPOCLIP_Agent:
         if self._norm_peer is not None:
             # sharded: this step's observation moments + the previous step's return sums in ONE exchange, then the global
             # return normaliser is merged before this step's rewards are scaled (same order as the reference, :87-92)
+            r = self._norm_n - 3              # the return sums follow the 2D + 1 observation moments
             if self.use_obsnorm:
-                ops.moments4(x_cur[:N], self._norm_local[:9], self._obs_ws)
-            ops.peer_allreduce_f64(self._norm_peer, 12, self._norm_global, offset=self._norm_off)
+                ops.moments4(x_cur[:N], self._norm_local[:r], self._obs_ws)
+            ops.peer_allreduce_f64(self._norm_peer, self._norm_n, self._norm_global, offset=self._norm_off)
             if self.use_rewnorm:
-                ops.rms_merge_scalar(self._norm_global[9:], self._ret_rms, self._rew_std)
+                ops.rms_merge_scalar(self._norm_global[r:], self._ret_rms, self._rew_std)
         x_in = self._normalize_obs(x_cur, update=True)            # obs_rms.update(obs); _process_observation (:63-64)
         dist, v = self._policy_forward(x_in)                      # V on [obs_t ; terminal obs of step t-1]
         boot = t > 0 and self._bootstrap_truncations
@@ -382,7 +384,7 @@ class PPOCLIP_Agent:
                              rew_std=self._rew_std if self.use_rewnorm else None, rew_clip=self.rewnorm_range)
         if self.use_rewnorm and self._track_returns:              # returns tracker + ret_rms.update (:87,:91-92)
             if self._norm_peer is not None:      # merged globally at the start of the next step (see above)
-                ops.returns_track(self._returns, env._rew, env._term, env._trunc, self.gamma, self._norm_local[9:], self._ret_ws,
+                ops.returns_track(self._returns, env._rew, env._term, env._trunc, self.gamma, self._norm_local[self._norm_n - 3:], self._ret_ws,
                                   mask_terminal=self._mask_terminal_returns)
             else:
                 ops.returns_track(self._returns, env._rew, env._term, env._trunc, self.gamma, self._ret_sums, self._ret_ws,
@@ -400,7 +402,7 @@ class PPOCLIP_Agent:
         s_in, s_out = self._obs_rms[self._rms_cur], self._obs_rms[self._rms_cur ^ 1]
         sums = self._obs_sums
         if update and self._norm_peer is not None:
-            sums = self._norm_global[:9]            # global moments, exchanged by _rollout_step
+            sums = self._norm_global[:self._norm_n - 3]     # global moments, exchanged by _rollout_step
         elif update:
             ops.moments4(x[:N], self._obs_sums, self._obs_ws)
         ops.rms_normalize(x, self._obs_dim, sums, s_in, s_out, self.obsnorm_range, self._xn, N if update else 0)
@@ -881,7 +883,10 @@ class PPG_Agent(PPOCLIP_Agent):
     (:103), no return tracker (`ret_rms` is never updated: `_process_reward` only clips), minibatches of
     `buffer_size // n_epoch` samples (:29).  The update (:69-98) — policy phase, critic phase, refresh of every stored old
     distribution from the current policy, auxiliary phase — runs on device minibatches (`memory.sample`, nothing crosses
-    PCIe) through PPG_Learner's three fused loss launches and the torch optimiser the caller built; single GPU."""
+    PCIe) through PPG_Learner's three fused loss launches and the torch optimiser the caller built.
+    Env-sharded (a process group of W > 1 ranks): every rank trains on minibatches of its own envs, normalises their advantages
+    with the GLOBAL minibatch statistics, and steps its optimiser on the rank-mean gradient (PPG_Learner.enable_sharding), so
+    the replicas stay bit-identical; the refresh of the stored old distributions stays local to each rank's shard."""
     _bootstrap_truncations = False
     _track_returns = False
     _graph_updates = False
@@ -921,12 +926,27 @@ class PPG_Agent(PPOCLIP_Agent):
         self._device_permutation()
         return self._perm
 
+    def _global_adv_stats(self, perm):
+        """(sum adv, sum adv^2) of every minibatch of the epoch, summed over the ranks (memory_tools.py:241-242 on the global
+        minibatch): one pass over the permutation and one exchange, as PPOCLIP_Agent._epoch_peer does."""
+        mem, B, lr = self.memory, self.batch_size, self.learner
+        M = self.buffer_size // B
+        if lr._peer is not None:
+            ops.adv_stats_minibatches(perm, M, B, mem.n_size, mem.n_envs, mem._adv, 1, lr._peer.stats)
+            ops.peer_allreduce_f64(lr._peer, 2 * M, self._mb_stats_all)
+        else:
+            ops.adv_stats_minibatches(perm, M, B, mem.n_size, mem.n_envs, mem._adv, 1, self._mb_stats_all)
+            xdist.allreduce_adv_stats(self._mb_stats_all[:2 * M], lr.process_group)
+        return self._mb_stats_all
+
     def _phase(self, n_epoch, update):
         mem, B, info = self.memory, self.batch_size, {}
         for ep in range(n_epoch):
             perm = self._draw_permutation()
-            for start in range(0, self.buffer_size, B):
-                obs, act, ret, _, adv, aux = mem.sample(perm[start:start + B])
+            stats = self._global_adv_stats(perm) if (self.world_size > 1 and mem.use_advnorm) else None
+            for k, start in enumerate(range(0, self.buffer_size, B)):
+                kw = {} if stats is None else dict(adv_stats=stats[2 * k:2 * k + 2], adv_count=B * self.world_size)
+                obs, act, ret, _, adv, aux = mem.sample(perm[start:start + B], **kw)
                 # log scalars are read back for the last update of a phase only (one sync per phase, not per update)
                 self.learner.read_back = ep == n_epoch - 1 and start + B >= self.buffer_size
                 info = update(obs, act, ret, adv, aux["old_dist"])
@@ -947,6 +967,8 @@ class PPG_Agent(PPOCLIP_Agent):
 
     def _collect_info(self):
         info = dict(getattr(self, "_phase_info", {}))
+        if self.learner._peer is not None:
+            self.learner._peer.check()
         st = self.envs.ep_stats.cpu().numpy()
         info["new_episodes"] = int(st[0]) - self.current_episode
         info["episodes"] = self.current_episode = int(st[0])

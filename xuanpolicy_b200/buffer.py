@@ -209,7 +209,9 @@ class DummyOnPolicyBuffer:
         self._gae_valid = True
 
     # ---------------------------------------------------------------------------------------------- sample
-    def sample(self, indexes):
+    def sample(self, indexes, adv_stats=None, adv_count=0):
+        """memory_tools.py:231-245.  `adv_stats` (fp64 [2] CUDA, optional): the (sum adv, sum adv^2) over `adv_count` samples
+        to normalise the advantages with instead of this minibatch's own — the global minibatch of an env-sharded agent."""
         assert self.full, "Not enough transitions for on-policy buffer to random sample"
         if not self.native:
             self._run_gae()
@@ -221,11 +223,14 @@ class DummyOnPolicyBuffer:
             obs = torch.empty((B, self.obs_dim), **f32)
             act = torch.empty((B, self.act_dim), **f32)
             ret, val, adv, logp = (torch.empty(B, **f32) for _ in range(4))
+            local = self.use_advnorm and adv_stats is None
             ops.gather_batch(idx, self.n_size, self.n_envs, self._obs, self.obs_dim, self._act, self.act_dim, self._ret,
                              self._val, self._adv, self._logp, obs, act, ret, val, adv, logp,
-                             stats=self._mb_stats if self.use_advnorm else None)
-            if self.use_advnorm:
+                             stats=self._mb_stats if local else None)
+            if local:
                 ops.normalize_adv(adv, self._mb_stats, B)
+            elif self.use_advnorm:
+                ops.normalize_adv(adv, adv_stats, adv_count)
             act = act.reshape((B,) + self._act_shape)
             aux = {"old_logp": logp if self.native else logp.cpu().numpy()} if self._has_logp else {}
             if self._has_dist:       # stays on the device in both modes: the learner is its only consumer

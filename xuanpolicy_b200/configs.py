@@ -53,7 +53,7 @@ _PPG = dict(_COMMON, agent="PPG", n_steps=256, n_epoch=1, n_minibatch=1, policy_
             log_dir="./logs/ppg/")
 
 
-def _build(defaults, env_id, agent_name, policy_builder, device, overrides, agent_class=None):
+def _build(defaults, env_id, agent_name, policy_builder, device, overrides, agent_class=None, process_group=None):
     import torch
     from torch import nn
 
@@ -71,22 +71,24 @@ def _build(defaults, env_id, agent_name, policy_builder, device, overrides, agen
     policy = policy_builder(cfg, envs, rep, act)
     optimizer = torch.optim.Adam(policy.parameters(), cfg.learning_rate, eps=1e-5)
     scheduler = torch.optim.lr_scheduler.LinearLR(optimizer, start_factor=1.0, end_factor=0.0, total_iters=int(cfg.running_steps))
-    return (agent_class or getattr(agents, agent_name))(cfg, envs, policy, optimizer, scheduler, device)
+    return (agent_class or getattr(agents, agent_name))(cfg, envs, policy, optimizer, scheduler, device, process_group=process_group)
 
 
-def build_pg(env_id, device="cuda", agent_class=None, **overrides):
-    """PG_Agent wired like Runner_DRL does for the pg yamls (Categorical_Actor / Gaussian_Actor policy)."""
+def build_pg(env_id, device="cuda", agent_class=None, process_group=None, **overrides):
+    """PG_Agent wired like Runner_DRL does for the pg yamls (Categorical_Actor / Gaussian_Actor policy).
+    `process_group`: env-sharded training as in build_ppo (default: the initialised default group, if any)."""
     from .policies import CategoricalActor, GaussianActor
     from .spaces import is_discrete
 
     def policy(cfg, envs, rep, act):
         cls = CategoricalActor if is_discrete(envs.action_space) else GaussianActor
         return cls(envs.action_space, rep, list(cfg.actor_hidden_size), activation=act, device=device)
-    return _build(_PG, env_id, "PG_Agent", policy, device, overrides, agent_class)
+    return _build(_PG, env_id, "PG_Agent", policy, device, overrides, agent_class, process_group)
 
 
-def build_ppg(env_id, device="cuda", agent_class=None, **overrides):
-    """PPG_Agent wired like Runner_DRL does for the ppg yamls (Categorical_PPG / Gaussian_PPG policy)."""
+def build_ppg(env_id, device="cuda", agent_class=None, process_group=None, **overrides):
+    """PPG_Agent wired like Runner_DRL does for the ppg yamls (Categorical_PPG / Gaussian_PPG policy).
+    `process_group`: env-sharded training as in build_ppo (default: the initialised default group, if any)."""
     from .policies import CategoricalPPGActorCritic, GaussianPPGActorCritic
     from .spaces import is_discrete
 
@@ -94,4 +96,4 @@ def build_ppg(env_id, device="cuda", agent_class=None, **overrides):
         cls = CategoricalPPGActorCritic if is_discrete(envs.action_space) else GaussianPPGActorCritic
         return cls(envs.action_space, rep, list(cfg.actor_hidden_size), list(cfg.critic_hidden_size), activation=act,
                    device=device)
-    return _build(_PPG, env_id, "PPG_Agent", policy, device, overrides, agent_class)
+    return _build(_PPG, env_id, "PPG_Agent", policy, device, overrides, agent_class, process_group)

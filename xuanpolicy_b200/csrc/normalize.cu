@@ -19,39 +19,49 @@ namespace xb {
 constexpr int kNormBlock = 256;
 constexpr int kNormMaxGrid = kNumSMs * 8;
 
-// sums[0..3] = sum x_d, sums[4..7] = sum x_d^2, sums[8] = N
+// rows of D = 4 * V floats: sums[0, D) = sum x_d, sums[D, 2D) = sum x_d^2, sums[2D] = N
+template <int V>
 __global__ void __launch_bounds__(kNormBlock)
-    moments4_kernel(const float4* __restrict__ x, int64_t N, double* __restrict__ sums, double* __restrict__ ws) {
-    __shared__ double smem[8 * 32];
+    moments_kernel(const float4* __restrict__ x, int64_t N, double* __restrict__ sums, double* __restrict__ ws) {
+    constexpr int D = 4 * V, K = 2 * D;
+    __shared__ double smem[K * 32];
     __shared__ bool is_last;
-    double a[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    double a[K];
+#pragma unroll
+    for (int k = 0; k < K; ++k) a[k] = 0.0;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x) {
-        const float4 v = x[i];
-        a[0] += v.x; a[1] += v.y; a[2] += v.z; a[3] += v.w;
-        a[4] += (double)v.x * v.x; a[5] += (double)v.y * v.y; a[6] += (double)v.z * v.z; a[7] += (double)v.w * v.w;
+#pragma unroll
+        for (int v = 0; v < V; ++v) {
+            const float4 q = x[i * V + v];
+            a[4 * v + 0] += q.x; a[4 * v + 1] += q.y; a[4 * v + 2] += q.z; a[4 * v + 3] += q.w;
+            a[D + 4 * v + 0] += (double)q.x * q.x; a[D + 4 * v + 1] += (double)q.y * q.y;
+            a[D + 4 * v + 2] += (double)q.z * q.z; a[D + 4 * v + 3] += (double)q.w * q.w;
+        }
     }
-    block_sum<8>(a, smem);
+    block_sum<K>(a, smem);
     unsigned int* ticket = reinterpret_cast<unsigned int*>(ws);
     double* partials = ws + 8;
     if (threadIdx.x == 0) {
 #pragma unroll
-        for (int k = 0; k < 8; ++k) partials[8 * blockIdx.x + k] = a[k];
+        for (int k = 0; k < K; ++k) partials[K * blockIdx.x + k] = a[k];
         __threadfence();
         is_last = (atomicAdd(ticket, 1u) == gridDim.x - 1);
     }
     __syncthreads();
     if (is_last) {
         __threadfence();
-        double t[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+        double t[K];
+#pragma unroll
+        for (int k = 0; k < K; ++k) t[k] = 0.0;
         for (int b = threadIdx.x; b < (int)gridDim.x; b += blockDim.x) {
 #pragma unroll
-            for (int k = 0; k < 8; ++k) t[k] += partials[8 * b + k];
+            for (int k = 0; k < K; ++k) t[k] += partials[K * b + k];
         }
-        block_sum<8>(t, smem);
+        block_sum<K>(t, smem);
         if (threadIdx.x == 0) {
 #pragma unroll
-            for (int k = 0; k < 8; ++k) sums[k] = t[k];
-            sums[8] = (double)N;
+            for (int k = 0; k < K; ++k) sums[k] = t[k];
+            sums[K] = (double)N;
             *ticket = 0u;
         }
     }
@@ -221,25 +231,25 @@ __global__ void __launch_bounds__(kNormBlock)
     step_stats_finish<D>(s, acc, N, smem, &flag);
 }
 
-// env-sharded form: `sums` [12] = the cross-rank totals (sum x[4], sum x^2[4], N, sum R, sum R^2, n finished) of one step
-__global__ void rms_merge_sums_kernel(const double* __restrict__ sums, const double* __restrict__ obs_state_in,
+// env-sharded form: `sums` [2D + 4] = the cross-rank totals (sum x[D], sum x^2[D], N, sum R, sum R^2, n finished) of one step
+__global__ void rms_merge_sums_kernel(const double* __restrict__ sums, int D, const double* __restrict__ obs_state_in,
                                       double* __restrict__ obs_state_out, int dim, double* __restrict__ ret_state,
                                       float* __restrict__ rew_std) {
-    const int d = threadIdx.x < 4 ? threadIdx.x : 0;
-    merge_step_stats<4>(obs_state_in, obs_state_out, dim, ret_state, rew_std, sums[d], sums[4 + d], sums[8], sums[9], sums[10],
-                        sums[11], threadIdx.x);
+    merge_step_sums(sums, D, obs_state_in, obs_state_out, dim, ret_state, rew_std, threadIdx.x);
 }
 
 }  // namespace xb
 
 using namespace xb;
 
-extern "C" int xb_rms_merge_sums(const double* sums, const double* obs_state_in, double* obs_state_out, int dim,
+extern "C" int xb_rms_merge_sums(const double* sums, int n, const double* obs_state_in, double* obs_state_out, int dim,
                                  double* ret_state, float* rew_std, xb_stream_t stream) {
-    if (!sums || (!obs_state_in && !ret_state) || (obs_state_in && (!obs_state_out || obs_state_in == obs_state_out || dim < 1 || dim > 4)) ||
+    if (n != 12 && n != 20) return XB_E_BADARG;          // 2D + 4 sums of D = 4 or 8 floats per row
+    const int D = (n - 4) / 2;
+    if (!sums || (!obs_state_in && !ret_state) || (obs_state_in && (!obs_state_out || obs_state_in == obs_state_out || dim < 1 || dim > D)) ||
         (ret_state && !rew_std))
         return XB_E_BADARG;
-    rms_merge_sums_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(sums, obs_state_in, obs_state_out, dim, ret_state, rew_std);
+    rms_merge_sums_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(sums, D, obs_state_in, obs_state_out, dim, ret_state, rew_std);
     XB_LAUNCH_CHECK();
     return 0;
 }
@@ -278,9 +288,12 @@ extern "C" int xb_rms_update_rows(const float* x, int row_floats, int dim, int64
     return 0;
 }
 
-extern "C" int xb_moments4(const float* x, double* sums, double* workspace, int64_t N, xb_stream_t stream) {
-    if (N <= 0 || !x || !sums || !workspace) return XB_E_BADARG;
-    moments4_kernel<<<grid_for(N, kNormBlock, 2), kNormBlock, 0, (cudaStream_t)stream>>>((const float4*)x, N, sums, workspace);
+extern "C" int xb_moments4(const float* x, int row_floats, double* sums, double* workspace, int64_t N, xb_stream_t stream) {
+    if (N <= 0 || !x || !sums || !workspace || (row_floats != 4 && row_floats != 8)) return XB_E_BADARG;
+    const int grid = grid_for(N, kNormBlock, 2);
+    cudaStream_t s = (cudaStream_t)stream;
+    if (row_floats == 4) moments_kernel<1><<<grid, kNormBlock, 0, s>>>((const float4*)x, N, sums, workspace);
+    else moments_kernel<2><<<grid, kNormBlock, 0, s>>>((const float4*)x, N, sums, workspace);
     XB_LAUNCH_CHECK();
     return 0;
 }

@@ -98,6 +98,19 @@ __device__ __forceinline__ void merge_step_stats(const double* obs_state_in, dou
     }
 }
 
+// merge_step_stats from the cross-rank totals of one step in the StepStats::sums_out layout [2D + 4] = sum x[D], sum x^2[D], N,
+// sum R, sum R^2, n finished, for D = 4 or 8 floats per observation row (threads 0..31 of one warp).
+__device__ __forceinline__ void merge_step_sums(const double* sums, int D, const double* obs_state_in, double* obs_state_out, int dim,
+                                                double* ret_state, float* rew_std, int tid) {
+    const int d = tid < D ? tid : 0;
+    if (D == 8)
+        merge_step_stats<8>(obs_state_in, obs_state_out, dim, ret_state, rew_std, sums[d], sums[8 + d], sums[16], sums[17], sums[18],
+                            sums[19], tid);
+    else
+        merge_step_stats<4>(obs_state_in, obs_state_out, dim, ret_state, rew_std, sums[d], sums[4 + d], sums[8], sums[9], sums[10],
+                            sums[11], tid);
+}
+
 // Sum of 32 doubles in shared memory, read in an order rotated by `rot` (lanes that walk rows 256 B apart then never share a
 // bank) and added as four independent chains: a fixed association order, a quarter of the dependent-add latency.
 __device__ __forceinline__ double row_sum32(const double* row, int rot) {

@@ -14,6 +14,8 @@
 //     (the sharded form of ppoclip_learner.py:47-49): the collective IS the first pass of the optimiser.
 //     The inbox is double-buffered by launch parity, so no second barrier is needed: a peer can only overwrite
 //     inbox[p] two launches later, after a barrier that this rank enters only once it has finished reading inbox[p].
+//   * xb_peer_allreduce_mean — the same push / barrier / rank-order sum, scaled by 1/W and written to local memory, without
+//     the optimiser scalars: the gradient exchange of a learner that steps a torch optimiser itself (PPG_Learner).
 //   * xb_peer_allreduce_f64 — the (sum adv, sum adv^2) of every minibatch of an epoch in one exchange
 //     (the sharded form of memory_tools.py:241-242), fed by xb_adv_stats_minibatches.  Pull-based, two barriers.
 //
@@ -94,15 +96,14 @@ __device__ __forceinline__ void peer_barrier(const PeerTable& t, int rank, int W
 
 constexpr int kPeerBlock = 512;
 
-// ws layout = optim.cu: [0] norm [1] clip [2] lr [3] bc1 [4] sqrt(bc2) [5] ticket bits, [8..) per-CTA partials.
-// tickets: u32 [kPeerSlots] local per-CTA barrier counters (one tick per launch; its parity selects the inbox half).
-__global__ void __launch_bounds__(kPeerBlock)
-    peer_allreduce_grad_norm_kernel(PeerTable t, int rank, int W, int64_t n4, const float* __restrict__ grad_in,
-                                    float* __restrict__ grad_out, uint32_t* __restrict__ tickets,
-                                    int64_t* __restrict__ step_dev, AdamHyper h, double* __restrict__ ws,
-                                    float* __restrict__ lr_out, float* __restrict__ gnorm_out) {
-    __shared__ double smem[32];
-    __shared__ bool is_last;
+// The gradient exchange shared by the kernels below (every CTA of the grid calls it): CTA b pushes its grid-stride slice of
+// grad_in (float4 [n4]) into inbox[parity][rank] of every peer, passes ONE cross-GPU barrier on flag slot b, then calls
+// visit(i, s) for each float4 i of its slice with s = the W inbox rows summed in rank order 0..W-1 out of LOCAL memory
+// (bit-identical on every rank).  tickets: u32 [kPeerSlots] local per-CTA barrier counters (one tick per launch; its parity
+// selects the inbox half).  Launches that share a comm block must use the same grid, i.e. the same n.
+template <class Visit>
+__device__ __forceinline__ void peer_grad_sum(const PeerTable& t, int rank, int W, int64_t n4, const float* __restrict__ grad_in,
+                                              uint32_t* __restrict__ tickets, Visit visit) {
     const int slot = blockIdx.x;
     const uint32_t base_ticket = tickets[slot];          // read by every thread before thread 0 advances it below
     const int64_t half = (int64_t)(base_ticket & 1u) * kPeerMaxRanks * n4;   // float4 offset of this launch's inbox half
@@ -115,20 +116,43 @@ __global__ void __launch_bounds__(kPeerBlock)
     peer_barrier(t, rank, W, slot, base_ticket + 1, tickets);     // every rank's slice has landed in my inbox
     if (threadIdx.x == 0) tickets[slot] = base_ticket + 1;
     const float4* box = reinterpret_cast<const float4*>(t.base[rank] + kPeerGradOff) + half;
-    double acc[1] = {0.0};
-    float4* out4 = reinterpret_cast<float4*>(grad_out);
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
         float4 s = ld_peer_f4(box + i);                  // written by remote stores: bypass any stale L1 line
         for (int r = 1; r < W; ++r) {
             const float4 g = ld_peer_f4(box + (int64_t)r * n4 + i);
             s.x += g.x; s.y += g.y; s.z += g.z; s.w += g.w;
         }
+        visit(i, s);
+    }
+}
+
+// ws layout = optim.cu: [0] norm [1] clip [2] lr [3] bc1 [4] sqrt(bc2) [5] ticket bits, [8..) per-CTA partials.
+__global__ void __launch_bounds__(kPeerBlock)
+    peer_allreduce_grad_norm_kernel(PeerTable t, int rank, int W, int64_t n4, const float* __restrict__ grad_in,
+                                    float* __restrict__ grad_out, uint32_t* __restrict__ tickets,
+                                    int64_t* __restrict__ step_dev, AdamHyper h, double* __restrict__ ws,
+                                    float* __restrict__ lr_out, float* __restrict__ gnorm_out) {
+    __shared__ double smem[32];
+    __shared__ bool is_last;
+    double acc[1] = {0.0};
+    float4* out4 = reinterpret_cast<float4*>(grad_out);
+    peer_grad_sum(t, rank, W, n4, grad_in, tickets, [&](int64_t i, const float4& s) {
         out4[i] = s;
         const double gx = (double)(s.x * h.grad_scale), gy = (double)(s.y * h.grad_scale);
         const double gz = (double)(s.z * h.grad_scale), gw = (double)(s.w * h.grad_scale);
         acc[0] += gx * gx + gy * gy + gz * gz + gw * gw;
-    }
+    });
     grad_norm_finish(acc[0], step_dev, h, ws, lr_out, gnorm_out, smem, &is_last);
+}
+
+// grad_out = (sum over ranks of grad_in) * inv_w: the data-parallel mean gradient, for a caller that steps its own optimiser.
+__global__ void __launch_bounds__(kPeerBlock)
+    peer_allreduce_mean_kernel(PeerTable t, int rank, int W, int64_t n4, const float* __restrict__ grad_in,
+                               float* __restrict__ grad_out, uint32_t* __restrict__ tickets, float inv_w) {
+    float4* out4 = reinterpret_cast<float4*>(grad_out);
+    peer_grad_sum(t, rank, W, n4, grad_in, tickets, [&](int64_t i, const float4& s) {
+        out4[i] = make_float4(s.x * inv_w, s.y * inv_w, s.z * inv_w, s.w * inv_w);
+    });
 }
 
 // out[j] = sum over ranks (rank order) of the peers' stats[j], j < n <= kPeerStatsMax.  One CTA, the last flag slot.
@@ -148,15 +172,15 @@ __global__ void __launch_bounds__(256)
 }
 
 // The per-vector-step exchange of the running-statistics sums (env-sharded use_obsnorm / use_rewnorm) as ONE kernel with ONE
-// cross-GPU barrier, followed in the same kernel by the normaliser merge (normalize.cuh merge_step_stats = xb_rms_merge_sums):
-// every rank PUSHES its n <= 16 sums into row [parity][rank] of an inbox inside every peer's statistics area, signals, waits, and
+// cross-GPU barrier, followed in the same kernel by the normaliser merge (normalize.cuh merge_step_sums = xb_rms_merge_sums):
+// every rank PUSHES its n <= kPeerPushMax sums into row [parity][rank] of an inbox inside every peer's statistics area, signals, waits, and
 // adds the W rows in rank order out of LOCAL memory (bit-identical totals on every rank).  parity = the launch counter's low bit
 // (a device counter: graph replays and odd horizons are fine); a row can only be overwritten two launches later, after a
 // barrier this rank enters only once it has read it — so no second barrier (the pull form above needs two), and no separate
 // merge launch.  Launched with the programmatic-serialization attribute: the rollout forward that follows may become resident
 // (set-up, resident weights) while this kernel waits for its peers.
 constexpr int kPeerPushSlot = kPeerSlots - 3;
-constexpr int kPeerPushMax = 16;
+constexpr int kPeerPushMax = 20;       // the 2D + 4 step sums of 8-float observation rows
 __global__ void __launch_bounds__(128)
     peer_allreduce_merge_kernel(PeerTable t, int rank, int W, int inbox_off, int n, const double* __restrict__ src,
                                 double* __restrict__ out, uint32_t* __restrict__ tickets, const double* __restrict__ obs_state_in,
@@ -184,11 +208,8 @@ __global__ void __launch_bounds__(128)
     }
     __syncthreads();
     if (threadIdx.x == 0) tickets[kPeerPushSlot] = ticket;
-    if (threadIdx.x < 32 && (obs_state_in || ret_state)) {
-        const int d = threadIdx.x < 4 ? threadIdx.x : 0;
-        merge_step_stats<4>(obs_state_in, obs_state_out, dim, ret_state, rew_std, sums[d], sums[4 + d], sums[8], sums[9], sums[10],
-                            sums[11], threadIdx.x);
-    }
+    if (threadIdx.x < 32 && (obs_state_in || ret_state))
+        merge_step_sums(sums, (n - 4) / 2, obs_state_in, obs_state_out, dim, ret_state, rew_std, threadIdx.x);
 }
 
 // (sum, sumsq) of the advantages of every minibatch of an epoch in one pass over the permutation:
@@ -280,6 +301,20 @@ extern "C" int xb_peer_allreduce_grad_norm(const void* const* peer_bases /* host
     return 0;
 }
 
+extern "C" int xb_peer_allreduce_mean(const void* const* peer_bases /* host [W] */, int rank, int W, int64_t n, const float* grad_in,
+                                      float* grad_out, uint32_t* tickets, xb_stream_t stream) {
+    PeerTable t;
+    int rc = make_table(peer_bases, rank, W, &t);
+    if (rc) return rc;
+    if (n <= 0 || (n & 3) || !grad_in || !grad_out || !tickets) return XB_E_BADARG;
+    const int64_t n4 = n / 4;
+    int grid = (int)((n4 + kPeerBlock - 1) / kPeerBlock);
+    if (grid > kPeerSlots - 3) grid = kPeerSlots - 3;
+    peer_allreduce_mean_kernel<<<grid, kPeerBlock, 0, (cudaStream_t)stream>>>(t, rank, W, n4, grad_in, grad_out, tickets, 1.0f / (float)W);
+    XB_LAUNCH_CHECK();
+    return 0;
+}
+
 extern "C" int xb_peer_allreduce_f64(const void* const* peer_bases /* host [W] */, int rank, int W, int offset, int n,
                                      double* out, uint32_t* tickets, xb_stream_t stream) {
     PeerTable t;
@@ -300,8 +335,8 @@ extern "C" int xb_peer_allreduce_merge(const void* const* peer_bases /* host [W]
     if (!src || !out || !tickets || n <= 0 || n > kPeerPushMax || inbox_offset < 0 ||
         inbox_offset + 2 * kPeerMaxRanks * kPeerPushMax > kPeerStatsMax)
         return XB_E_BADARG;
-    if ((obs_state_in || ret_state) && n != 12) return XB_E_BADARG;       // the merge reads the 12 step sums
-    if (obs_state_in && (!obs_state_out || obs_state_in == obs_state_out || dim < 1 || dim > 4)) return XB_E_BADARG;
+    if ((obs_state_in || ret_state) && n != 12 && n != 20) return XB_E_BADARG;     // the merge reads the 2D + 4 step sums, D = 4 or 8
+    if (obs_state_in && (!obs_state_out || obs_state_in == obs_state_out || dim < 1 || dim > (n - 4) / 2)) return XB_E_BADARG;
     if (ret_state && !rew_std) return XB_E_BADARG;
     XB_CUDA(launch_pdl(peer_allreduce_merge_kernel, dim3(1), dim3(128), 0, (cudaStream_t)stream, true, t, rank, W, inbox_offset, n, src,
                        out, tickets, obs_state_in, obs_state_out, dim, ret_state, rew_std));

@@ -562,16 +562,65 @@ class PPG_Learner(_DistLossLearner):
     """PPG_Learner drop-in (xuance/torch/learners/policy_gradient/ppg_learner.py:5-91): same constructor and the
     three phase updates `update_policy / update_critic / update_auxiliary(obs, act, ret, adv, old_dists)` over a
     policy returning `(outputs, a_dist, v, aux_v)`.  Each phase is one launch of the generic kernel of
-    csrc/dist_loss.cu with that phase's coefficients."""
+    csrc/dist_loss.cu with that phase's coefficients.
+
+    `process_group` (or `enable_sharding`): env-sharded data parallelism over W ranks, each updating on its equal share of the
+    minibatch.  Rank 0's parameters are broadcast once; after every phase's backward the gradients the phase reached are
+    averaged over the ranks (xb_peer_allreduce_mean over NVLink peer memory; an NCCL all-reduce when XB_PEER_COMM=0 or CUDA IPC
+    is unavailable), so the caller's torch optimiser takes the same step on every rank.  Parameters the phase did not reach
+    keep `grad = None` and the optimiser skips them, as it does for the reference's `loss.backward()`."""
 
     def __init__(self, policy, optimizer, scheduler=None, device=None, model_dir="./", ent_coef=0.005, clip_range=0.25,
-                 kl_beta=1.0):
+                 kl_beta=1.0, process_group=None):
         super().__init__(policy, optimizer, scheduler, device, model_dir, vf_coef=0.0, ent_coef=ent_coef,
                          clip_range=clip_range, clip_grad_norm=None, use_grad_clip=False)
         self.kl_beta = kl_beta
         self.policy_iterations = 0
         self.value_iterations = 0
         self.read_back = True       # False: the phase update returns {} without reading the log scalars back (no sync)
+        self._shard = None          # (params, flat gradient in, flat mean out, their per-parameter views) when env-sharded
+        if process_group is not None:
+            self.enable_sharding(process_group)
+
+    def enable_sharding(self, process_group=None):
+        """Switch to env-sharded updates when `process_group` (default: the initialised default group) has W > 1 ranks."""
+        d = torch.distributed
+        if self._shard is not None or (process_group is None and not (d.is_available() and d.is_initialized())):
+            return
+        world = d.get_world_size(process_group)
+        if world == 1:
+            return
+        self.process_group, self.world_size = process_group, world
+        params = [p for p in self.policy.parameters() if p.requires_grad]
+        for p in params:                    # replicated policy: every rank starts from rank 0's parameters
+            xdist.broadcast_parameters(p.data, 0, process_group)
+        pad4 = lambda k: (k + 3) // 4 * 4   # the peer kernels move float4s
+        offs = np.cumsum([0] + [pad4(p.numel()) for p in params])
+        g_in = torch.zeros(int(offs[-1]), dtype=torch.float32, device=self.device)
+        g_out = torch.zeros_like(g_in)
+        view = lambda buf: [buf[o:o + p.numel()].view_as(p) for o, p in zip(offs, params)]
+        self._shard = (params, g_in, g_out, view(g_in), view(g_out))
+        if os.environ.get("XB_PEER_COMM", "1") != "0":
+            self._open_peer_comm(g_in.numel())
+
+    def _average_grads(self):
+        """The gradients this phase reached -> one flat buffer -> mean over the ranks -> back into `.grad`."""
+        params, g_in, g_out, v_in, v_out = self._shard
+        live = [k for k, p in enumerate(params) if p.grad is not None]
+        torch._foreach_copy_([v_in[k] for k in live], [params[k].grad for k in live])
+        if self._peer is not None:
+            ops.peer_allreduce_mean(self._peer, g_in, g_out)
+        else:
+            xdist.allreduce_flat_grad(g_in, self.process_group)
+            torch.mul(g_in, 1.0 / self.world_size, out=g_out)
+        torch._foreach_copy_([params[k].grad for k in live], [v_out[k] for k in live])
+
+    def _backward_step(self, *args, scheduler=True, **kw):
+        """_dist_loss_backward, the cross-rank gradient mean when env-sharded, then the optimiser (and scheduler) step."""
+        count = self._dist_loss_backward(*args, **kw)
+        if self._shard is not None:
+            self._average_grads()
+        return count, self._step(scheduler)
 
     def _forward(self, obs_batch):
         return self.policy(torch.as_tensor(obs_batch, device=self.device))
@@ -582,9 +631,8 @@ class PPG_Learner(_DistLossLearner):
             B = ret.shape[0]
             _, a_dist, v, _ = self._forward(obs_batch)
             self.optimizer.zero_grad()
-            self._dist_loss_backward(a_dist, v, None, act, ret, adv, old_dists, clip_range=self.clip_range, surr_coef=1.0,
-                                     kl_coef=0.0, vf_coef=0.0, ent_coef=self.ent_coef)
-            lr = self._step()
+            _, lr = self._backward_step(a_dist, v, None, act, ret, adv, old_dists, clip_range=self.clip_range, surr_coef=1.0,
+                                        kl_coef=0.0, vf_coef=0.0, ent_coef=self.ent_coef)
             self.policy_iterations += 1
             if not self.read_back:
                 return {}
@@ -598,9 +646,8 @@ class PPG_Learner(_DistLossLearner):
             B = ret.shape[0]
             _, a_dist, v, _ = self._forward(obs_batch)
             self.optimizer.zero_grad()
-            self._dist_loss_backward(a_dist, v, None, act, ret, adv, old_dists, clip_range=0.0, surr_coef=0.0, kl_coef=0.0,
-                                     vf_coef=1.0, ent_coef=0.0)
-            self._step(scheduler=False)                       # the reference steps no scheduler here (:63)
+            self._backward_step(a_dist, v, None, act, ret, adv, old_dists, clip_range=0.0, surr_coef=0.0, kl_coef=0.0,
+                                vf_coef=1.0, ent_coef=0.0, scheduler=False)     # the reference steps no scheduler here (:63)
             self.value_iterations += 1
             if not self.read_back:
                 return {}
@@ -613,9 +660,9 @@ class PPG_Learner(_DistLossLearner):
             B = ret.shape[0]
             _, a_dist, v, aux_v = self._forward(obs_batch)
             self.optimizer.zero_grad()
-            kl_count = self._dist_loss_backward(a_dist, v, aux_v, act, ret, adv, old_dists, clip_range=0.0, surr_coef=0.0,
-                                                kl_coef=self.kl_beta, vf_coef=1.0, ent_coef=0.0, aux_coef=1.0)
-            self._step(scheduler=False)                       # (:84)
+            kl_count, _ = self._backward_step(a_dist, v, aux_v, act, ret, adv, old_dists, clip_range=0.0, surr_coef=0.0,
+                                              kl_coef=self.kl_beta, vf_coef=1.0, ent_coef=0.0, aux_coef=1.0,
+                                              scheduler=False)                            # (:84)
             if not self.read_back:
                 return {}
             s = self._scalars.cpu().numpy()

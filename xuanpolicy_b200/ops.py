@@ -242,6 +242,13 @@ def adam_apply_split(param, grad, exp_avg, exp_avg_sq, beta1, beta2, eps, grad_s
               _p(lo0, F32), off(w1), _p(hi1, F32), _p(lo1, F32), N, K, _p(thi, F32), _p(tlo, F32), _stream())
 
 
+def peer_allreduce_mean(peer, grad_in, grad_out):
+    """grad_out = the mean over ranks of every rank's grad_in (fp32 [peer.n]), summed in rank order over peer memory and
+    bit-identical on every rank (xb_peer_allreduce_mean)."""
+    _lib.call("xb_peer_allreduce_mean", peer.bases, peer.rank, peer.world, peer.n, _p(grad_in, F32), _p(grad_out, F32),
+              _p(peer.tickets, I32), _stream())
+
+
 def peer_allreduce_f64(peer, n, out, offset=0):
     """out[:n] = sum over ranks of doubles [offset, offset + n) of each rank's comm-block statistics."""
     _lib.call("xb_peer_allreduce_f64", peer.bases, peer.rank, peer.world, int(offset), int(n), _p(out, F64),
@@ -266,7 +273,8 @@ def act_bias_bwd(dy, y, slope, dz, dbias, workspace):
 
 
 def moments4(x, sums, workspace):
-    _lib.call("xb_moments4", _p(x, F32), _p(sums, F64), _p(workspace, F64), x.shape[0], _stream())
+    """sums[:2D + 1] = column sums, column sums of squares and the row count of x [N, D], D = 4 or 8."""
+    _lib.call("xb_moments4", _p(x, F32), x.shape[1], _p(sums, F64), _p(workspace, F64), x.shape[0], _stream())
 
 
 def rms_normalize(x, dim, sums, state_in, state_out, clip, out, n_merged_rows):
@@ -285,7 +293,8 @@ def rms_update_rows(x, dim, state_in, state_out, partials, ticket):
 
 
 def rms_merge_sums(sums, obs_in, obs_out, dim, ret_state, rew_std):
-    _lib.call("xb_rms_merge_sums", _p(sums, F64), _p(obs_in, F64), _p(obs_out, F64), int(dim), _p(ret_state, F64),
+    """Merges one step's cross-rank totals sums [2D + 4] (D = 4 or 8 floats per observation row) into the normalisers."""
+    _lib.call("xb_rms_merge_sums", _p(sums, F64), sums.numel(), _p(obs_in, F64), _p(obs_out, F64), int(dim), _p(ret_state, F64),
               _p(rew_std, F32), _stream())
 
 
