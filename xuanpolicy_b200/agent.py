@@ -28,10 +28,13 @@ every rank holds the global statistics.
 `train(train_steps)` accepts any step count (ppoclip_agent.py:59-61): whole rollouts replay the captured graph, a
 partial rollout runs the same launches eagerly and the buffer position carries over to the next call.
 """
+import os
+import time
+
 import numpy as np
 import torch
 
-from . import _lib, ops
+from . import _lib, checkpoint, ops
 from . import dist as xdist
 from .buffer import DummyOnPolicyBuffer
 from .learner import PPOCLIP_Learner
@@ -75,6 +78,13 @@ class HostPermutationFeeder:
         ev.record()
         self.consumed[iteration & 1] = ev
         self.futures.pop(iteration, None)
+
+    def drain(self):
+        """Waits for every outstanding draw and forgets it (before the iteration number changes under the feeder)."""
+        for futures in self.futures.values():
+            for f in futures:
+                f.result()
+        self.futures.clear()
 
 
 class PPOCLIP_Agent:
@@ -690,16 +700,25 @@ class PPOCLIP_Agent:
             xdist.allreduce_flat_grad(lr._flat.flat_grad, lr.process_group)
             lr.stage_optimizer()
 
+    def _state_tensors(self):
+        """The device tensors of the training state, by name: everything a rollout or an update phase carries forward.
+        Graph capture snapshots and restores them around its warm-up (_snapshot); checkpoints save them with the buffer
+        rows and host counters on top (_checkpoint_tensors, _host_state).  Left out because nothing reads them before
+        rewriting them: scratch (statistics partials, tickets, workspaces, minibatch buffers), the trig cache (results do
+        not depend on it), the tf32 operand copies and the folded head (derived from the weights), peer comm blocks."""
+        env = self.envs
+        named = {"env.state": env._state, "env.rng": env._rng, "env.elapsed": env._elapsed, "env.ep_score": env._ep_score,
+                 "env.ep_stats": env.ep_stats, "ctr": self._ctr, "perm_ctr": self._perm_ctr, "x0": self._x[0], "x1": self._x[1],
+                 "obs_rms0": self._obs_rms[0], "obs_rms1": self._obs_rms[1], "ret_rms": self._ret_rms,
+                 "returns": self._returns, "rew_std": self._rew_std}
+        if self._norm_peer is not None:
+            named["norm_local"] = self._norm_local      # pending return sums of the last step (merged at the next step)
+        named.update(self.learner.state_tensors())
+        return named
+
     def _snapshot(self):
         """Everything a warm-up rollout/update mutates, so that capturing leaves training state untouched."""
-        env, fl = self.envs, self.learner._flat
-        tensors = [env._state, env._rng, env._elapsed, env._ep_score, env.ep_stats, self._ctr, self._perm_ctr, self._x[0], self._x[1],
-                   self._obs_rms[0], self._obs_rms[1], self._ret_rms, self._returns, self._rew_std]
-        if fl is not None:
-            tensors += [fl.flat_param, fl.exp_avg, fl.exp_avg_sq, fl.step, fl.lr]
-        if self._norm_peer is not None:
-            tensors.append(self._norm_local)      # pending return sums of the last step (merged at the next step)
-        return [(t, t.clone()) for t in tensors] + [("cur", self._cur)]
+        return [(t, t.clone()) for t in self._state_tensors().values()] + [("cur", self._cur)]
 
     def _restore(self, snap):
         for t, c in snap:
@@ -707,6 +726,136 @@ class PPOCLIP_Agent:
                 self._cur = c
             else:
                 t.copy_(c)
+
+    # ---------------------------------------------------------------------------------------------- checkpoints
+    def _checkpoint_tensors(self, t):
+        """_state_tensors plus rows [0, t) of every per-step array the rollout writes: the part of an unfinished rollout
+        that is already in the buffer (at a rollout boundary, t = 0, the next rollout overwrites every row)."""
+        named = self._state_tensors()
+        if t > 0:
+            mem = self.memory
+            for n in ("_obs", "_act", "_rew", "_val", "_term", "_trunc", "_logp", "_boot", "_dist"):
+                if getattr(mem, n) is not None:
+                    named["buffer." + n[1:]] = getattr(mem, n)[:t]
+        return named
+
+    def _host_state(self):
+        mem = self.memory
+        return {"t": self._t, "cur": self._cur, "rms_cur": self._rms_cur, "iteration": self._iteration,
+                "current_step": self.current_step, "current_episode": self.current_episode, "memory_ptr": mem.ptr,
+                "memory_size": mem.size, "last_info": self.last_info, "learner": self.learner.host_state()}
+
+    def _load_host_state(self, st):
+        self._t, self._cur, self._rms_cur, self._iteration = st["t"], st["cur"], st["rms_cur"], st["iteration"]
+        self.current_step, self.current_episode = st["current_step"], st["current_episode"]
+        self.memory.ptr, self.memory.size = st["memory_ptr"], st["memory_size"]
+        self.last_info = st["last_info"]
+        self.learner.load_host_state(st["learner"])
+
+    def _checkpoint_meta(self):
+        return {"format_version": checkpoint.FORMAT_VERSION, "agent_class": type(self).__name__, "env_id": self.envs.env_id,
+                "n_envs": self.n_envs, "n_steps": self.n_steps, "obs_row": self.memory.obs_row, "world_size": self.world_size,
+                "rank": self._rank(), "params": [(n, list(p.shape)) for n, p in self.policy.named_parameters()],
+                "config": checkpoint.plain_config(self.config)}
+
+    def _rebuild_derived(self):
+        """The tf32 hi/lo operand copies and the folded Discrete(3) head follow the weights; a rollout resumed part-way runs
+        its forwards without the refresh at the rollout's start, so they are rebuilt from the loaded weights here."""
+        if self.learner._fused is not None:
+            self.learner._fused.refresh_weights()
+
+    def save_checkpoint(self, path):
+        """Writes the full training state into the directory `path`, one file per rank (`rank<r>-of-<W>.pt`): env physics
+        and RNG streams, sampling and permutation counters, observation ping-pong, normalisers, optimiser state, the
+        buffer rows of an unfinished rollout and the host counters.  A fresh agent built with the same config continues
+        from it with `load_checkpoint` as if the run had never stopped.  Call it between `train()` calls (mid-rollout
+        included).  Each file is written under a temporary name and moved into place, so a save that is cut off leaves
+        the previous checkpoint.  Env-sharded, every rank calls it; they pass one barrier after writing."""
+        with torch.cuda.device(self.device):
+            tensors = {k: v.detach().to("cpu", copy=True) for k, v in self._checkpoint_tensors(self._t).items()}
+        payload = {"meta": self._checkpoint_meta(), "tensors": tensors, "host": checkpoint.to_cpu(self._host_state())}
+        os.makedirs(path, exist_ok=True)
+        checkpoint.write_atomic(payload, checkpoint.rank_file(path, self._rank(), self.world_size))
+        if self.world_size > 1:
+            torch.distributed.barrier(group=self.learner.process_group)
+
+    def load_checkpoint(self, path):
+        """Restores what `save_checkpoint` wrote.  Refuses with a ValueError naming the field, before anything is copied,
+        when the checkpoint belongs to another agent class, env, env count, horizon, world size or rank, another policy
+        shape, or another config (keys that only name places or logging, checkpoint.PLACE_KEYS, may differ).  Every tensor
+        is copied in place, so CUDA graphs the agent has already captured stay valid.  Env-sharded, every rank calls it;
+        the replicated tensors (parameters, optimiser state, normalisers) must be bit-identical across the ranks' files."""
+        rank, world = self._rank(), self.world_size
+        err = None
+        try:
+            payload = checkpoint.read(path, rank, world)
+            checkpoint.check_compatible(payload["meta"], self._checkpoint_meta())
+            t = payload["host"]["t"]
+            if not 0 <= t < self.n_steps:
+                raise ValueError("checkpoint t (steps into the rollout) is %r, outside [0, %d)" % (t, self.n_steps))
+            live = self._checkpoint_tensors(t)
+            checkpoint.check_tensors(payload["tensors"], live)
+        except (ValueError, FileNotFoundError) as e:
+            err = e
+        if world > 1:          # every rank refuses together, or none does
+            group = self.learner.process_group
+            bad = torch.tensor([int(err is not None)], dtype=torch.int32, device=self.device)
+            torch.distributed.all_reduce(bad, group=group)
+            if err is None and int(bad.item()):
+                err = ValueError("checkpoint refused on another rank")
+            if err is None:
+                differ = checkpoint.differing_across_ranks(checkpoint.replicated(payload), self.device, group)
+                if differ:
+                    err = ValueError("checkpoint replicated tensors differ across the ranks' files: %s" % ", ".join(differ))
+        if err is not None:
+            raise err
+        with torch.cuda.device(self.device), torch.no_grad():
+            if self._feeder is not None:     # outstanding draws write pinned sets that the new iteration may reuse
+                self._feeder.drain()
+            for k, v in live.items():
+                v.copy_(payload["tensors"][k])
+            self._trig_cache.fill_(float("nan"))
+            self._load_host_state(payload["host"])
+            self._perm_staged = False
+            self._rebuild_derived()
+            torch.cuda.synchronize(self.device)
+            if self._feeder is not None:
+                self._feeder.prefetch(self._iteration)
+
+    def save_model(self, model_name):
+        """The reference's Agent.save_model: the policy's state_dict (learner.save_model) into
+        `<config.model_dir>/seed_<seed>_<time>/<model_name>` (one directory per agent, the layout learner.load_model
+        searches), and with `use_obsnorm` the observation statistics as `obs_rms.npy` beside it.  Weights only: a run is
+        resumed from save_checkpoint.  Env-sharded, rank 0 writes (policy and statistics are replicated)."""
+        if self._rank() != 0:
+            return
+        if getattr(self, "_model_dir_save", None) is None:
+            stamp = time.asctime().replace(" ", "").replace(":", "_")
+            self._model_dir_save = os.path.join(getattr(self.config, "model_dir", "./"), "seed_%d_%s" % (self.seed, stamp))
+        os.makedirs(self._model_dir_save, exist_ok=True)
+        self.learner.save_model(os.path.join(self._model_dir_save, model_name))
+        if self.use_obsnorm:
+            st, D, od = self._obs_rms[self._rms_cur].cpu().numpy(), self.memory.obs_row, self._obs_dim
+            np.save(os.path.join(self._model_dir_save, "obs_rms.npy"),
+                    {"count": float(st[2 * D]), "mean": st[:od].copy(), "var": st[D:D + od].copy()})
+
+    def load_model(self, path, seed=1):
+        """The reference's Agent.load_model: the newest policy file of the `seed_<seed>` directory under `path`, and with
+        `use_obsnorm` its `obs_rms.npy` into both observation-statistics slots.  Returns the directory it read."""
+        path = self.learner.load_model(path, seed)
+        with torch.cuda.device(self.device):
+            self._rebuild_derived()
+            if self.use_obsnorm:
+                f = os.path.join(path, "obs_rms.npy")
+                if not os.path.exists(f):
+                    raise RuntimeError("Failed to load observation status file 'obs_rms.npy' from %s!" % f)
+                stat = np.load(f, allow_pickle=True).item()
+                D, od = self.memory.obs_row, self._obs_dim
+                for st in self._obs_rms:
+                    st[:od].copy_(torch.from_numpy(np.asarray(stat["mean"], np.float64).reshape(od)))
+                    st[D:D + od].copy_(torch.from_numpy(np.asarray(stat["var"], np.float64).reshape(od)))
+                    st[2 * D].fill_(float(stat["count"]))
+        return path
 
     # ---------------------------------------------------------------------------------------------- public API
     def train(self, train_steps):
@@ -964,6 +1113,13 @@ class PPG_Agent(PPOCLIP_Agent):
         info.update(self._phase(self.aux_nepoch, L.update_auxiliary))
         self._phase_info = info
         self._iteration += 1
+
+    def _host_state(self):
+        return dict(super()._host_state(), phase_info=getattr(self, "_phase_info", {}))
+
+    def _load_host_state(self, st):
+        super()._load_host_state(st)
+        self._phase_info = st["phase_info"]
 
     def _collect_info(self):
         info = dict(getattr(self, "_phase_info", {}))

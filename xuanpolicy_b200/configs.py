@@ -53,7 +53,8 @@ _PPG = dict(_COMMON, agent="PPG", n_steps=256, n_epoch=1, n_minibatch=1, policy_
             log_dir="./logs/ppg/")
 
 
-def _build(defaults, env_id, agent_name, policy_builder, device, overrides, agent_class=None, process_group=None):
+def _build(defaults, env_id, agent_name, policy_builder, device, overrides, agent_class=None, process_group=None,
+           policy_seed=None):
     import torch
     from torch import nn
 
@@ -63,7 +64,7 @@ def _build(defaults, env_id, agent_name, policy_builder, device, overrides, agen
     cfg = dict(defaults, env_id=env_id, device=device)
     cfg.update(overrides)
     cfg = Namespace(**cfg)
-    torch.manual_seed(cfg.seed)
+    torch.manual_seed(cfg.seed if policy_seed is None else policy_seed)
     envs = DummyVecEnv_Gym(make_env_fns(env_id, cfg.seed, cfg.parallels), device=device, native=True)
     envs.reset()
     act = {"ReLU": nn.ReLU, "LeakyReLU": nn.LeakyReLU}[cfg.activation]
@@ -74,21 +75,23 @@ def _build(defaults, env_id, agent_name, policy_builder, device, overrides, agen
     return (agent_class or getattr(agents, agent_name))(cfg, envs, policy, optimizer, scheduler, device, process_group=process_group)
 
 
-def build_pg(env_id, device="cuda", agent_class=None, process_group=None, **overrides):
+def build_pg(env_id, device="cuda", agent_class=None, process_group=None, policy_seed=None, **overrides):
     """PG_Agent wired like Runner_DRL does for the pg yamls (Categorical_Actor / Gaussian_Actor policy).
-    `process_group`: env-sharded training as in build_ppo (default: the initialised default group, if any)."""
+    `process_group`: env-sharded training as in build_ppo (default: the initialised default group, if any); `policy_seed`:
+    the torch seed of the policy's initialisation, as in build_ppo (default: the config seed)."""
     from .policies import CategoricalActor, GaussianActor
     from .spaces import is_discrete
 
     def policy(cfg, envs, rep, act):
         cls = CategoricalActor if is_discrete(envs.action_space) else GaussianActor
         return cls(envs.action_space, rep, list(cfg.actor_hidden_size), activation=act, device=device)
-    return _build(_PG, env_id, "PG_Agent", policy, device, overrides, agent_class, process_group)
+    return _build(_PG, env_id, "PG_Agent", policy, device, overrides, agent_class, process_group, policy_seed)
 
 
-def build_ppg(env_id, device="cuda", agent_class=None, process_group=None, **overrides):
+def build_ppg(env_id, device="cuda", agent_class=None, process_group=None, policy_seed=None, **overrides):
     """PPG_Agent wired like Runner_DRL does for the ppg yamls (Categorical_PPG / Gaussian_PPG policy).
-    `process_group`: env-sharded training as in build_ppo (default: the initialised default group, if any)."""
+    `process_group`: env-sharded training as in build_ppo (default: the initialised default group, if any); `policy_seed`:
+    the torch seed of the policy's initialisation, as in build_ppo (default: the config seed)."""
     from .policies import CategoricalPPGActorCritic, GaussianPPGActorCritic
     from .spaces import is_discrete
 
@@ -96,4 +99,4 @@ def build_ppg(env_id, device="cuda", agent_class=None, process_group=None, **ove
         cls = CategoricalPPGActorCritic if is_discrete(envs.action_space) else GaussianPPGActorCritic
         return cls(envs.action_space, rep, list(cfg.actor_hidden_size), list(cfg.critic_hidden_size), activation=act,
                    device=device)
-    return _build(_PPG, env_id, "PPG_Agent", policy, device, overrides, agent_class, process_group)
+    return _build(_PPG, env_id, "PPG_Agent", policy, device, overrides, agent_class, process_group, policy_seed)

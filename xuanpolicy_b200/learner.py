@@ -160,6 +160,38 @@ class PPOCLIP_Learner:
         self.policy.load_state_dict(state)
         if self._fused is not None:
             self._fused.splits_fresh = False      # the tf32 operand copies no longer match the weights
+        return path
+
+    # ---------------------------------------------------------------------------------------------- training state
+    def state_tensors(self):
+        """The learner's share of the agent's training state (PPOCLIP_Agent._state_tensors): the fused Adam's flat
+        parameters, moments, step and learning rate, and the log scalars of the last update.  A learner whose torch
+        optimiser steps (no flat state) holds its parameters in the policy: those are listed instead."""
+        fl = self._flat
+        named = {"learner.scalars": self._scalars}
+        if fl is not None:
+            named.update({"learner.flat_param": fl.flat_param, "learner.exp_avg": fl.exp_avg,
+                          "learner.exp_avg_sq": fl.exp_avg_sq, "learner.step": fl.step, "learner.lr": fl.lr})
+        else:
+            named.update(("policy." + k, v) for k, v in self.policy.state_dict().items())
+        return named
+
+    def host_state(self):
+        """Host-side training state: the update counter, and the torch optimiser's and scheduler's state where the torch
+        optimiser is the one that steps."""
+        st = {"iterations": self.iterations}
+        if self._flat is None:
+            st["optimizer"] = self.optimizer.state_dict()
+            if self.scheduler is not None:
+                st["scheduler"] = self.scheduler.state_dict()
+        return st
+
+    def load_host_state(self, st):
+        self.iterations = st["iterations"]
+        if "optimizer" in st:
+            self.optimizer.load_state_dict(st["optimizer"])
+        if "scheduler" in st:
+            self.scheduler.load_state_dict(st["scheduler"])
 
     # ---------------------------------------------------------------------------------------------- loss kernel
     def _loss_backward(self, a_dist, v_pred, act, ret, adv, old_logp, val_old, inv_batch, idx=None, T=0, N=0,
@@ -530,6 +562,9 @@ class PPOKL_Learner(_DistLossLearner):
         self.target_kl = target_kl
         self._kl_coef_dev = torch.ones(1, dtype=torch.float32, device=self.device)
 
+    def state_tensors(self):
+        return dict(super().state_tensors(), **{"learner.kl_coef": self._kl_coef_dev})
+
     @property
     def kl_coef(self):
         return float(self._kl_coef_dev.item())
@@ -581,6 +616,13 @@ class PPG_Learner(_DistLossLearner):
         self._shard = None          # (params, flat gradient in, flat mean out, their per-parameter views) when env-sharded
         if process_group is not None:
             self.enable_sharding(process_group)
+
+    def host_state(self):
+        return dict(super().host_state(), policy_iterations=self.policy_iterations, value_iterations=self.value_iterations)
+
+    def load_host_state(self, st):
+        super().load_host_state(st)
+        self.policy_iterations, self.value_iterations = st["policy_iterations"], st["value_iterations"]
 
     def enable_sharding(self, process_group=None):
         """Switch to env-sharded updates when `process_group` (default: the initialised default group) has W > 1 ranks."""
