@@ -356,6 +356,31 @@ int xb_rollout_step(int env_kind, const float* act_param, const float* logstd, c
                     uint32_t* stat_ticket, double* stat_sums_out, int64_t N, xb_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * One vector step of the evaluation loop in ONE launch.  Replaces the body of PPOCLIP_Agent.test (ppoclip_agent.py:113-165):
+ * `dist.stochastic_sample()`, `envs.step(acts)` with auto-reset (gym_vec_env.py:200-212), `scores.append(infos[i]
+ * ["episode_score"])` for every finished env, and the `obs_rms.update(obs)` of the next loop iteration (:126).
+ *   act_param / logstd  policy outputs as in xb_rollout_step; the action is drawn with Philox keyed by *key (u64 [1]) at
+ *                       counter (env, *step); the launch adds 1 to *step (u64 [1]).  act_tape (nullable): the actions are also
+ *                       written to row *step of [tape_steps][N] (int64, Pendulum float32) while *step < tape_steps.
+ *   state .. ep_score   env state as in xb_env_step; next_obs f32 [N][4] or [N][8] receives the observation the policy acts
+ *                       on next (reset observation for finished envs); trig_cache as in xb_rollout_step.
+ *   scores / count      episode queue fp64 [cap] and its length (int64 [1]): the final ep_score of every env that finished in
+ *                       this step is appended in env order (an ordered multi-CTA compaction, independent of CTA scheduling).
+ *                       cap >= test_episode + N - 1 holds every score the loop can produce.
+ *   test_episode        int64 [1].  Stop rule: a launch that finds *count >= *test_episode changes nothing.
+ *   obs_state           nullable, fp64 [2D+1] (D = floats per obs row): merged IN PLACE with the moments of next_obs when
+ *                       the new count is still below *test_episode (the loop goes round again); obs_state_cand fp64 [2D+1] is
+ *                       the merge's scratch.  obs_dim real floats per row.
+ *   partials fp64 [20 * ceil(N / 32)], workspace u64 [2 + ceil(N / 32)]: scratch, zero-initialised once, reset by every launch.
+ * Physics bit-identical to xb_env_step.
+ * ---------------------------------------------------------------------------------------------------------- */
+int xb_eval_step(int env_kind, const float* act_param, const float* logstd, const uint64_t* key, uint64_t* step, double* state,
+                 uint64_t* rng, int32_t* elapsed, double* ep_score, float* next_obs, double* trig_cache, int max_episode_steps,
+                 void* act_tape, int64_t tape_steps, double* scores, int64_t* count, const int64_t* test_episode, int64_t cap,
+                 double* obs_state, double* obs_state_cand, int obs_dim, double* partials, uint64_t* workspace, int64_t N,
+                 xb_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------------------
  * Dense layers of the policy/value MLP at large batch on the tcgen05 tensor cores with fp32-level accuracy
  * ("3xTF32": x = hi + lo split, three kind::tf32 MMAs per k-step, fp32 accumulation in TMEM; csrc/dense_tc.cu).
  * Replace the cuBLAS SIMT sgemm calls torch issues for Basic_MLP / ActorNet / CriticNet forward

@@ -21,6 +21,8 @@ SIGNATURES = {
     "xb_rollout_step": [_i32, _vp, _vp, _vp, _u64, _vp, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                         _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f32, _vp, _vp, _vp,
                         _vp, _vp, _i32, _f32, _vp, _vp, _vp, _f64, _i32, _vp, _vp, _vp, _i64, _vp],
+    "xb_eval_step": [_i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _vp,
+                     _i32, _vp, _vp, _i64, _vp],
     "xb_sincos_f64": [_vp, _vp, _vp, _i64, _vp],
     "xb_store": [_vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f32, _i32, _i64, _vp],
     "xb_gae": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _f64, _f64, _i32, _i32, _vp],

@@ -39,6 +39,7 @@ from . import dist as xdist
 from .buffer import DummyOnPolicyBuffer
 from .learner import PPOCLIP_Learner
 from .spaces import is_discrete
+from .vec_env import DummyVecEnv_Gym
 
 
 class HostPermutationFeeder:
@@ -85,6 +86,77 @@ class HostPermutationFeeder:
             for f in futures:
                 f.result()
         self.futures.clear()
+
+
+def _mix64(x):
+    """splitmix64's finaliser: a bijection of 64-bit integers that scatters nearby inputs."""
+    m = (1 << 64) - 1
+    x = (x + 0x9E3779B97F4A7C15) & m
+    x = ((x ^ (x >> 30)) * 0xBF58476D1CE4E5B9) & m
+    x = ((x ^ (x >> 27)) * 0x94D049BB133111EB) & m
+    return x ^ (x >> 31)
+
+
+class DeviceEvaluator:
+    """The evaluation loop of `test()` (ppoclip_agent.py:113-165) on the device, for one test-env count N.  It owns the loop's
+    state: env physics and RNG streams, the observation the policy acts on, the observation statistics being merged, and the
+    episode queue (scores, count, step).  One captured graph runs `chunk` vector steps, each the agent's `_policy_forward` and
+    one xb_eval_step launch.  The host replays it and reads the 8-byte queue count after every chunk: one sync per chunk."""
+
+    def __init__(self, agent, envs, cap, chunk, tape_steps=0):
+        N, dev = envs.num_envs, agent.device
+        f64, i64 = dict(dtype=torch.float64, device=dev), dict(dtype=torch.int64, device=dev)
+        self.N, self.chunk, self.tape_steps = N, chunk, tape_steps
+        self.kind, self.max_steps = envs._kind, envs.max_episode_length
+        self.state, self.rng = torch.zeros_like(envs._state), torch.zeros_like(envs._rng)
+        self.elapsed, self.ep_score = torch.zeros_like(envs._elapsed), torch.zeros_like(envs._ep_score)
+        self.x = torch.zeros_like(envs._obs)                            # the observation the policy acts on [N, row]
+        self.xn = torch.zeros_like(envs._obs)                           # its normalised form, where the forward needs one
+        self.trig_cache = torch.full((3, N), float("nan"), **f64)
+        D = envs._obs_row
+        self.stats, self.stats_cand = torch.zeros(2 * D + 1, **f64), torch.zeros(2 * D + 1, **f64)
+        self.scores = torch.zeros(cap, **f64)
+        self.count, self.step, self.key, self.test_episode = (torch.zeros(1, **i64) for _ in range(4))
+        ctas = -(-N // 32)                                              # CTAs of the widest launch (32 envs each)
+        self.partials, self.workspace = torch.zeros(20 * ctas, **f64), torch.zeros(2 + ctas, **i64)
+        self.tape = None
+        if tape_steps:                  # test hook: the sampled actions, row = evaluation step
+            self.tape = torch.zeros((tape_steps, N), dtype=torch.float32 if envs._kind == 1 else torch.int64, device=dev)
+        self.graph = None
+
+    def load(self, envs, key, test_episode):
+        """The reset state of `envs` in, the queue emptied, this evaluation's Philox key and episode target set."""
+        for dst, src in ((self.state, envs._state), (self.rng, envs._rng), (self.elapsed, envs._elapsed),
+                         (self.ep_score, envs._ep_score), (self.x, envs._obs)):
+            dst.copy_(src)
+        self.count.zero_()
+        self.step.zero_()
+        self.key.fill_(key - (1 << 64) if key >= 1 << 63 else key)
+        self.test_episode.fill_(test_episode)
+
+    def steps(self, agent, k):
+        N = self.N
+        stats = self.stats if agent.use_obsnorm else None
+        for _ in range(k):
+            norm = (stats, stats, N, agent.obsnorm_range) if stats is not None else None
+            dist, _ = agent._policy_forward(self.x, norm, xn=self.xn)
+            act_param, logstd = agent._act_params(dist, N)
+            ops.eval_step(self.kind, act_param, logstd, self.key, self.step, self.state, self.rng, self.elapsed, self.ep_score,
+                          self.x, self.trig_cache, self.max_steps, self.scores, self.count, self.test_episode, self.partials,
+                          self.workspace, obs_state=stats, obs_state_cand=self.stats_cand if stats is not None else None,
+                          obs_dim=agent._obs_dim, act_tape=self.tape)
+
+    def capture(self, agent):
+        """Warm up one step on a side stream (lazy module state, library workspaces), then capture `chunk` steps."""
+        s = torch.cuda.Stream(device=agent.device)
+        s.wait_stream(torch.cuda.current_stream(agent.device))
+        with torch.cuda.stream(s):
+            self.steps(agent, 1)
+        torch.cuda.current_stream(agent.device).wait_stream(s)
+        torch.cuda.synchronize(agent.device)
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph):
+            self.steps(agent, self.chunk)
 
 
 class PPOCLIP_Agent:
@@ -214,7 +286,7 @@ class PPOCLIP_Agent:
                                       "(XB_FUSED_STEP / XB_FUSED_NORM on)")
         self._stat_partials = torch.zeros(20 * max(148, N // 32 + 2), **f64)
         self._stat_ticket = torch.zeros(1, dtype=torch.int32, device=dev)
-        self._zero_v = None
+        self._zero_v = {}                  # rows -> the zero value vector of an actor-only policy
         self._chain = False
         self._rollout_graph = None
         self._epoch_graph = None
@@ -222,6 +294,12 @@ class PPOCLIP_Agent:
         self.current_step = 0
         self.current_episode = 0
         self.last_info = {}
+        # test() on native device envs: DeviceEvaluator of the latest test-env count, vector steps per captured chunk, the
+        # number of device evaluations so far (it keys their action sampler) and, for tests, the steps of actions to record
+        self._evaluator = None
+        self._eval_chunk = 32
+        self._eval_index = 0
+        self._eval_tape_steps = 0
         # first observation: whatever the envs currently hold (Runner_Base calls envs.reset() before the agent, runner_basic.py:12)
         self._x[0][:N].copy_(envs._obs)
         self._x[0][N:].copy_(envs._obs)
@@ -253,29 +331,33 @@ class PPOCLIP_Agent:
         return d.get_rank() if (d.is_available() and d.is_initialized()) else 0
 
     # ---------------------------------------------------------------------------------------------- rollout
-    def _policy_forward(self, x, norm=None):
+    def _policy_forward(self, x, norm=None, xn=None):
         """norm = (state_new, state_old, n_new_rows, clip): `x` holds raw observations (fused-statistics path); the
-        one-launch rollout forward normalises them itself, otherwise xb_rms_apply does in front of the MLP."""
+        one-launch rollout forward normalises them itself, otherwise xb_rms_apply does in front of the MLP, into `xn`
+        (default: the rollout's buffer of 2 * n_envs rows)."""
         fused = self.learner._fused
         if fused is not None and x.shape[0] >= fused.MIN_ROWS:     # weights were split at the start of the rollout
             if norm is not None and not fused.fwd_from_obs_ok():
-                x, norm = self._apply_norm(x, norm), None
+                x, norm = self._apply_norm(x, norm, xn), None
             # (`_chain`: the launch before this forward is a rollout step of this loop, which writes no weights — the
             #  forward's set-up and weight loads may then overlap it: programmatic dependent launch, csrc/common.cuh)
             act_out, v = fused.forward_inference(x[:, :self._obs_dim], norm=norm, weights_stable=self._chain)
             return fused.dist_params(act_out), v
         if norm is not None:
-            x = self._apply_norm(x, norm)
+            x = self._apply_norm(x, norm, xn)
         out = self.policy(x[:, :self._obs_dim])       # (outputs, dist, v) | actor-only (outputs, dist) | PPG (outputs, dist, v, aux_v)
         if len(out) < 3:
-            if self._zero_v is None or self._zero_v.shape[0] != x.shape[0]:
-                self._zero_v = torch.zeros(x.shape[0], dtype=torch.float32, device=self.device)
-            return out[1], self._zero_v
+            # one vector per row count: a captured graph keeps reading the one it was captured with
+            zero = self._zero_v.get(x.shape[0])
+            if zero is None:
+                zero = self._zero_v[x.shape[0]] = torch.zeros(x.shape[0], dtype=torch.float32, device=self.device)
+            return out[1], zero
         return out[1], out[2]
 
-    def _apply_norm(self, x, norm):
-        ops.rms_apply(x, self._obs_dim, norm[0], norm[1], norm[2], norm[3], self._xn)
-        return self._xn
+    def _apply_norm(self, x, norm, xn=None):
+        xn = self._xn if xn is None else xn
+        ops.rms_apply(x, self._obs_dim, norm[0], norm[1], norm[2], norm[3], xn)
+        return xn
 
     def _obs_norm_args(self):
         if not self.use_obsnorm:
@@ -294,6 +376,14 @@ class PPOCLIP_Agent:
             logstd = logstd.detach() if logstd is not None else std.log().contiguous()
             ops.sample_gaussian(mu[:N].contiguous(), logstd, self._sample_seed, self._ctr, offset, self._act, self._logp)
 
+    def _act_params(self, dist, N):
+        """(action parameters of rows [0, N), log-std) as the fused step kernels take them: logits, or mu and the log-std."""
+        prm = dist.get_param()
+        if self.discrete:
+            return prm[:N], None
+        logstd = getattr(getattr(self.policy, "actor", None), "logstd", None)
+        return prm[0][:N], (logstd.detach() if logstd is not None else prm[1].log().contiguous())
+
     _NORM_INBOX = 1024      # doubles [1024, 1280) of the comm block's statistics area (the epoch's advantage sums use [0, 2 M))
 
     def _rollout_step(self, t):
@@ -305,13 +395,7 @@ class PPOCLIP_Agent:
             # Leaving only per-CTA partial sums and merging them in the forward's prologue was tried and measured slower, 3.11 vs
             # 2.96 ms per C2 rollout: the reduction then sits in front of the forward's first operand tile)
             dist, v = self._policy_forward(x_cur, self._obs_norm_args())
-            prm = dist.get_param()
-            if self.discrete:
-                act_param, logstd = prm[:N], None
-            else:
-                act_param = prm[0][:N]
-                logstd = getattr(getattr(self.policy, "actor", None), "logstd", None)
-                logstd = logstd.detach() if logstd is not None else prm[1].log().contiguous()
+            act_param, logstd = self._act_params(dist, N)
             stats = dict(partials=self._stat_partials, ticket=self._stat_ticket, gamma=self.gamma,
                          mask_terminal=self._mask_terminal_returns)
             if self.use_obsnorm:
@@ -370,13 +454,7 @@ class PPOCLIP_Agent:
         self._store_extra(t, dist)
         if self._fused_step:
             # sample + env step + store in one launch (csrc/env_classic.cu: rollout_step_kernel)
-            prm = dist.get_param()
-            if self.discrete:
-                act_param, logstd = prm[:N], None
-            else:
-                act_param = prm[0][:N]
-                logstd = getattr(getattr(self.policy, "actor", None), "logstd", None)
-                logstd = logstd.detach() if logstd is not None else prm[1].log().contiguous()
+            act_param, logstd = self._act_params(dist, N)
             ops.rollout_step(env._kind, act_param, logstd, v[:N], self._sample_seed, self._ctr, t, env._state, env._rng,
                              env._elapsed, env._ep_score, x_nxt[N:], x_nxt[:N], env._rew, env._term, env._trunc,
                              env._reset_obs, env._ep_step_out, env._ep_score_out, env.ep_stats, env.max_episode_length,
@@ -743,7 +821,8 @@ class PPOCLIP_Agent:
         mem = self.memory
         return {"t": self._t, "cur": self._cur, "rms_cur": self._rms_cur, "iteration": self._iteration,
                 "current_step": self.current_step, "current_episode": self.current_episode, "memory_ptr": mem.ptr,
-                "memory_size": mem.size, "last_info": self.last_info, "learner": self.learner.host_state()}
+                "memory_size": mem.size, "last_info": self.last_info, "learner": self.learner.host_state(),
+                "eval_index": self._eval_index}
 
     def _load_host_state(self, st):
         self._t, self._cur, self._rms_cur, self._iteration = st["t"], st["cur"], st["rms_cur"], st["iteration"]
@@ -751,6 +830,7 @@ class PPOCLIP_Agent:
         self.memory.ptr, self.memory.size = st["memory_ptr"], st["memory_size"]
         self.last_info = st["last_info"]
         self.learner.load_host_state(st["learner"])
+        self._eval_index = st.get("eval_index", 0)        # absent from checkpoints written before device evaluation
 
     def _checkpoint_meta(self):
         return {"format_version": checkpoint.FORMAT_VERSION, "agent_class": type(self).__name__, "env_id": self.envs.env_id,
@@ -937,14 +1017,22 @@ class PPOCLIP_Agent:
         return torch.clamp((x - mean) / (var.sqrt() + 1e-8), -self.obsnorm_range, self.obsnorm_range).float()
 
     def test(self, env_fn, test_episode):
-        """Evaluation episodes on fresh envs (reference :113-165): stochastic actions, scores of finished episodes."""
+        """Evaluation episodes on fresh envs (reference :113-165): stochastic actions, scores of finished episodes, in (step,
+        env index) order; the loop stops at the first step after which there are at least `test_episode` of them.  With
+        `use_obsnorm`, every observation the policy acts on is merged into the observation statistics first.
+        Native device envs of the training env on this device, on one rank, run the loop on the device (_test_device);
+        any other envs (compat numpy envs, other vec envs, env-sharded runs) run it on the host."""
         envs = env_fn()
         obs, _ = envs.reset()
+        index = lambda d: d.index if d.index is not None else torch.cuda.current_device()
+        if (isinstance(envs, DummyVecEnv_Gym) and envs.native and index(envs.device) == index(self.device)
+                and self.world_size == 1 and envs._kind == self.envs._kind):
+            return self._test_device(envs, int(test_episode))
         scores = []
         with torch.no_grad(), torch.cuda.device(self.device):
             while len(scores) < test_episode:
                 obs = obs if torch.is_tensor(obs) else torch.as_tensor(obs, device=self.device)
-                _, dist, _ = self.policy(self._test_observation(obs))
+                dist = self.policy(self._test_observation(obs))[1]
                 acts = dist.stochastic_sample()
                 obs, _, term, trunc, infos = envs.step(acts if envs.native else acts.cpu().numpy())
                 done = (term | trunc)
@@ -957,6 +1045,47 @@ class PPOCLIP_Agent:
                     for i in np.nonzero(done)[0]:
                         obs[i] = infos[int(i)]["reset_obs"]
         envs.close()
+        return scores
+
+    def _test_device(self, envs, test_episode):
+        """test() on the device: the reset state of `envs` is copied into the DeviceEvaluator of this env count, the first
+        observations are merged into the statistics, and chunks of captured steps run until the episode queue holds
+        `test_episode` scores.  The Philox key of the sampler derives from (seed, evaluation index), not from the training
+        sampler's key or counter; the only training state that changes is the current observation statistics."""
+        if test_episode <= 0:
+            envs.close()
+            return []
+        N = envs.num_envs
+        with torch.no_grad(), torch.cuda.device(self.device):
+            ev = self._evaluator
+            if (ev is None or ev.N != N or ev.scores.numel() < test_episode + N - 1 or ev.chunk != self._eval_chunk
+                    or ev.tape_steps != self._eval_tape_steps):
+                self._evaluator = None           # (its graph and buffers go before the new ones are made)
+                ev = self._evaluator = DeviceEvaluator(self, envs, test_episode + N - 1, self._eval_chunk, self._eval_tape_steps)
+            key = _mix64((self._sample_seed & ((1 << 64) - 1)) ^ _mix64(0xE7A1 + self._eval_index))
+            self._chain = False
+            if self.learner._fused is not None:
+                self.learner._fused.refresh_weights()        # tf32 operand copies of the current weights
+            if self.use_graphs and ev.graph is None:
+                ev.load(envs, key, test_episode)
+                ev.capture(self)
+            ev.load(envs, key, test_episode)
+            envs.close()
+            if self.use_obsnorm:           # `obs_rms.update(obs)` of the first loop iteration
+                ops.rms_update_rows(ev.x, self._obs_dim, self._obs_rms[self._rms_cur], ev.stats, self._stat_partials,
+                                    self._stat_ticket)
+            while True:
+                if ev.graph is not None:
+                    ev.graph.replay()
+                else:
+                    ev.steps(self, ev.chunk)
+                count = int(ev.count.item())
+                if count >= test_episode:
+                    break
+            scores = ev.scores[:count].tolist()
+            if self.use_obsnorm:
+                self._obs_rms[self._rms_cur].copy_(ev.stats)
+        self._eval_index += 1
         return scores
 
 

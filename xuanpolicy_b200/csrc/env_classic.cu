@@ -626,6 +626,210 @@ __global__ void __launch_bounds__(128) rollout_step_kernel(RolloutStepArgs a) {
     if (with_stats) step_stats_finish<D>(a.stats, acc, N, stat_smem, &stat_flag);
 }
 
+// ------------------------------------------------------------------------------------------------ evaluation step
+// One launch per vector step of the evaluation loop (PPOCLIP_Agent.test, ppoclip_agent.py:113-165): sample the action from the
+// policy outputs, step the env with auto-reset, append the scores of the episodes that ended to a queue in env order, and merge
+// the moments of the observations the policy acts on next into the observation statistics (`obs_rms.update(obs)` at the top of
+// the next loop iteration).  Sampling, env functors, trig cache and statistics are those of rollout_step_kernel; nothing is
+// stored for training.
+struct EvalStepArgs {
+    const float* act_param;       // logits [N][A] or mu [N][1]
+    const float* logstd;          // [1] (Gaussian)
+    const uint64_t* key;          // Philox key of this evaluation
+    uint64_t* step;               // evaluation step = the Philox counter's high half; +1 per step that runs
+    double* state;
+    uint64_t* rng;
+    int32_t* elapsed;
+    double* ep_score;
+    float4* next_obs;             // reset-substituted observation the policy acts on next
+    double* trig_cache;
+    int max_steps;
+    void* act_tape;               // nullable: [tape_steps][N] sampled actions, row = evaluation step
+    int64_t tape_steps;
+    double* scores;               // the episode queue, fp64 [cap]
+    int64_t* count;               // entries in the queue
+    const int64_t* test_episode;
+    int64_t cap;
+    uint64_t* ws;                 // [0] start ticket, [1] statistics ticket, [2, 2 + grid) look-back words
+    int64_t N;
+    StepStats stats;              // obs_state_in = the live statistics (nullable), obs_state_out = the merge candidate
+};
+
+__device__ __forceinline__ void st_release_u64(uint64_t* p, uint64_t v) {
+    asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+__device__ __forceinline__ uint64_t ld_acquire_u64(const uint64_t* p) {
+    uint64_t v;
+    asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+    return v;
+}
+
+// look-back word of a CTA: status in the top two bits, a count of finished episodes in the low 32
+constexpr uint64_t kLbAggregate = 1ull << 62, kLbInclusive = 2ull << 62, kLbValue = 0xffffffffull;
+
+template <class Env>
+__global__ void __launch_bounds__(128) eval_step_kernel(EvalStepArgs a) {
+    constexpr int V = Env::kObsVec, D = 4 * V;
+    __shared__ double stat_smem[(2 * D + 3) * 32];
+    __shared__ bool stat_flag;
+    __shared__ int64_t s_c0, s_base;
+    __shared__ uint64_t s_step;
+    __shared__ unsigned s_cta, s_warp[4];
+    __shared__ bool s_active;
+    // The stop rule reads the count the previous step left.  It is written only by this launch's last CTA, after every CTA
+    // has taken its statistics ticket, so every CTA reads the same value.  A launch that finds the queue full changes nothing.
+    if (threadIdx.x == 0) {
+        s_c0 = *a.count;
+        s_active = s_c0 < *a.test_episode;
+        if (s_active) {
+            s_step = *a.step;
+            s_cta = ticket_take((unsigned int*)a.ws);     // CTAs take their place in env order in the order they start
+        }
+    }
+    __syncthreads();
+    if (!s_active) return;
+    const int64_t N = a.N;
+    const unsigned cta = s_cta;
+    const uint64_t step = s_step;
+    const int64_t e = (int64_t)cta * blockDim.x + threadIdx.x;
+    double acc[2 * D + 3];
+#pragma unroll
+    for (int k = 0; k < 2 * D + 3; ++k) acc[k] = 0.0;
+    bool done = false;
+    double final_score = 0.0;
+    if (e < N) {
+        const Philox ph = philox_setup(*a.key, nullptr, step);
+        typename Env::action_t act;
+        float logp;
+        if (Env::kDiscrete) {
+            act = (typename Env::action_t)sample_categorical_one(a.act_param + e * Env::kActions, Env::kActions, e, ph, &logp);
+            if (a.act_tape && (int64_t)step < a.tape_steps) ((int64_t*)a.act_tape)[(int64_t)step * N + e] = (int64_t)act;
+        } else {
+            float x;
+            sample_gaussian_one(a.act_param + e, a.logstd, 1, e, ph, &x);
+            act = (typename Env::action_t)x;
+            if (a.act_tape && (int64_t)step < a.tape_steps) ((float*)a.act_tape)[(int64_t)step * N + e] = x;
+        }
+        // env step: the arithmetic of rollout_step_kernel / env_step_kernel
+        double st[Env::S];
+#pragma unroll
+        for (int k = 0; k < Env::S; ++k) st[k] = a.state[k * N + e];
+        int32_t el = a.elapsed[e];
+        double score = a.ep_score[e];
+        bool terminated;
+        double reward;
+        float4 o[V];
+        double sc_s = 0.0, sc_c = 0.0;
+        if constexpr (Env::kTrigCache) {
+            bool hit = false;
+            if (a.trig_cache && a.trig_cache[e] == st[0]) {
+                sc_s = a.trig_cache[N + e];
+                hit = true;
+            }
+            if (!hit) sincos_cr(st[0], &sc_s, &sc_c);
+            reward = Env::step_sc(st, act, terminated, sc_s);
+            sincos_cr(st[0], &sc_s, &sc_c);
+            o[0] = Env::observe_sc(st, sc_s, sc_c);
+        } else {
+            reward = Env::step(st, act, terminated);
+            observe_row<Env>(st, o);
+        }
+        el += 1;
+        const bool truncated = el >= a.max_steps;
+        score = __dadd_rn(score, reward);
+        done = terminated || truncated;
+        final_score = score;
+        if (done) {
+            Pcg64 g = load_rng<Env>(a.rng, N, e);
+            Env::draw(st, g);
+            a.rng[e] = g.hi;
+            a.rng[N + e] = g.lo;
+            el = 0;
+            score = 0.0;
+            if constexpr (Env::kTrigCache) {
+                sincos_cr(st[0], &sc_s, &sc_c);
+                o[0] = Env::observe_sc(st, sc_s, sc_c);
+            } else {
+                observe_row<Env>(st, o);
+            }
+        }
+        put_row<Env>(a.next_obs, e, o);
+        if constexpr (Env::kTrigCache) {
+            if (a.trig_cache) {
+                a.trig_cache[e] = st[0];
+                a.trig_cache[N + e] = sc_s;
+                a.trig_cache[2 * N + e] = sc_c;
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < Env::S; ++k) a.state[k * N + e] = st[k];
+        a.elapsed[e] = el;
+        a.ep_score[e] = score;
+        if (a.stats.obs_state_in) {
+#pragma unroll
+            for (int v = 0; v < V; ++v) {
+                const float in[4] = {o[v].x, o[v].y, o[v].z, o[v].w};
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    acc[4 * v + k] = (double)in[k];
+                    acc[D + 4 * v + k] = (double)in[k] * (double)in[k];
+                }
+            }
+        }
+    }
+    // ---- ordered compaction of the finished episodes: ballots within the CTA, decoupled look-back across CTAs
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const unsigned m = __ballot_sync(0xffffffffu, done);
+    if (lane == 0) s_warp[warp] = __popc(m);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        uint64_t local = 0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) {
+            const unsigned c = s_warp[w];
+            s_warp[w] = (unsigned)local;
+            local += c;
+        }
+        uint64_t* words = a.ws + 2;
+        uint64_t excl = 0;
+        if (cta == 0) {
+            st_release_u64(words, kLbInclusive | local);
+        } else {
+            st_release_u64(words + cta, kLbAggregate | local);
+            for (int64_t j = (int64_t)cta - 1;;) {
+                const uint64_t f = ld_acquire_u64(words + j);
+                if (f == 0) continue;                       // CTA j has started (its place was taken before ours) but not published
+                excl += f & kLbValue;
+                if (f & kLbInclusive) break;
+                --j;
+            }
+            st_release_u64(words + cta, kLbInclusive | (excl + local));
+        }
+        s_base = s_c0 + (int64_t)excl;
+    }
+    __syncthreads();
+    if (done) {
+        const int64_t pos = s_base + s_warp[warp] + __popc(m & ((1u << lane) - 1u));
+        if (pos < a.cap) a.scores[pos] = final_score;
+    }
+    // ---- statistics (partials in CTA order), then the last CTA publishes the step
+    step_stats_finish_at<D>(a.stats, acc, N, stat_smem, &stat_flag, (int)cta);
+    if (!stat_flag || threadIdx.x >= 32) return;
+    const uint64_t last = ld_acquire_u64(a.ws + 2 + (gridDim.x - 1));
+    const int64_t c1 = s_c0 + (int64_t)(last & kLbValue);
+    // the reference merges the next observations only when its loop goes round again (len(scores) < test_episode)
+    if (a.stats.obs_state_in && c1 < *a.test_episode) {
+        __syncwarp();
+        double* live = const_cast<double*>(a.stats.obs_state_in);
+        if (lane < 2 * D + 1) live[lane] = a.stats.obs_state_out[lane];
+    }
+    for (int64_t i = lane; i < (int64_t)gridDim.x; i += 32) a.ws[2 + i] = 0ull;
+    if (lane == 0) {
+        *a.count = c1;
+        *a.step = step + 1;
+        a.ws[0] = 0ull;
+    }
+}
+
 __global__ void sincos_kernel(const double* __restrict__ x, double* __restrict__ s, double* __restrict__ c, int64_t n) {
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) sincos_cr(x[i], &s[i], &c[i]);
@@ -756,6 +960,36 @@ extern "C" int xb_rollout_step(int env_kind, const float* act_param, const float
     else if (env_kind == XB_ENV_MOUNTAINCAR) XB_CUDA(launch_pdl(rollout_step_kernel<MountainCar>, dim3(grid), dim3(block), 0, s, true, a));
     else if (env_kind == XB_ENV_ACROBOT) XB_CUDA(launch_pdl(rollout_step_kernel<Acrobot>, dim3(grid), dim3(block), 0, s, true, a));
     else if (env_kind == XB_ENV_MOUNTAINCAR_STACK4) XB_CUDA(launch_pdl(rollout_step_kernel<MountainCarStack>, dim3(grid), dim3(block), 0, s, true, a));
+    else return XB_E_UNSUPPORTED;
+    XB_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int xb_eval_step(int env_kind, const float* act_param, const float* logstd, const uint64_t* key, uint64_t* step,
+                            double* state, uint64_t* rng, int32_t* elapsed, double* ep_score, float* next_obs, double* trig_cache,
+                            int max_episode_steps, void* act_tape, int64_t tape_steps, double* scores, int64_t* count,
+                            const int64_t* test_episode, int64_t cap, double* obs_state, double* obs_state_cand, int obs_dim,
+                            double* partials, uint64_t* workspace, int64_t N, xb_stream_t stream) {
+    if (N <= 0 || !act_param || !key || !step || !state || !rng || !elapsed || !ep_score || !next_obs || !scores || !count ||
+        !test_episode || cap < 1 || !partials || !workspace || tape_steps < 0 || (act_tape && tape_steps == 0))
+        return XB_E_BADARG;
+    if (env_kind == XB_ENV_PENDULUM && !logstd) return XB_E_BADARG;
+    if (obs_state && (!obs_state_cand || obs_state == obs_state_cand || obs_dim < 1 || obs_dim > 8)) return XB_E_BADARG;
+    StepStats st{};
+    st.obs_state_in = obs_state;
+    st.obs_state_out = obs_state_cand;
+    st.dim = obs_dim;
+    st.partials = partials;
+    st.ticket = (unsigned int*)(workspace + 1);
+    EvalStepArgs a{act_param, logstd, key, step, state, rng, elapsed, ep_score, (float4*)next_obs, trig_cache, max_episode_steps,
+                   act_tape, tape_steps, scores, count, test_episode, cap, workspace, N, st};
+    cudaStream_t s = (cudaStream_t)stream;
+    int block = env_block(N), grid = ceil_div_i64(N, block);
+    if (env_kind == XB_ENV_CARTPOLE) eval_step_kernel<CartPole><<<grid, block, 0, s>>>(a);
+    else if (env_kind == XB_ENV_PENDULUM) eval_step_kernel<Pendulum><<<grid, block, 0, s>>>(a);
+    else if (env_kind == XB_ENV_MOUNTAINCAR) eval_step_kernel<MountainCar><<<grid, block, 0, s>>>(a);
+    else if (env_kind == XB_ENV_ACROBOT) eval_step_kernel<Acrobot><<<grid, block, 0, s>>>(a);
+    else if (env_kind == XB_ENV_MOUNTAINCAR_STACK4) eval_step_kernel<MountainCarStack><<<grid, block, 0, s>>>(a);
     else return XB_E_UNSUPPORTED;
     XB_LAUNCH_CHECK();
     return 0;

@@ -138,14 +138,15 @@ __device__ __forceinline__ unsigned int ticket_take(unsigned int* ticket) {
 // stores it.  The last CTA's warp 0 loads the per-CTA rows with ALL their loads in flight at once (lane l takes rows l,
 // l + 32, ...; up to 4 rows x K values per lane and pass), transposes the lanes' subtotals through shared memory the same way,
 // and merges: observation dimensions on lanes 0..D-1, the return normaliser on lane 16, side by side.  Every association order
-// depends on the launch geometry only: replays give the same bits.
+// depends on the launch geometry only: replays give the same bits.  `cta`: the partials row of this CTA (its place in the
+// CTA order the last CTA adds in); on return, *flag tells whether this CTA was the last one.
 template <int D>
-__device__ __forceinline__ void step_stats_finish(const StepStats& s, double (&acc)[2 * D + 3], int64_t N, double* smem,
-                                                  bool* flag) {
+__device__ __forceinline__ void step_stats_finish_at(const StepStats& s, double (&acc)[2 * D + 3], int64_t N, double* smem,
+                                                     bool* flag, int cta) {
     constexpr int K = 2 * D + 3;
     constexpr unsigned kFull = 0xffffffffu;
     const int lane = threadIdx.x & 31;
-    double* mine = s.partials + (int64_t)blockIdx.x * kStepStatSlots;
+    double* mine = s.partials + (int64_t)cta * kStepStatSlots;
     if (blockDim.x == 32) {
 #pragma unroll
         for (int k = 0; k < K; ++k) smem[k * 32 + lane] = acc[k];
@@ -252,6 +253,11 @@ __device__ __forceinline__ void step_stats_finish(const StepStats& s, double (&a
     XB_STEP_STAMP(s.ts, 107);
     if (lane == 0) *s.ticket = 0u;
     XB_STEP_STAMP(s.ts, 103);
+}
+template <int D>
+__device__ __forceinline__ void step_stats_finish(const StepStats& s, double (&acc)[2 * D + 3], int64_t N, double* smem,
+                                                  bool* flag) {
+    step_stats_finish_at<D>(s, acc, N, smem, flag, blockIdx.x);
 }
 
 }  // namespace xb

@@ -67,6 +67,17 @@ def rollout_step(kind, act_param, logstd, val, seed, counter, offset, state, rng
               _p(st.get("ticket"), I32), _p(st.get("sums_out"), F64), N, _stream())
 
 
+def eval_step(kind, act_param, logstd, key, step, state, rng, elapsed, ep_score, next_obs, trig_cache, max_steps, scores, count,
+              test_episode, partials, workspace, obs_state=None, obs_state_cand=None, obs_dim=0, act_tape=None):
+    """Sample + env step + episode queue + observation statistics of one evaluation step in one launch (xb_eval_step)."""
+    N = elapsed.numel()
+    _lib.call("xb_eval_step", kind, _p(act_param, F32), _p(logstd, F32), _p(key, I64), _p(step, I64), _p(state, F64),
+              _p(rng, I64), _p(elapsed, I32), _p(ep_score, F64), _p(next_obs, F32), _p(trig_cache, F64), max_steps,
+              _p(act_tape, F32 if kind == 1 else I64), act_tape.shape[0] if act_tape is not None else 0, _p(scores, F64),
+              _p(count, I64), _p(test_episode, I64), scores.numel(), _p(obs_state, F64), _p(obs_state_cand, F64), int(obs_dim),
+              _p(partials, F64), _p(workspace, I64), N, _stream())
+
+
 def sincos_f64(x):
     s, c = torch.empty_like(x), torch.empty_like(x)
     _lib.call("xb_sincos_f64", _p(x, F64), _p(s, F64), _p(c, F64), x.numel(), _stream())
