@@ -372,13 +372,20 @@ int xb_rollout_step(int env_kind, const float* act_param, const float* logstd, c
  *                       the new count is still below *test_episode (the loop goes round again); obs_state_cand fp64 [2D+1] is
  *                       the merge's scratch.  obs_dim real floats per row.
  *   partials fp64 [20 * ceil(N / 32)], workspace u64 [2 + ceil(N / 32)]: scratch, zero-initialised once, reset by every launch.
+ *   local_count / score_step / record  all NULL, or all set for the ENV-SHARDED form (these N envs are one rank's shard of a
+ *                       global vector env): the scores are appended to this rank's queue at *local_count (int64 [1]) instead,
+ *                       score_step (int32 [cap]) receives the evaluation step of each, and *count (the GLOBAL count, read by
+ *                       the stop rule only) and obs_state are left alone: the last CTA writes this rank's step record to
+ *                       record (fp64 [2D+4], the layout of xb_rollout_step's stat_sums_out: sum x[D], sum x^2[D], N, 0, 0,
+ *                       number of envs that finished in this step).  obs_state (nullable, obs_state_cand unused) then only
+ *                       asks for the moments.  xb_peer_eval_merge completes the step.
  * Physics bit-identical to xb_env_step.
  * ---------------------------------------------------------------------------------------------------------- */
 int xb_eval_step(int env_kind, const float* act_param, const float* logstd, const uint64_t* key, uint64_t* step, double* state,
                  uint64_t* rng, int32_t* elapsed, double* ep_score, float* next_obs, double* trig_cache, int max_episode_steps,
                  void* act_tape, int64_t tape_steps, double* scores, int64_t* count, const int64_t* test_episode, int64_t cap,
-                 double* obs_state, double* obs_state_cand, int obs_dim, double* partials, uint64_t* workspace, int64_t N,
-                 xb_stream_t stream);
+                 double* obs_state, double* obs_state_cand, int obs_dim, double* partials, uint64_t* workspace,
+                 int64_t* local_count, int32_t* score_step, double* record, int64_t N, xb_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * Dense layers of the policy/value MLP at large batch on the tcgen05 tensor cores with fp32-level accuracy
@@ -621,6 +628,17 @@ int xb_peer_allreduce_f64(const void* const* peer_bases /* host [W] */, int rank
 int xb_peer_allreduce_merge(const void* const* peer_bases, int rank, int W, const double* src, int n, int inbox_offset,
                             double* out, uint32_t* tickets, const double* obs_state_in, double* obs_state_out, int dim,
                             double* ret_state, float* rew_std, xb_stream_t stream);
+/*   xb_peer_eval_merge        completes one step of the env-sharded evaluation loop after the sharded xb_eval_step: if
+ *                             *count (int64, the GLOBAL episode count) < *test_episode, every rank pushes its step record
+ *                             (n = 2D + 4 = 12 or 20 doubles) into the inbox of xb_peer_allreduce_merge, ONE barrier, the W
+ *                             records are summed in rank order into totals (fp64 [n]), *count += the finishers of all ranks, and when the new count is
+ *                             still below *test_episode, obs_state (nullable, fp64 [2D+1], dim <= D) is merged in place with the
+ *                             global moments (obs_state_cand: scratch, a different buffer), with the bits of xb_eval_step's own
+ *                             merge on one rank.  A launch that finds the target met returns at once: no push, no barrier.
+ *                             Shares the flag slot and the inbox of xb_peer_allreduce_merge (never interleaved with a rollout). */
+int xb_peer_eval_merge(const void* const* peer_bases, int rank, int W, const double* record, int n, int inbox_offset,
+                       double* totals, int64_t* count, const int64_t* test_episode, double* obs_state, double* obs_state_cand, int dim,
+                       uint32_t* tickets, xb_stream_t stream);
 int xb_adv_stats_minibatches(const int64_t* idx, int64_t n_minibatches, int64_t B, int64_t T, int64_t N, const float* adv,
                              int64_t stride, double* stats, xb_stream_t stream);
 

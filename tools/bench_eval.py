@@ -1,7 +1,12 @@
-"""Times `test()` (evaluation episodes) on one GPU: native device envs (the device evaluation loop) against compat numpy envs
-of the same size (the host loop), for CartPole-v1 and Pendulum-v1 at N test envs with test_episode = N.
+"""Times `test()` (evaluation episodes): native device envs (the device evaluation loop) against compat numpy envs of the same
+size (the host loop), for CartPole-v1 and Pendulum-v1 at N test envs with test_episode = N.
 
     python tools/bench_eval.py [--n 16 1024 8192 65536] [--envs CartPole-v1 Pendulum-v1] [--out FILE]
+    python -m torch.distributed.run --nproc-per-node W tools/bench_eval.py [...]
+
+Under torch.distributed.run each --n is the TOTAL env count, split evenly over the W ranks: the device path is the env-sharded
+evaluation (one loop over all ranks' envs, exchanged over peer memory), the host path runs each rank's loop on its own envs to
+test_episode = N, which is what an env-sharded run without the device path does.  Rank 0 prints the lines, with `world_size`.
 
 Each path gets one warm-up call, then one timed call: a host clock around the call, which ends with the scores on the host
 (the device path synchronises before it returns them).  A third call under torch.profiler counts what one call issues: device
@@ -20,25 +25,25 @@ REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, REPO)
 
 
-def card():
+def card(index=0):
     try:
-        out = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit", "--format=csv,noheader"],
+        out = subprocess.run(["nvidia-smi", "-i", str(index), "--query-gpu=name,power.limit", "--format=csv,noheader"],
                              capture_output=True, text=True, check=True).stdout
         name, limit = [x.strip() for x in out.split(",")[:2]]
         return {"name": name, "power_limit": limit}
     except Exception as e:      # noqa: BLE001 - the card name from torch is still worth printing
-        return {"name": torch.cuda.get_device_name(0), "power_limit": "unknown (%s)" % type(e).__name__}
+        return {"name": torch.cuda.get_device_name(index), "power_limit": "unknown (%s)" % type(e).__name__}
 
 
 class CountingEnvFn:
     """env_fn that also counts the vector steps taken on the envs it makes (the host loop's steps)."""
 
-    def __init__(self, env_id, n, native):
-        self.env_id, self.n, self.native, self.steps = env_id, n, native, 0
+    def __init__(self, env_id, n, native, device="cuda"):
+        self.env_id, self.n, self.native, self.device, self.steps = env_id, n, native, device, 0
 
     def __call__(self):
         import xuanpolicy_b200 as xb
-        envs = xb.DummyVecEnv_Gym(xb.make_env_fns(self.env_id, 11, self.n), device="cuda", native=self.native)
+        envs = xb.DummyVecEnv_Gym(xb.make_env_fns(self.env_id, 11, self.n), device=self.device, native=self.native)
         step = envs.step
 
         def counted(actions):
@@ -64,10 +69,13 @@ def profile_call(agent, env_fn, test_episode):
     return d2h, launches
 
 
-def run_path(agent, env_id, n, native):
-    fn = CountingEnvFn(env_id, n, native)
+def run_path(agent, env_id, n, native, world=1):
+    """n: the total env count, n // world on this rank."""
+    fn = CountingEnvFn(env_id, n // world, native, agent.device)
     agent.test(fn, n)                                           # warm-up (the device path captures its chunk graph here)
     torch.cuda.synchronize()
+    if world > 1:
+        torch.distributed.barrier()
     fn.steps = 0
     t0 = time.perf_counter()
     scores = agent.test(fn, n)
@@ -88,26 +96,34 @@ def main():
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("bench_eval.py measures on a CUDA device; none is available")
+    from xuanpolicy_b200 import dist as xd
     from xuanpolicy_b200.configs import build_ppo
     from xuanpolicy_b200.fused_mlp import FusedActorCritic
-    gpu = card()
-    torch.cuda.set_device(0)
+    rank, local, world = xd.init_from_env("nccl")
+    gpu = card(local)
+    torch.cuda.set_device(local)
     for env_id in args.envs:
         for n in args.n:
-            agent = build_ppo(env_id, parallels=64, n_steps=16, n_epoch=1, n_minibatch=1, seed=1)
+            xd.shard_envs(n, world, rank)                       # refuses an N that does not split evenly
+            agent = build_ppo(env_id, parallels=64, n_steps=16, n_epoch=1, n_minibatch=1, seed=1, device="cuda:%d" % local)
             with torch.no_grad():
-                dev = run_path(agent, env_id, n, native=True)
-                host = run_path(agent, env_id, n, native=False)
+                dev = run_path(agent, env_id, n, native=True, world=world)
+                host = run_path(agent, env_id, n, native=False, world=world)
             line = {"bench": "eval", "env_id": env_id, "n_envs": n, "test_episode": n, "chunk": agent._eval_chunk,
-                    "forward": "tcgen05" if n >= FusedActorCritic.MIN_ROWS and agent.learner._fused is not None else "torch",
+                    "forward": "tcgen05" if n // world >= FusedActorCritic.MIN_ROWS and agent.learner._fused is not None else "torch",
                     "device": dev, "host": host, "speedup": round(host["wall_s"] / dev["wall_s"], 2),
                     "gpu": gpu["name"], "power_limit": gpu["power_limit"]}
-            print(json.dumps(line), flush=True)
-            if args.out:
+            if world > 1:
+                line["world_size"] = world
+            if rank == 0:
+                print(json.dumps(line), flush=True)
+            if args.out and rank == 0:
                 with open(args.out, "a") as f:
                     f.write(json.dumps(line) + "\n")
             del agent
             torch.cuda.empty_cache()
+    if world > 1:
+        torch.distributed.destroy_process_group()
 
 
 if __name__ == "__main__":

@@ -22,7 +22,7 @@ SIGNATURES = {
                         _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f32, _vp, _vp, _vp,
                         _vp, _vp, _i32, _f32, _vp, _vp, _vp, _f64, _i32, _vp, _vp, _vp, _i64, _vp],
     "xb_eval_step": [_i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _vp,
-                     _i32, _vp, _vp, _i64, _vp],
+                     _i32, _vp, _vp, _vp, _vp, _vp, _i64, _vp],
     "xb_sincos_f64": [_vp, _vp, _vp, _i64, _vp],
     "xb_store": [_vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f32, _i32, _i64, _vp],
     "xb_gae": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _f64, _f64, _i32, _i32, _vp],
@@ -105,6 +105,7 @@ SIGNATURES = {
     "xb_peer_allreduce_mean": [_vp, _i32, _i32, _i64, _vp, _vp, _vp, _vp],
     "xb_peer_allreduce_f64": [_vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp],
     "xb_peer_allreduce_merge": [_vp, _i32, _i32, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp],
+    "xb_peer_eval_merge": [_vp, _i32, _i32, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp],
     "xb_adv_stats_minibatches": [_vp, _i64, _i64, _i64, _i64, _vp, _i64, _vp, _vp],
     "xb_clip_adam_step": [_vp, _vp, _vp, _vp, _i64, _vp, _f32, _f32, _i64, _f32, _f32, _f32, _f32, _f32, _vp, _vp, _vp, _vp],
 }

@@ -97,16 +97,54 @@ def _mix64(x):
     return x ^ (x >> 31)
 
 
+def agree_eval_plan(plans):
+    """The host check at the start of an env-sharded `test()`: `plans` holds one (device path, env count, env kind, test_episode)
+    row per rank.  Returns True when every rank takes the device path with the same env count, env kind and episode target,
+    False when no rank takes it (each rank then runs the host loop on its own envs), and raises ValueError otherwise, on every
+    rank alike, before any rank reaches a cross-GPU barrier."""
+    rows = [tuple(int(v) for v in p) for p in plans]
+    device = [r for r, p in enumerate(rows) if p[0]]
+    if not device:
+        return False
+    if len(device) < len(rows):
+        raise ValueError("test(): ranks %s would run the device evaluation loop and ranks %s the host loop; every rank must "
+                         "pass native device envs of the training env" % (device, [r for r in range(len(rows)) if r not in device]))
+    for k, what in ((1, "test env counts"), (2, "env kinds"), (3, "test_episode values")):
+        values = [p[k] for p in rows]
+        if len(set(values)) > 1:
+            raise ValueError("test(): the ranks' %s differ (%s); the env-sharded evaluation needs the same on every rank"
+                             % (what, values))
+    return True
+
+
+def order_eval_scores(scores, steps):
+    """The scores of an env-sharded evaluation in the order of the reference's loop over the global vector env, whose env
+    r * n + e is env e of rank r: by step, then rank, then env.  scores[r] / steps[r]: rank r's episode queue and the step each
+    score finished in (already in (step, env) order).  Returns a list of floats."""
+    if len(scores) != len(steps) or any(len(a) != len(b) for a, b in zip(scores, steps)):
+        raise ValueError("every rank needs one step tag per score")
+    for t in steps:
+        if np.any(np.diff(np.asarray(t, dtype=np.int64)) < 0):
+            raise ValueError("a rank's episode queue is not in step order")
+    flat = np.concatenate([np.asarray(s, dtype=np.float64) for s in scores]) if scores else np.zeros(0)
+    step = np.concatenate([np.asarray(t, dtype=np.int64) for t in steps]) if steps else np.zeros(0, np.int64)
+    rank = np.concatenate([np.full(len(s), r, np.int64) for r, s in enumerate(scores)]) if scores else np.zeros(0, np.int64)
+    return flat[np.lexsort((rank, step))].tolist()         # a stable sort: each rank's env order is kept
+
+
 class DeviceEvaluator:
     """The evaluation loop of `test()` (ppoclip_agent.py:113-165) on the device, for one test-env count N.  It owns the loop's
     state: env physics and RNG streams, the observation the policy acts on, the observation statistics being merged, and the
     episode queue (scores, count, step).  One captured graph runs `chunk` vector steps, each the agent's `_policy_forward` and
-    one xb_eval_step launch.  The host replays it and reads the 8-byte queue count after every chunk: one sync per chunk."""
+    one xb_eval_step launch.  The host replays it and reads the 8-byte queue count after every chunk: one sync per chunk.
+    With a peer comm block (`peer`), the N envs are this rank's shard of a global vector env: each step is followed by the
+    xb_peer_eval_merge exchange, `count` is the global episode count and the scores, tagged with their steps, go to a local
+    queue of `local_count` entries."""
 
-    def __init__(self, agent, envs, cap, chunk, tape_steps=0):
+    def __init__(self, agent, envs, cap, chunk, tape_steps=0, peer=None):
         N, dev = envs.num_envs, agent.device
         f64, i64 = dict(dtype=torch.float64, device=dev), dict(dtype=torch.int64, device=dev)
-        self.N, self.chunk, self.tape_steps = N, chunk, tape_steps
+        self.N, self.chunk, self.tape_steps, self.peer = N, chunk, tape_steps, peer
         self.kind, self.max_steps = envs._kind, envs.max_episode_length
         self.state, self.rng = torch.zeros_like(envs._state), torch.zeros_like(envs._rng)
         self.elapsed, self.ep_score = torch.zeros_like(envs._elapsed), torch.zeros_like(envs._ep_score)
@@ -122,6 +160,12 @@ class DeviceEvaluator:
         self.tape = None
         if tape_steps:                  # test hook: the sampled actions, row = evaluation step
             self.tape = torch.zeros((tape_steps, N), dtype=torch.float32 if envs._kind == 1 else torch.int64, device=dev)
+        self.local_count = self.score_step = self.record = None
+        if peer is not None:
+            self.local_count = torch.zeros(1, **i64)
+            self.score_step = torch.zeros(cap, dtype=torch.int32, device=dev)
+            self.record = torch.zeros(2 * D + 4, **f64)      # this rank's step record: sum x[D], sum x^2[D], N, 0, 0, finishers
+            self.totals = torch.zeros(2 * D + 4, **f64)      # the global moments of the first / the latest observations
         self.graph = None
 
     def load(self, envs, key, test_episode):
@@ -131,6 +175,8 @@ class DeviceEvaluator:
             dst.copy_(src)
         self.count.zero_()
         self.step.zero_()
+        if self.local_count is not None:
+            self.local_count.zero_()
         self.key.fill_(key - (1 << 64) if key >= 1 << 63 else key)
         self.test_episode.fill_(test_episode)
 
@@ -144,7 +190,11 @@ class DeviceEvaluator:
             ops.eval_step(self.kind, act_param, logstd, self.key, self.step, self.state, self.rng, self.elapsed, self.ep_score,
                           self.x, self.trig_cache, self.max_steps, self.scores, self.count, self.test_episode, self.partials,
                           self.workspace, obs_state=stats, obs_state_cand=self.stats_cand if stats is not None else None,
-                          obs_dim=agent._obs_dim, act_tape=self.tape)
+                          obs_dim=agent._obs_dim, act_tape=self.tape, local_count=self.local_count, score_step=self.score_step,
+                          record=self.record)
+            if self.peer is not None:
+                ops.peer_eval_merge(self.peer, self.record, self.totals, self.count, self.test_episode, agent._NORM_INBOX, obs_state=stats,
+                                    obs_state_cand=self.stats_cand if stats is not None else None, obs_dim=agent._obs_dim)
 
     def capture(self, agent):
         """Warm up one step on a side stream (lazy module state, library workspaces), then capture `chunk` steps."""
@@ -300,6 +350,8 @@ class PPOCLIP_Agent:
         self._eval_chunk = 32
         self._eval_index = 0
         self._eval_tape_steps = 0
+        # the comm block of the env-sharded device evaluation (None: one rank, the plain device loop)
+        self._eval_peer = self.learner._peer if self.world_size > 1 else None
         # first observation: whatever the envs currently hold (Runner_Base calls envs.reset() before the agent, runner_basic.py:12)
         self._x[0][:N].copy_(envs._obs)
         self._x[0][N:].copy_(envs._obs)
@@ -1020,13 +1072,28 @@ class PPOCLIP_Agent:
         """Evaluation episodes on fresh envs (reference :113-165): stochastic actions, scores of finished episodes, in (step,
         env index) order; the loop stops at the first step after which there are at least `test_episode` of them.  With
         `use_obsnorm`, every observation the policy acts on is merged into the observation statistics first.
-        Native device envs of the training env on this device, on one rank, run the loop on the device (_test_device);
-        any other envs (compat numpy envs, other vec envs, env-sharded runs) run it on the host."""
+        Native device envs of the training env on this device run the loop on the device (_test_device).  Env-sharded, every
+        rank calls test() together and `env_fn()` returns the rank's shard of the test envs: the W ranks' envs form one vector
+        env (env r * n + e = env e of rank r), the stop rule counts the episodes of all ranks, the statistics merge the
+        observations of all ranks, and every rank returns the same scores in (step, rank, env) order; this needs the peer
+        memory exchange (`_eval_peer`).  Any other envs (compat numpy envs, other vec envs, no peer memory) run the loop on the
+        host, each rank on its own envs."""
         envs = env_fn()
         obs, _ = envs.reset()
         index = lambda d: d.index if d.index is not None else torch.cuda.current_device()
-        if (isinstance(envs, DummyVecEnv_Gym) and envs.native and index(envs.device) == index(self.device)
-                and self.world_size == 1 and envs._kind == self.envs._kind):
+        device = (isinstance(envs, DummyVecEnv_Gym) and envs.native and index(envs.device) == index(self.device)
+                  and envs._kind == self.envs._kind and (self.world_size == 1 or self._eval_peer is not None))
+        if self.world_size > 1:
+            plan = torch.tensor([int(device), envs.num_envs if device else 0, envs._kind if device else -1, int(test_episode)],
+                                dtype=torch.int64, device=self.device)
+            plans = torch.empty((self.world_size, 4), dtype=torch.int64, device=self.device)
+            torch.distributed.all_gather_into_tensor(plans, plan, group=self.learner.process_group)
+            try:
+                device = agree_eval_plan(plans.cpu().tolist())
+            except ValueError:
+                envs.close()
+                raise
+        if device:
             return self._test_device(envs, int(test_episode))
         scores = []
         with torch.no_grad(), torch.cuda.device(self.device):
@@ -1055,13 +1122,14 @@ class PPOCLIP_Agent:
         if test_episode <= 0:
             envs.close()
             return []
-        N = envs.num_envs
+        N, peer = envs.num_envs, self._eval_peer
         with torch.no_grad(), torch.cuda.device(self.device):
             ev = self._evaluator
             if (ev is None or ev.N != N or ev.scores.numel() < test_episode + N - 1 or ev.chunk != self._eval_chunk
-                    or ev.tape_steps != self._eval_tape_steps):
+                    or ev.tape_steps != self._eval_tape_steps or ev.peer is not peer):
                 self._evaluator = None           # (its graph and buffers go before the new ones are made)
-                ev = self._evaluator = DeviceEvaluator(self, envs, test_episode + N - 1, self._eval_chunk, self._eval_tape_steps)
+                ev = self._evaluator = DeviceEvaluator(self, envs, test_episode + N - 1, self._eval_chunk, self._eval_tape_steps,
+                                                       peer)
             key = _mix64((self._sample_seed & ((1 << 64) - 1)) ^ _mix64(0xE7A1 + self._eval_index))
             self._chain = False
             if self.learner._fused is not None:
@@ -1071,22 +1139,45 @@ class PPOCLIP_Agent:
                 ev.capture(self)
             ev.load(envs, key, test_episode)
             envs.close()
-            if self.use_obsnorm:           # `obs_rms.update(obs)` of the first loop iteration
+            if self.use_obsnorm and peer is None:           # `obs_rms.update(obs)` of the first loop iteration
                 ops.rms_update_rows(ev.x, self._obs_dim, self._obs_rms[self._rms_cur], ev.stats, self._stat_partials,
                                     self._stat_ticket)
+            elif self.use_obsnorm:         # ... over the observations of every rank (the exchange of __init__)
+                m = 2 * self.memory.obs_row + 1
+                off = peer.stats.numel() - ev.record.numel()
+                ops.moments4(ev.x, peer.stats[off:off + m], self._obs_ws)
+                ops.peer_allreduce_f64(peer, m, ev.totals[:m], offset=off)
+                ops.rms_merge_sums(ev.totals, self._obs_rms[self._rms_cur], ev.stats, self._obs_dim, None, None)
             while True:
                 if ev.graph is not None:
                     ev.graph.replay()
                 else:
                     ev.steps(self, ev.chunk)
                 count = int(ev.count.item())
+                if peer is not None:
+                    peer.check()
                 if count >= test_episode:
                     break
-            scores = ev.scores[:count].tolist()
+            scores = ev.scores[:count].tolist() if peer is None else self._gather_eval_scores(ev, test_episode + N - 1, count)
             if self.use_obsnorm:
                 self._obs_rms[self._rms_cur].copy_(ev.stats)
         self._eval_index += 1
         return scores
+
+    def _gather_eval_scores(self, ev, cap, count):
+        """Every rank's queue (local count, scores, step tags) in one all_gather and one device -> host copy, in (step, rank,
+        env) order."""
+        mine = torch.cat([ev.local_count.double(), ev.scores[:cap], ev.score_step[:cap].double()])
+        if self.world_size > 1:
+            rows = torch.empty((self.world_size, mine.numel()), dtype=torch.float64, device=self.device)
+            torch.distributed.all_gather_into_tensor(rows, mine, group=self.learner.process_group)
+        else:
+            rows = mine[None]
+        rows = rows.cpu().numpy()
+        k = rows[:, 0].astype(np.int64)
+        if int(k.sum()) != count:
+            raise RuntimeError("env-sharded test(): the ranks' queues hold %d scores, the global count is %d" % (k.sum(), count))
+        return order_eval_scores([r[1:1 + n] for r, n in zip(rows, k)], [r[1 + cap:1 + cap + n] for r, n in zip(rows, k)])
 
 
 class A2C_Agent(PPOCLIP_Agent):

@@ -632,6 +632,10 @@ __global__ void __launch_bounds__(128) rollout_step_kernel(RolloutStepArgs a) {
 // the moments of the observations the policy acts on next into the observation statistics (`obs_rms.update(obs)` at the top of
 // the next loop iteration).  Sampling, env functors, trig cache and statistics are those of rollout_step_kernel; nothing is
 // stored for training.
+// Env-sharded form (local_count != nullptr): this rank's envs are one shard of a global vector env.  The scores go to a LOCAL
+// queue at *local_count, each tagged with its step, and the last CTA neither merges nor touches the global *count: it writes
+// this rank's step record to stats.sums_out instead (the StepStats::sums_out layout, with the number of envs that finished in
+// the n-finished slot), which xb_peer_eval_merge exchanges.  The stop rule still reads the global count.
 struct EvalStepArgs {
     const float* act_param;       // logits [N][A] or mu [N][1]
     const float* logstd;          // [1] (Gaussian)
@@ -653,6 +657,8 @@ struct EvalStepArgs {
     uint64_t* ws;                 // [0] start ticket, [1] statistics ticket, [2, 2 + grid) look-back words
     int64_t N;
     StepStats stats;              // obs_state_in = the live statistics (nullable), obs_state_out = the merge candidate
+    int64_t* local_count;         // sharded form (nullable): entries in this rank's queue
+    int32_t* score_step;          // sharded form: the evaluation step of every queued score [cap]
 };
 
 __device__ __forceinline__ void st_release_u64(uint64_t* p, uint64_t v) {
@@ -672,7 +678,7 @@ __global__ void __launch_bounds__(128) eval_step_kernel(EvalStepArgs a) {
     constexpr int V = Env::kObsVec, D = 4 * V;
     __shared__ double stat_smem[(2 * D + 3) * 32];
     __shared__ bool stat_flag;
-    __shared__ int64_t s_c0, s_base;
+    __shared__ int64_t s_c0, s_q0, s_base;
     __shared__ uint64_t s_step;
     __shared__ unsigned s_cta, s_warp[4];
     __shared__ bool s_active;
@@ -682,6 +688,7 @@ __global__ void __launch_bounds__(128) eval_step_kernel(EvalStepArgs a) {
         s_c0 = *a.count;
         s_active = s_c0 < *a.test_episode;
         if (s_active) {
+            s_q0 = a.local_count ? *a.local_count : s_c0;     // where this step's scores go in the queue
             s_step = *a.step;
             s_cta = ticket_take((unsigned int*)a.ws);     // CTAs take their place in env order in the order they start
         }
@@ -804,27 +811,31 @@ __global__ void __launch_bounds__(128) eval_step_kernel(EvalStepArgs a) {
             }
             st_release_u64(words + cta, kLbInclusive | (excl + local));
         }
-        s_base = s_c0 + (int64_t)excl;
+        s_base = s_q0 + (int64_t)excl;
     }
     __syncthreads();
     if (done) {
         const int64_t pos = s_base + s_warp[warp] + __popc(m & ((1u << lane) - 1u));
-        if (pos < a.cap) a.scores[pos] = final_score;
+        if (pos < a.cap) {
+            a.scores[pos] = final_score;
+            if (a.score_step) a.score_step[pos] = (int32_t)step;
+        }
     }
+    acc[2 * D + 2] = done ? 1.0 : 0.0;      // the record's n-finished slot (sharded form); no return normaliser reads it here
     // ---- statistics (partials in CTA order), then the last CTA publishes the step
     step_stats_finish_at<D>(a.stats, acc, N, stat_smem, &stat_flag, (int)cta);
     if (!stat_flag || threadIdx.x >= 32) return;
     const uint64_t last = ld_acquire_u64(a.ws + 2 + (gridDim.x - 1));
-    const int64_t c1 = s_c0 + (int64_t)(last & kLbValue);
+    const int64_t c1 = s_q0 + (int64_t)(last & kLbValue);
     // the reference merges the next observations only when its loop goes round again (len(scores) < test_episode)
-    if (a.stats.obs_state_in && c1 < *a.test_episode) {
+    if (!a.local_count && a.stats.obs_state_in && c1 < *a.test_episode) {
         __syncwarp();
         double* live = const_cast<double*>(a.stats.obs_state_in);
         if (lane < 2 * D + 1) live[lane] = a.stats.obs_state_out[lane];
     }
     for (int64_t i = lane; i < (int64_t)gridDim.x; i += 32) a.ws[2 + i] = 0ull;
     if (lane == 0) {
-        *a.count = c1;
+        *(a.local_count ? a.local_count : a.count) = c1;
         *a.step = step + 1;
         a.ws[0] = 0ull;
     }
@@ -969,20 +980,24 @@ extern "C" int xb_eval_step(int env_kind, const float* act_param, const float* l
                             double* state, uint64_t* rng, int32_t* elapsed, double* ep_score, float* next_obs, double* trig_cache,
                             int max_episode_steps, void* act_tape, int64_t tape_steps, double* scores, int64_t* count,
                             const int64_t* test_episode, int64_t cap, double* obs_state, double* obs_state_cand, int obs_dim,
-                            double* partials, uint64_t* workspace, int64_t N, xb_stream_t stream) {
+                            double* partials, uint64_t* workspace, int64_t* local_count, int32_t* score_step, double* record,
+                            int64_t N, xb_stream_t stream) {
     if (N <= 0 || !act_param || !key || !step || !state || !rng || !elapsed || !ep_score || !next_obs || !scores || !count ||
         !test_episode || cap < 1 || !partials || !workspace || tape_steps < 0 || (act_tape && tape_steps == 0))
         return XB_E_BADARG;
     if (env_kind == XB_ENV_PENDULUM && !logstd) return XB_E_BADARG;
-    if (obs_state && (!obs_state_cand || obs_state == obs_state_cand || obs_dim < 1 || obs_dim > 8)) return XB_E_BADARG;
+    if ((local_count != nullptr) != (score_step != nullptr) || (local_count != nullptr) != (record != nullptr)) return XB_E_BADARG;
+    if (obs_state && (obs_dim < 1 || obs_dim > 8)) return XB_E_BADARG;
+    if (obs_state && !record && (!obs_state_cand || obs_state == obs_state_cand)) return XB_E_BADARG;     // the merge's scratch
     StepStats st{};
     st.obs_state_in = obs_state;
     st.obs_state_out = obs_state_cand;
     st.dim = obs_dim;
     st.partials = partials;
     st.ticket = (unsigned int*)(workspace + 1);
+    st.sums_out = record;
     EvalStepArgs a{act_param, logstd, key, step, state, rng, elapsed, ep_score, (float4*)next_obs, trig_cache, max_episode_steps,
-                   act_tape, tape_steps, scores, count, test_episode, cap, workspace, N, st};
+                   act_tape, tape_steps, scores, count, test_episode, cap, workspace, N, st, local_count, score_step};
     cudaStream_t s = (cudaStream_t)stream;
     int block = env_block(N), grid = ceil_div_i64(N, block);
     if (env_kind == XB_ENV_CARTPOLE) eval_step_kernel<CartPole><<<grid, block, 0, s>>>(a);

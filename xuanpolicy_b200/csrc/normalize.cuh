@@ -111,6 +111,30 @@ __device__ __forceinline__ void merge_step_sums(const double* sums, int D, const
                             sums[11], tid);
 }
 
+// The observation merge of merge_step_sums (thread tid < D: dimension tid) with every product that feeds a sum rounded on its
+// own: __fmul_rn / __dmul_rn are never contracted into a multiply-add, so the bits are those of the merge compiled with
+// -fmad=false in any translation unit.  The env-sharded evaluation step merges with it in peer_comm.cu and so equals, on one
+// rank, the merge that xb_eval_step's last CTA does itself (env_classic.cu).
+__device__ __forceinline__ void merge_obs_sums_rn(const double* sums, int D, const double* obs_state_in, double* obs_state_out, int dim,
+                                                  int tid) {
+    if (tid >= D) return;
+    const double n = sums[2 * D], count = obs_state_in[2 * D];
+    float nm = (float)obs_state_in[tid], nv = (float)obs_state_in[D + tid];
+    if (tid < dim) {
+        const double bm = sums[tid] / n;
+        double bv = sums[D + tid] / n - __dmul_rn(bm, bm);
+        bv = bv > 0.0 ? bv : 0.0;
+        const float fc = (float)count, fb = (float)n, ft = (float)(count + n);    // chan_merge
+        const float delta = (float)bm - nm;
+        const float m2 = __fmul_rn(nv, fc) + __fmul_rn((float)bv, fb) + delta * delta * fc * fb / ft;
+        nm = nm + delta * fb / ft;
+        nv = m2 / ft;
+    }
+    obs_state_out[tid] = (double)nm;
+    obs_state_out[D + tid] = (double)nv;
+    if (tid == 0) obs_state_out[2 * D] = count + n;
+}
+
 // Sum of 32 doubles in shared memory, read in an order rotated by `rot` (lanes that walk rows 256 B apart then never share a
 // bank) and added as four independent chains: a fixed association order, a quarter of the dependent-add latency.
 __device__ __forceinline__ double row_sum32(const double* row, int rot) {

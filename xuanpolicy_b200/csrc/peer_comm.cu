@@ -18,6 +18,8 @@
 //     the optimiser scalars: the gradient exchange of a learner that steps a torch optimiser itself (PPG_Learner).
 //   * xb_peer_allreduce_f64 — the (sum adv, sum adv^2) of every minibatch of an epoch in one exchange
 //     (the sharded form of memory_tools.py:241-242), fed by xb_adv_stats_minibatches.  Pull-based, two barriers.
+//   * xb_peer_allreduce_merge / xb_peer_eval_merge — one step's running-statistics sums of the env-sharded rollout / of the
+//     env-sharded evaluation loop (test()), pushed into a small inbox, one barrier, merged in the same kernel.
 //
 // Cross-GPU barrier (per CTA, no grid-wide sync): CTA b of rank r release-stores a monotonically increasing ticket
 // into flags[b][r] of every peer, then acquire-spins until its own flags[b][*] have reached the ticket.  Tickets
@@ -181,14 +183,12 @@ __global__ void __launch_bounds__(256)
 // (set-up, resident weights) while this kernel waits for its peers.
 constexpr int kPeerPushSlot = kPeerSlots - 3;
 constexpr int kPeerPushMax = 20;       // the 2D + 4 step sums of 8-float observation rows
-__global__ void __launch_bounds__(128)
-    peer_allreduce_merge_kernel(PeerTable t, int rank, int W, int inbox_off, int n, const double* __restrict__ src,
-                                double* __restrict__ out, uint32_t* __restrict__ tickets, const double* __restrict__ obs_state_in,
-                                double* __restrict__ obs_state_out, int dim, double* __restrict__ ret_state,
-                                float* __restrict__ rew_std) {
-    __shared__ double sums[kPeerPushMax];
-    pdl_wait();
-    pdl_trigger();
+
+// The push exchange of one CTA (every thread calls it): src[0, n) goes into inbox row [parity][rank] of every peer, one
+// cross-GPU barrier on flag slot kPeerPushSlot, then sums[j] (shared, kPeerPushMax) = the W rows added in rank order out of
+// LOCAL memory, 0 for j >= n; out[j] = sums[j] for j < n.
+__device__ __forceinline__ void peer_push_sum(const PeerTable& t, int rank, int W, int inbox_off, int n, const double* __restrict__ src,
+                                              double* __restrict__ out, uint32_t* __restrict__ tickets, double* sums) {
     const uint32_t ticket = tickets[kPeerPushSlot] + 1;
     const int parity = (int)(ticket & 1u);
     for (int i = threadIdx.x; i < n * W; i += blockDim.x) {
@@ -208,8 +208,48 @@ __global__ void __launch_bounds__(128)
     }
     __syncthreads();
     if (threadIdx.x == 0) tickets[kPeerPushSlot] = ticket;
+}
+
+__global__ void __launch_bounds__(128)
+    peer_allreduce_merge_kernel(PeerTable t, int rank, int W, int inbox_off, int n, const double* __restrict__ src,
+                                double* __restrict__ out, uint32_t* __restrict__ tickets, const double* __restrict__ obs_state_in,
+                                double* __restrict__ obs_state_out, int dim, double* __restrict__ ret_state,
+                                float* __restrict__ rew_std) {
+    __shared__ double sums[kPeerPushMax];
+    pdl_wait();
+    pdl_trigger();
+    peer_push_sum(t, rank, W, inbox_off, n, src, out, tickets, sums);
     if (threadIdx.x < 32 && (obs_state_in || ret_state))
         merge_step_sums(sums, (n - 4) / 2, obs_state_in, obs_state_out, dim, ret_state, rew_std, threadIdx.x);
+}
+
+// One step of the env-sharded evaluation loop, after xb_eval_step wrote this rank's step record (the StepStats::sums_out layout
+// [2D + 4], finishers in the n-finished slot): the ranks' records are summed in rank order, the global episode count advances
+// by the finishers of every rank, and the next observations' moments are merged into the observation statistics when the loop
+// goes round again (count still below test_episode), as xb_eval_step does on one rank.  A launch that finds the target met
+// returns before it pushes or waits: the count is bit-identical on every rank, so every rank skips the same barriers.
+__global__ void __launch_bounds__(128)
+    peer_eval_merge_kernel(PeerTable t, int rank, int W, int inbox_off, int n, const double* __restrict__ record,
+                           double* __restrict__ totals, int64_t* __restrict__ count, const int64_t* __restrict__ test_episode, double* __restrict__ obs_state,
+                           double* __restrict__ obs_state_cand, int dim, uint32_t* __restrict__ tickets) {
+    __shared__ double sums[kPeerPushMax];
+    __shared__ int64_t s_c0, s_target;
+    if (threadIdx.x == 0) {
+        s_c0 = *count;
+        s_target = *test_episode;
+    }
+    __syncthreads();
+    if (s_c0 >= s_target) return;
+    peer_push_sum(t, rank, W, inbox_off, n, record, totals, tickets, sums);
+    if (threadIdx.x >= 32) return;
+    const int D = (n - 4) / 2;
+    const int64_t c1 = s_c0 + (int64_t)sums[2 * D + 3];
+    if (obs_state && c1 < s_target) {
+        merge_obs_sums_rn(sums, D, obs_state, obs_state_cand, dim, threadIdx.x);
+        __syncwarp();
+        if ((int)threadIdx.x < 2 * D + 1) obs_state[threadIdx.x] = obs_state_cand[threadIdx.x];
+    }
+    if (threadIdx.x == 0) *count = c1;
 }
 
 // (sum, sumsq) of the advantages of every minibatch of an epoch in one pass over the permutation:
@@ -340,6 +380,22 @@ extern "C" int xb_peer_allreduce_merge(const void* const* peer_bases /* host [W]
     if (ret_state && !rew_std) return XB_E_BADARG;
     XB_CUDA(launch_pdl(peer_allreduce_merge_kernel, dim3(1), dim3(128), 0, (cudaStream_t)stream, true, t, rank, W, inbox_offset, n, src,
                        out, tickets, obs_state_in, obs_state_out, dim, ret_state, rew_std));
+    XB_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int xb_peer_eval_merge(const void* const* peer_bases /* host [W] */, int rank, int W, const double* record, int n,
+                                  int inbox_offset, double* totals, int64_t* count, const int64_t* test_episode, double* obs_state,
+                                  double* obs_state_cand, int dim, uint32_t* tickets, xb_stream_t stream) {
+    PeerTable t;
+    int rc = make_table(peer_bases, rank, W, &t);
+    if (rc) return rc;
+    if (!record || !totals || !count || !test_episode || !tickets || (n != 12 && n != 20) || inbox_offset < 0 ||
+        inbox_offset + 2 * kPeerMaxRanks * kPeerPushMax > kPeerStatsMax)
+        return XB_E_BADARG;
+    if (obs_state && (!obs_state_cand || obs_state == obs_state_cand || dim < 1 || dim > (n - 4) / 2)) return XB_E_BADARG;
+    peer_eval_merge_kernel<<<1, 128, 0, (cudaStream_t)stream>>>(t, rank, W, inbox_offset, n, record, totals, count, test_episode, obs_state,
+                                                                obs_state_cand, dim, tickets);
     XB_LAUNCH_CHECK();
     return 0;
 }

@@ -68,14 +68,18 @@ def rollout_step(kind, act_param, logstd, val, seed, counter, offset, state, rng
 
 
 def eval_step(kind, act_param, logstd, key, step, state, rng, elapsed, ep_score, next_obs, trig_cache, max_steps, scores, count,
-              test_episode, partials, workspace, obs_state=None, obs_state_cand=None, obs_dim=0, act_tape=None):
-    """Sample + env step + episode queue + observation statistics of one evaluation step in one launch (xb_eval_step)."""
+              test_episode, partials, workspace, obs_state=None, obs_state_cand=None, obs_dim=0, act_tape=None, local_count=None,
+              score_step=None, record=None):
+    """Sample + env step + episode queue + observation statistics of one evaluation step in one launch (xb_eval_step).
+    local_count / score_step / record: the env-sharded form (this rank's queue, step tags and step record)."""
     N = elapsed.numel()
+    if score_step is not None and score_step.numel() < scores.numel():
+        raise _lib.XB200Error("score_step needs one entry per queue slot (%d < %d)" % (score_step.numel(), scores.numel()))
     _lib.call("xb_eval_step", kind, _p(act_param, F32), _p(logstd, F32), _p(key, I64), _p(step, I64), _p(state, F64),
               _p(rng, I64), _p(elapsed, I32), _p(ep_score, F64), _p(next_obs, F32), _p(trig_cache, F64), max_steps,
               _p(act_tape, F32 if kind == 1 else I64), act_tape.shape[0] if act_tape is not None else 0, _p(scores, F64),
               _p(count, I64), _p(test_episode, I64), scores.numel(), _p(obs_state, F64), _p(obs_state_cand, F64), int(obs_dim),
-              _p(partials, F64), _p(workspace, I64), N, _stream())
+              _p(partials, F64), _p(workspace, I64), _p(local_count, I64), _p(score_step, I32), _p(record, F64), N, _stream())
 
 
 def sincos_f64(x):
@@ -270,6 +274,16 @@ def peer_allreduce_merge(peer, src, n, out, inbox_offset, obs_in=None, obs_out=N
     """One-barrier push exchange of `src[:n]` (out[:n] = totals over ranks) + the normaliser merge (xb_peer_allreduce_merge)."""
     _lib.call("xb_peer_allreduce_merge", peer.bases, peer.rank, peer.world, _p(src, F64), int(n), int(inbox_offset), _p(out, F64),
               _p(peer.tickets, I32), _p(obs_in, F64), _p(obs_out, F64), int(obs_dim), _p(ret_state, F64), _p(rew_std, F32), _stream())
+
+
+def peer_eval_merge(peer, record, totals, count, test_episode, inbox_offset, obs_state=None, obs_state_cand=None, obs_dim=0):
+    """The exchange that completes one env-sharded evaluation step: the ranks' records (fp64 [2D + 4]) summed in rank order into
+    `totals`, the global episode count advanced, the observation statistics merged while the loop goes on (xb_peer_eval_merge)."""
+    if totals.numel() < record.numel():
+        raise _lib.XB200Error("totals needs %d doubles" % record.numel())
+    _lib.call("xb_peer_eval_merge", peer.bases, peer.rank, peer.world, _p(record, F64), record.numel(), int(inbox_offset),
+              _p(totals, F64), _p(count, I64), _p(test_episode, I64), _p(obs_state, F64), _p(obs_state_cand, F64), int(obs_dim),
+              _p(peer.tickets, I32), _stream())
 
 
 def adv_stats_minibatches(idx, n_minibatches, B, T, N, adv, stride, stats):
