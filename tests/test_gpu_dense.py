@@ -115,7 +115,7 @@ def test_dense_dgrad_matches_fp64_autograd(M, H, nh0, nh1):
 
 
 @pytest.mark.parametrize("B,H,nh0,nh1", [(65536, 128, 1, 1), (4099, 128, 2, 1), (8192, 256, 1, 1), (4096, 128, 1, 0),
-                                         (100, 128, 1, 1)])
+                                         (100, 128, 1, 1), (8192 + 33, 256, 2, 1)])
 def test_dense_wgrad_matches_fp64_autograd(B, H, nh0, nh1):
     """dW, db of the actor / critic hidden layers and dw2, db2 of their heads, from the saved activations."""
     from xuanpolicy_b200 import ops
