@@ -38,6 +38,26 @@ def gae_close(a, b, rtol=1e-5):
     return bool(np.all(np.abs(a - b) <= rtol * scale)), float(np.max(np.abs(a - b) / scale))
 
 
+def rel_err(a, ref):
+    """max_i |a_i - ref_i| / max(|ref_i|, rms(ref)) of two torch tensors — the metric the GAE parity test uses (values
+    cross zero)."""
+    ref = ref.double()
+    rms = ref.pow(2).mean().sqrt().clamp_min(1e-30)
+    return float(((a.double() - ref).abs() / rms.maximum(ref.abs())).max())
+
+
+def rel_rms_err(a, ref):
+    """rms(a - ref) / rms(ref) of two torch tensors."""
+    ref = ref.double()
+    return float((a.double() - ref).pow(2).mean().sqrt() / ref.pow(2).mean().sqrt().clamp_min(1e-30))
+
+
+# Bars of the tensor-core dense kernels against fp64 (rel_err, rel_rms_err).  The tensor core accumulates in fp32 with
+# truncation, so the worst element of ~10^7 sits near 1e-5 of the output scale (cuBLAS fp32 SIMT: ~1e-6; single-pass
+# TF32: ~1e-3); the rms error is ~1e-6.  Both are far inside north_star's 1e-4 loss/gradient tolerance.
+MAX_BAR, RMS_BAR = 5e-5, 5e-6
+
+
 def rel_close(a, b, rtol):
     a = np.asarray(a, np.float64)
     b = np.asarray(b, np.float64)

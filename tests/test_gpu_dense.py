@@ -8,27 +8,14 @@ plain TF32 would sit at ~1e-3.
 import pytest
 import torch
 
+# (bars: see tests/helpers.py)
+from tests.helpers import MAX_BAR, RMS_BAR
+from tests.helpers import rel_err as _rel
+from tests.helpers import rel_rms_err as _rel_rms
+
 pytestmark = pytest.mark.gpu
 
 SLOPE = 0.01
-
-
-def _rel(a, ref):
-    """max_i |a_i - ref_i| / max(|ref_i|, rms(ref)) — the metric the GAE parity test uses (values cross zero)."""
-    ref = ref.double()
-    rms = ref.pow(2).mean().sqrt().clamp_min(1e-30)
-    return float(((a.double() - ref).abs() / torch.maximum(ref.abs(), rms)).max())
-
-
-def _rel_rms(a, ref):
-    ref = ref.double()
-    return float((a.double() - ref).pow(2).mean().sqrt() / ref.pow(2).mean().sqrt().clamp_min(1e-30))
-
-
-# Bars.  The tensor core accumulates in fp32 with truncation, so the worst element of ~10^7 sits near 1e-5 of the output
-# scale (cuBLAS fp32 SIMT: ~1e-6; single-pass TF32: ~1e-3); the rms error is ~1e-6.  Both are far inside north_star's
-# 1e-4 loss/gradient tolerance.
-MAX_BAR, RMS_BAR = 5e-5, 5e-6
 
 
 def _split(W, transposed_into=None, toff=0):

@@ -12,23 +12,14 @@ import math
 import pytest
 import torch
 
+from tests.helpers import MAX_BAR, RMS_BAR
+from tests.helpers import rel_err as _rel
+from tests.helpers import rel_rms_err as _rel_rms
+
 pytestmark = pytest.mark.gpu
 
 SLOPE = 0.01
-MAX_BAR, RMS_BAR = 5e-5, 5e-6
 GRAD_BAR = 1e-4
-
-
-def _rel(a, ref):
-    """max_i |a_i - ref_i| / max(|ref_i|, rms(ref))"""
-    ref = ref.double()
-    rms = ref.pow(2).mean().sqrt().clamp_min(1e-30)
-    return float(((a.double() - ref).abs() / torch.maximum(ref.abs(), rms)).max())
-
-
-def _rel_rms(a, ref):
-    ref = ref.double()
-    return float((a.double() - ref).pow(2).mean().sqrt() / ref.pow(2).mean().sqrt().clamp_min(1e-30))
 
 
 def _spaces(env_id):
