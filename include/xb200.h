@@ -220,6 +220,35 @@ int xb_dist_loss_gaussian(int64_t B, const float* mu, const float* logstd, const
 int xb_kl_coef_adapt(const double* scalars, float* kl_coef_dev, float target_kl, int64_t count, xb_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * PPO-KL minibatch loss of the native update on packed minibatch rows (PPOKL_Learner.update, ppokl_learner.py:21-61),
+ * forward + backward w.r.t. the network outputs in one launch; 2 logits (gaussian = 0) or one Gaussian dimension with a
+ * shared log-std (gaussian = 1).  The general shapes use xb_dist_loss_*.
+ *   idx [B] int64    the reference's flat indices (env = k / T, step = k % T) of the minibatch
+ *   scal f32 [B][4]  {act, old_logp, adv, ret} as written by xb_gather_records (16-byte aligned)
+ *   old_dist f32 [T][N][2]  the rollout's old-distribution pairs: logits (z0, z1), or (mu, std); read at each sample's row
+ *   act_out          the forward's head outputs: logits [B][2] (8-byte aligned) or mu [B]; logstd f32 [1] (Gaussian)
+ *   adv_stats        nullable fp64 [2] (sum adv, sum adv^2) over adv_count samples: advantages are normalised with them
+ *   inv_batch        1 / (global minibatch size); kl_coef f32 [1]: the adaptive coefficient (read, then adapted)
+ *   kl_used          nullable f32 [1]: receives the coefficient this launch used (the `actor-loss` log)
+ *   adapt != 0       adapt kl_coef in this launch from KL sum / kl_count (count = B, x2 above 1.5 target_kl, /2 below
+ *                    0.5 target_kl, clip [0.1, 20]; any target, like the reference); 0: leave it (env-sharded: exchange
+ *                    the KL sum, then xb_ppokl_kl_adapt)
+ *   kl_sum_out       nullable fp64 [1]: this launch's KL sum is also written there
+ *   dact [B][2] / [B], dv [B]  dL/d(act_out), dL/dv; dlogstd fp64 [1] (Gaussian): dL/dlogstd
+ *   scalars fp64 [8] (overwritten) = sums of {ratio * adv, (v-R)^2, entropy, v_pred, 0, KL, 0, 0}
+ * Deterministic (per-CTA partials added in CTA order by the last CTA); one such launch at a time per device.
+ * xb_ppokl_kl_adapt: the same adaptation from a KL sum on the device (kl_sum fp64 [1], e.g. the cross-rank total),
+ *   recording the coefficient before the change in kl_used (nullable).
+ * ---------------------------------------------------------------------------------------------------------- */
+int xb_ppokl_loss_packed(const int64_t* idx, int64_t B, int64_t T, int64_t N, const float* scal, const float* old_dist,
+                         const float* act_out, const float* logstd, int gaussian, const float* v_pred,
+                         const double* adv_stats, int64_t adv_count, float vf_coef, float ent_coef, float inv_batch,
+                         float* kl_coef, float* kl_used, float target_kl, int adapt, int64_t kl_count, double* kl_sum_out,
+                         float* dact, float* dv, double* dlogstd, double* scalars, xb_stream_t stream);
+int xb_ppokl_kl_adapt(const double* kl_sum, float* kl_coef, float* kl_used, float target_kl, int64_t count,
+                      xb_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------------------
  * Action sampling fused with log-prob (after the actor GEMM).  Replaces dists.stochastic_sample()+log_prob in
  * PPOCLIP_Agent._action (ppoclip_agent.py:50-57; distributions.py:57-58,89-90).  Philox4x32-10, counter-based:
  * stream position = (*counter_dev + offset, env index), so a captured graph replays with fresh numbers once
@@ -343,6 +372,8 @@ int xb_bias_act_fwd(float* y, const float* bias, float slope, int64_t B, int H, 
  *   stat_sums_out (nullable, fp64 [2D + 4], env-sharded form): this rank's totals (sum x[D], sum x^2[D], N, sum R, sum R^2,
  *     n finished) are written there INSTEAD of being merged (obs_state_out / ret_state unused); exchange them across ranks
  *     (xb_peer_allreduce_merge, or xb_peer_allreduce_f64 and xb_rms_merge_sums).
+ * dist_row (nullable, f32 [N][W], PPO-KL's `{"old_dist": dists}`): row t of the rollout's old-distribution array receives the
+ *   parameters the action was drawn from: the W = 2 / 3 logits, or (mu, std = exp(logstd)) for Pendulum-v1 (W = 2).
  * ---------------------------------------------------------------------------------------------------------- */
 int xb_rollout_step(int env_kind, const float* act_param, const float* logstd, const float* val, uint64_t seed,
                     const uint64_t* counter_dev, uint64_t offset, double* state, uint64_t* rng, int32_t* elapsed,
@@ -353,7 +384,7 @@ int xb_rollout_step(int env_kind, const float* act_param, const float* logstd, c
                     const float* rew_scale, float rew_clip, const float* boot_src, float* boot_row, double* trig_cache,
                     const double* obs_state_in, double* obs_state_out, int obs_dim, float obs_clip, double* ret_state,
                     float* rew_std_io, double* returns, double gamma, int mask_terminal, double* stat_partials,
-                    uint32_t* stat_ticket, double* stat_sums_out, int64_t N, xb_stream_t stream);
+                    uint32_t* stat_ticket, double* stat_sums_out, float* dist_row, int64_t N, xb_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * One vector step of the evaluation loop in ONE launch.  Replaces the body of PPOCLIP_Agent.test (ppoclip_agent.py:113-165):

@@ -8,6 +8,7 @@ Drop-in classes (same names / signatures as the reference, see each module's doc
     PPOCLIP_Agent        agent.py     <- xuance/torch/agents/policy_gradient/ppoclip_agent.py:4-165 (vectorised loop)
     A2C_Agent            agent.py     <- xuance/torch/agents/policy_gradient/a2c_agent.py:6-100 (same loop, A2C surrogate)
     PG_Agent             agent.py     <- xuance/torch/agents/policy_gradient/pg_agent.py:4-96 (same loop, returns as weights)
+    PPOKL_Agent          agent.py     <- xuance/torch/agents/policy_gradient/ppokl_agent.py (same loop, adaptive KL penalty)
     PPG_Agent            agent.py     <- xuance/torch/agents/policy_gradient/ppg_agent.py:4-109 (device rollout, 3 update phases)
 All arithmetic on the path runs in hand-written CUDA kernels reached through the C ABI of include/xb200.h
 (libxb200.so, bound with ctypes in _lib.py).  There is no CPU fallback: importing works anywhere, but
@@ -26,7 +27,7 @@ __version__ = "0.1.0"
 
 
 def __getattr__(name):
-    if name in ("PPOCLIP_Agent", "A2C_Agent", "PG_Agent", "PPG_Agent"):
+    if name in ("PPOCLIP_Agent", "A2C_Agent", "PG_Agent", "PPOKL_Agent", "PPG_Agent"):
         from . import agent
         return getattr(agent, name)
     raise AttributeError(name)

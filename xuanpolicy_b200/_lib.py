@@ -20,7 +20,7 @@ SIGNATURES = {
     "xb_env_step": [_i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _vp],
     "xb_rollout_step": [_i32, _vp, _vp, _vp, _u64, _vp, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                         _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f32, _vp, _vp, _vp,
-                        _vp, _vp, _i32, _f32, _vp, _vp, _vp, _f64, _i32, _vp, _vp, _vp, _i64, _vp],
+                        _vp, _vp, _i32, _f32, _vp, _vp, _vp, _f64, _i32, _vp, _vp, _vp, _vp, _i64, _vp],
     "xb_eval_step": [_i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _vp,
                      _i32, _vp, _vp, _vp, _vp, _vp, _i64, _vp],
     "xb_sincos_f64": [_vp, _vp, _vp, _i64, _vp],
@@ -39,6 +39,9 @@ SIGNATURES = {
     "xb_dist_loss_gaussian": [_i64, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _f32, _vp, _f32, _f32,
                               _f32, _f32, _vp, _vp, _vp, _vp, _vp, _vp],
     "xb_kl_coef_adapt": [_vp, _vp, _f32, _i64, _vp],
+    "xb_ppokl_loss_packed": [_vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _i64, _f32, _f32, _f32, _vp, _vp, _f32,
+                             _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp],
+    "xb_ppokl_kl_adapt": [_vp, _vp, _vp, _f32, _i64, _vp],
     "xb_pack_records": [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp],
     "xb_gather_records": [_vp, _i64, _i64, _i64, _vp, _i32, _vp, _vp, _vp, _vp],
     "xb_gather_trunk_fwd": [_vp, _i64, _i64, _i64, _vp, _i32, _vp, _vp, _f32, _i32, _vp, _vp, _vp, _vp, _vp, _vp],

@@ -377,6 +377,10 @@ class PPOCLIP_Agent:
     def _store_extra(self, t, dist):
         """Per-step auxiliaries beyond old_logp (PPG: the old action distribution's parameters)."""
 
+    def _dist_out(self, t):
+        """Row t of the old-distribution array when the fused rollout step writes it (PPO-KL), else None."""
+        return None
+
     @staticmethod
     def _rank():
         d = torch.distributed
@@ -469,7 +473,7 @@ class PPOCLIP_Agent:
                              mem._term[t], mem._trunc[t], mem._logp[t],
                              rew_std=self._rew_std if self.use_rewnorm else None, rew_clip=self.rewnorm_range,
                              boot_src=v[N:] if boot else None, boot_row=mem._boot[t - 1] if boot else None,
-                             trig_cache=self._trig_cache, stats=stats)
+                             trig_cache=self._trig_cache, stats=stats, dist_row=self._dist_out(t))
             if self._shard_norm:      # the ranks' sums of this step -> global sums -> merged normalisers (for the next step)
                 c = self._rms_cur
                 if self._norm_push:
@@ -514,7 +518,7 @@ class PPOCLIP_Agent:
                              mem._term[t], mem._trunc[t], mem._logp[t],
                              rew_std=self._rew_std if self.use_rewnorm else None, rew_clip=self.rewnorm_range,
                              boot_src=v[N:] if boot else None, boot_row=mem._boot[t - 1] if boot else None,
-                             trig_cache=self._trig_cache)
+                             trig_cache=self._trig_cache, dist_row=self._dist_out(t))
         else:
             self._sample(dist, t)
             ops.env_step(env._kind, env._state, env._rng, env._elapsed, env._ep_score, self._act.reshape(N),
@@ -662,7 +666,7 @@ class PPOCLIP_Agent:
                 g[1].replay()
             else:
                 lr.stage_forward_backward(mem, idx, mb)
-            xdist.allreduce_flat_grad(lr._flat.flat_grad, lr.process_group)
+            lr.allreduce_grads()
             if g is not None:
                 g[2].replay()
             else:
@@ -827,7 +831,7 @@ class PPOCLIP_Agent:
             if mem.use_advnorm:
                 xdist.allreduce_adv_stats(mb["stats"], lr.process_group)
             lr.stage_forward_backward(mem, idx, mb)
-            xdist.allreduce_flat_grad(lr._flat.flat_grad, lr.process_group)
+            lr.allreduce_grads()
             lr.stage_optimizer()
 
     def _state_tensors(self):
@@ -1242,6 +1246,59 @@ class PG_Agent(PPOCLIP_Agent):
         info = super()._collect_info()
         for k in ("critic-loss", "predict_value", "clip_ratio"):    # pg_learner.py:38-42 logs three scalars
             info.pop(k, None)
+        return info
+
+
+class PPOKL_Agent(PPOCLIP_Agent):
+    """PPOKL_Agent (xuance/torch/agents/policy_gradient/ppokl_agent.py) on the device loop above: PPOCLIP_Agent's training
+    loop with the old action distribution stored per transition (`{"old_dist": dists}`, device rows [T, N, W]: the logits,
+    or mu and std) and PPOKL_Learner's update: a_loss = -(ratio * adv).mean() + kl_coef * KL(new || old).mean(), no gradient
+    clipping, the coefficient adapted on the device after every minibatch from that minibatch's KL (x2 above 1.5 target_kl,
+    /2 below 0.5 target_kl, clipped to [0.1, 20]; the update that measured the KL used the old value).  The update phase is
+    the captured epoch graphs: the coefficient changes between replays on the device.  The fused rollout step writes the old
+    distribution in the same launch; the unfused step stores it from the forward's parameters.
+    The reference's own train loop cannot run (ppokl_agent.py:22, 26 and 80-82, see DESIGN.md §8 f3); this is the loop
+    those lines evidently intend: PPOCLIP_Agent's, with the auxiliary and the five-argument `PPOKL_Learner.update`."""
+    _aux_shape = {"old_dist": None}
+
+    def __init__(self, config, envs, policy, optimizer, scheduler=None, device=None, process_group=None):
+        super().__init__(config, envs, policy, optimizer, scheduler, device, process_group)
+        M = self.buffer_size // self.batch_size
+        if self.learner._peer is not None and 2 * M > self._NORM_INBOX:
+            # the epoch's advantage sums take doubles [0, 2M) of the comm block's statistics area: they must stay clear of
+            # the normaliser inbox [1024, 1344) and of the KL slot (PPOKL_Learner._KL_SLOT)
+            raise ValueError("env-sharded PPO-KL over peer memory supports n_minibatch <= %d (got %d minibatches per epoch)"
+                             % (self._NORM_INBOX // 2, M))
+        mem, A = self.memory, (int(self.action_space.n) if self.discrete else self.memory.act_dim)
+        mem._dist_kind = "categorical" if self.discrete else "gaussian"
+        mem._dist = torch.zeros((self.n_steps, self.n_envs, A if self.discrete else 2 * A), dtype=torch.float32,
+                                device=self.device)
+        self._n_act = A
+
+    def _make_learner(self, config, policy, optimizer, scheduler):
+        from .learner import PPOKL_Learner
+        return PPOKL_Learner(policy, optimizer, scheduler, self.device, getattr(config, "model_dir", "./"),
+                             vf_coef=config.vf_coef, ent_coef=config.ent_coef, target_kl=config.target_kl)
+
+    def _dist_out(self, t):
+        return self.memory._dist[t] if self._fused_step else None
+
+    def _store_extra(self, t, dist):
+        if self._fused_step:
+            return
+        out, prm, N, A = self.memory._dist[t], dist.get_param(), self.n_envs, self._n_act
+        if self.discrete:
+            out.copy_(prm[:N])
+            return
+        out[:, :A].copy_(prm[0][:N])
+        std = prm[1]
+        if std is None:                 # the tensor-core forward returns mu only; the log-std is the policy's parameter
+            std = self.policy.actor.logstd.detach().exp()
+        out[:, A:].copy_(std.reshape(-1, A).expand(N, A) if std.numel() == A else std[:N])
+
+    def _collect_info(self):
+        info = super()._collect_info()
+        info.pop("clip_ratio", None)
         return info
 
 

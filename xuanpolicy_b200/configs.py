@@ -100,3 +100,12 @@ def build_ppg(env_id, device="cuda", agent_class=None, process_group=None, polic
         return cls(envs.action_space, rep, list(cfg.actor_hidden_size), list(cfg.critic_hidden_size), activation=act,
                    device=device)
     return _build(_PPG, env_id, "PPG_Agent", policy, device, overrides, agent_class, process_group, policy_seed)
+
+
+def build_ppokl(env_id, device="cuda", agent_class=None, process_group=None, policy_seed=None, **overrides):
+    """PPOKL_Agent wired like build_ppo (envs, the actor-critic policy, Adam, LinearLR, the agent).  The reference's ppokl
+    yamls are not restated here, so the defaults are the PPO classic-control ones of `_COMMON` (including its `target_kl`)
+    with `agent="PPO_KL"`; every key can be overridden.  `process_group` / `policy_seed` as in build_ppo."""
+    from .agent import PPOKL_Agent
+    return build_ppo(env_id, device=device, process_group=process_group, policy_seed=policy_seed,
+                     agent_class=agent_class or PPOKL_Agent, **dict(dict(agent="PPO_KL"), **overrides))

@@ -24,6 +24,7 @@ SOURCES = {
     "gae.cu": [],
     "ppo_loss.cu": [],
     "dist_loss.cu": [],
+    "ppokl_loss.cu": [],
     "sample.cu": [],
     "optim.cu": [],
     "peer_comm.cu": [],

@@ -453,6 +453,9 @@ struct RolloutStepArgs {
     // stats.obs_state_in set, x_in holds RAW observations and the stored row is their normalised form (the same arithmetic
     // as the forward kernel's, agent.py:112-113); the next observations' moments are merged into stats.obs_state_out.
     StepStats stats;
+    // nullable: row t of the old-distribution array [T][N][W] (PPO-KL): the kActions logits the action was drawn from, or
+    // (mu, std = exp(logstd)) of the one-dim Gaussian
+    float* dist_row;
 #ifdef XB_STEP_TS
     unsigned long long* ts;
 #endif
@@ -497,6 +500,15 @@ __global__ void __launch_bounds__(128) rollout_step_kernel(RolloutStepArgs a) {
     }
     a.logp_out[e] = logp;
     a.logp_row[e] = logp;
+    if (a.dist_row) {
+        if (Env::kDiscrete) {
+#pragma unroll
+            for (int j = 0; j < Env::kActions; ++j) a.dist_row[e * Env::kActions + j] = a.act_param[e * Env::kActions + j];
+        } else {
+            a.dist_row[2 * e] = a.act_param[e];
+            a.dist_row[2 * e + 1] = expf(a.logstd[0]);
+        }
+    }
     if (with_stats && a.stats.obs_state_in) {          // stored observation = the normalised one the policy acted on
 #pragma unroll
         for (int v = 0; v < V; ++v) {
@@ -940,7 +952,7 @@ extern "C" int xb_rollout_step(int env_kind, const float* act_param, const float
                                const float* boot_src, float* boot_row, double* trig_cache, const double* obs_state_in,
                                double* obs_state_out, int obs_dim, float obs_clip, double* ret_state, float* rew_std_io,
                                double* returns, double gamma, int mask_terminal, double* stat_partials, uint32_t* stat_ticket,
-                               double* stat_sums_out, int64_t N, xb_stream_t stream) {
+                               double* stat_sums_out, float* dist_row, int64_t N, xb_stream_t stream) {
     if (N <= 0 || !act_param || !val || !state || !rng || !elapsed || !ep_score || !obs || !rew || !term || !trunc ||
         !reset_obs || !ep_step_out || !ep_score_out || !x_in || !act_out || !logp_out || !obs_row || !act_row ||
         !rew_row || !val_row || !term_row || !logp_row)
@@ -950,7 +962,8 @@ extern "C" int xb_rollout_step(int env_kind, const float* act_param, const float
     RolloutStepArgs a{act_param, logstd, val, seed, counter_dev, offset, state, rng, elapsed, ep_score, (float4*)obs,
                       (float4*)next_obs, rew, term, trunc, (float4*)reset_obs, ep_step_out, ep_score_out, ep_stats,
                       max_episode_steps, (const float4*)x_in, act_out, logp_out, (float4*)obs_row, act_row, rew_row,
-                      val_row, term_row, trunc_row, logp_row, rew_scale, rew_clip, boot_src, boot_row, trig_cache, N, StepStats{}};
+                      val_row, term_row, trunc_row, logp_row, rew_scale, rew_clip, boot_src, boot_row, trig_cache, N, StepStats{},
+                      dist_row};
     if (stat_partials) {
         if (!stat_ticket || (!obs_state_in && !returns)) return XB_E_BADARG;
         if (obs_state_in && (obs_dim < 1 || obs_dim > 8)) return XB_E_BADARG;

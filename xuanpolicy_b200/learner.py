@@ -433,18 +433,26 @@ class PPOCLIP_Learner:
             xdist.allreduce_adv_stats(mb["stats"], self.process_group)
         self.stage_forward_backward(memory, idx, mb)
         if self.world_size > 1 and self._peer is None:
-            xdist.allreduce_flat_grad(self._flat.flat_grad, self.process_group)
+            self.allreduce_grads()
         self.stage_optimizer()
+
+    def allreduce_grads(self):
+        """NCCL form of the env-sharded exchange between `stage_forward_backward` and `stage_optimizer` (no peer memory):
+        the flat gradient summed over the ranks, in place."""
+        xdist.allreduce_flat_grad(self._flat.flat_grad, self.process_group)
 
     def info(self, batch_size):
         """Host copy of the last update's log scalars (one sync; the native loop calls it once per rollout)."""
         s = self._scalars.cpu().numpy() / batch_size
+        return {"actor-loss": float(-s[0]), "critic-loss": float(s[1]), "entropy": float(s[2]), "learning_rate": self._native_lr(),
+                "predict_value": float(s[3]), "clip_ratio": torch.tensor(s[4], dtype=torch.float32)}
+
+    def _native_lr(self):
         lr = float(self._flat.lr.item()) if self._flat is not None else self.optimizer.param_groups[0]["lr"]
         if self._flat is not None and self._flat.total_iters > 0:   # the reference reports the lr AFTER scheduler.step()
             it = min(int(self._flat.step.item()), self._flat.total_iters)
             lr = self._flat.lr0 * (1.0 + (self._flat.end_factor - 1.0) * it / self._flat.total_iters)
-        return {"actor-loss": float(-s[0]), "critic-loss": float(s[1]), "entropy": float(s[2]), "learning_rate": lr,
-                "predict_value": float(s[3]), "clip_ratio": torch.tensor(s[4], dtype=torch.float32)}
+        return lr
 
 
 class A2C_Learner(PPOCLIP_Learner):
@@ -561,9 +569,159 @@ class PPOKL_Learner(_DistLossLearner):
                          clip_range=0.0, clip_grad_norm=None, use_grad_clip=False)
         self.target_kl = target_kl
         self._kl_coef_dev = torch.ones(1, dtype=torch.float32, device=self.device)
+        self._kl_used = torch.ones(1, dtype=torch.float32, device=self.device)   # the coefficient the last update used
+        self._kl_glob = torch.zeros(1, dtype=torch.float64, device=self.device)  # env-sharded: the global KL sum
+        self._kl_count = 1                                                       # KL terms per sample (A for a Gaussian)
+
+    _KL_SLOT = 1536      # double of the comm block's statistics area for the KL sum: clear of the epoch's advantage sums
+                         # [0, 2M), the normaliser inbox [1024, 1344) and the pull-form slots at the end
 
     def state_tensors(self):
-        return dict(super().state_tensors(), **{"learner.kl_coef": self._kl_coef_dev})
+        return dict(super().state_tensors(), **{"learner.kl_coef": self._kl_coef_dev, "learner.kl_used": self._kl_used})
+
+    # ---------------------------------------------------------------------------------------------- native stages
+    def _packed_loss_ok(self, memory, B):
+        """The one-launch loss of csrc/ppokl_loss.cu: packed records with [T, N, 2] old-distribution pairs, the tensor-core
+        MLP at this minibatch size, and a 2-logit head or a one-dim Gaussian head with its log-std held directly."""
+        f = self._fused
+        if f is None or B < FusedActorCritic.MIN_ROWS or not memory.packed or memory._dist is None or memory._dist.shape[2] != 2:
+            return False
+        if f.gaussian:
+            p = getattr(f.policy.actor, "logstd", None)
+            return f.A == 1 and p is not None and p.requires_grad and p.numel() == 1
+        return f.A == 2
+
+    def stage_gather(self, memory, idx, compute_stats=True):
+        if self._packed_loss_ok(memory, idx.numel()):
+            return super().stage_gather(memory, idx, compute_stats)
+        # general path: every per-sample array of the minibatch, and its old-distribution rows
+        B = idx.numel()
+        mb = self._minibatch_buffers(B, memory.obs_dim)
+        if "dist" not in mb:
+            f32 = dict(dtype=torch.float32, device=self.device)
+            mb.update(act=torch.empty((B, memory.act_dim), **f32), ret=torch.empty(B, **f32), val=torch.empty(B, **f32),
+                      adv=torch.empty(B, **f32), logp=torch.empty(B, **f32),
+                      dist=torch.empty((B, memory._dist.shape[2]), **f32))
+        want = memory.use_advnorm and compute_stats
+        ops.gather_batch(idx, memory.n_size, memory.n_envs, memory._obs, memory.obs_dim, memory._act, memory.act_dim,
+                         memory._ret, memory._val, memory._adv, memory._logp, mb["obs"], mb["act"], mb["ret"], mb["val"],
+                         mb["adv"], mb["logp"], stats=mb["stats"] if want else None)
+        ops.gather_rows(idx, memory.n_size, memory.n_envs, memory._dist, mb["dist"])
+        return mb
+
+    def stage_forward_backward(self, memory, idx, mb, stats=None):
+        """The PPO-KL loss on the native path.  Packed rows at tensor-core sizes: the forward without the PPO-Clip epilogue,
+        one csrc/ppokl_loss.cu launch (which also adapts the coefficient on one rank) and the fused backward.  Otherwise the
+        general path: the forward (tensor-core or torch), the advantage normalisation and csrc/dist_loss.cu.  Env-sharded,
+        the KL sum is exchanged (peer memory here, NCCL in `allreduce_grads`) before the coefficient adapts."""
+        B, W = idx.numel(), self.world_size
+        self._mb_rows = B
+        fl, fused = self._flat, (self._fused if (self._fused is not None and B >= FusedActorCritic.MIN_ROWS) else None)
+        if self._fused is not None:
+            single = W == 1 and os.environ.get("XB_TAIL_NORM", "1") != "0"
+            self._fused.norm_sink = (fl, 0.0) if (fused is not None and single) else None
+            self._fused.norm_done = False
+        stats = (stats if stats is not None else mb["stats"]) if memory.use_advnorm else None
+        inv_batch = 1.0 / (B * W)
+        peer_slot = self._peer.stats[self._KL_SLOT:self._KL_SLOT + 1] if self._peer is not None else None
+        if self._packed_loss_ok(memory, B):
+            act_out, v = fused.forward(mb["obs"], refresh=not fused.splits_fresh, trunk_done=mb.get("trunk_done", False),
+                                       keep_y=not fused.can_skip_y(softmax_pair=not fused.gaussian),
+                                       trunk_in_kernel=mb.get("trunk_in_fwd", False))
+            b = fused._last[1]
+            if "kl_dact" not in b:
+                b["kl_dact"], b["kl_dv"] = torch.empty_like(act_out), torch.empty(B, dtype=torch.float32, device=self.device)
+            logstd = fused.policy.actor.logstd.detach() if fused.gaussian else None
+            if fused.gaussian and self._dls64 is None:
+                self._dls64 = torch.zeros(1, dtype=torch.float64, device=self.device)
+            self._kl_count = 1
+            kl_out = peer_slot if peer_slot is not None else (self._kl_glob if W > 1 else None)
+            ops.ppokl_loss_packed(idx, memory.n_size, memory.n_envs, mb["scal"], memory._dist, act_out, logstd, v, stats,
+                                  B * W, self.vf_coef, self.ent_coef, inv_batch, self._kl_coef_dev, self._kl_used,
+                                  self.target_kl, W == 1, B, b["kl_dact"], b["kl_dv"], self._dls64, self._scalars,
+                                  kl_sum_out=kl_out)
+            if fused.gaussian:
+                dls32 = fl.grad_views[[id(q) for q in fl.params].index(id(fused.policy.actor.logstd))]
+                fused.backward(b["kl_dact"], b["kl_dv"], self._dls64, dls32)
+            else:
+                fused.backward(b["kl_dact"], b["kl_dv"], softmax_pair=True)
+        else:
+            self._general_loss_backward(mb, fused, stats, B * W, inv_batch)
+            if W == 1:
+                ops.ppokl_kl_adapt(self._scalars[5:6], self._kl_coef_dev, self._kl_used, self.target_kl, B * self._kl_count)
+            else:
+                (peer_slot if peer_slot is not None else self._kl_glob).copy_(self._scalars[5:6])
+        if self._peer is not None:         # every rank takes the decision of the global minibatch's KL
+            ops.peer_allreduce_f64(self._peer, 1, self._kl_glob, offset=self._KL_SLOT)
+            ops.ppokl_kl_adapt(self._kl_glob, self._kl_coef_dev, self._kl_used, self.target_kl, B * W * self._kl_count)
+
+    def _general_loss_backward(self, mb, fused, stats, count, inv_batch):
+        fl = self._flat
+        adv = mb["adv"]
+        if stats is not None:
+            ops.normalize_adv(adv, stats, count)
+        if fused is not None:
+            act_out, v_pred = fused.forward(mb["obs"], refresh=not fused.splits_fresh)
+            a_dist = fused.dist_params(act_out)
+        else:
+            out = self.policy(mb["obs"])
+            a_dist, v_pred = out[1], out[2]
+        kind, p0, p1 = _dist_params(a_dist)
+        B = adv.shape[0]
+        v = v_pred.detach().contiguous()
+        dv = torch.empty_like(v)
+        kw = dict(clip_range=0.0, surr_coef=1.0, kl_coef=1.0, vf_coef=self.vf_coef, ent_coef=self.ent_coef,
+                  inv_batch=inv_batch, kl_coef_dev=self._kl_coef_dev)
+        if kind == "categorical":
+            self._kl_count = 1
+            logits = p0.detach().contiguous()
+            dlogits = torch.empty_like(logits)
+            ops.dist_loss_categorical(logits, mb["dist"], v, mb["act"].reshape(B), mb["ret"], adv, dlogits, dv, self._scalars,
+                                      **kw)
+            if fused is not None:
+                fused.backward(dlogits, dv, softmax_pair=logits.shape[1] == 2)
+            else:
+                fl.backward_into([p0, v_pred], [dlogits, dv])
+            return
+        mu = p0.detach().contiguous()
+        A = mu.shape[1]
+        self._kl_count = A
+        param = getattr(getattr(self.policy, "actor", None), "logstd", None)   # gaussian.py:25
+        direct = param is not None and param.requires_grad and param.numel() == A
+        logstd = param.detach() if direct else p1.detach().log().contiguous()
+        dmu = torch.empty_like(mu)
+        dls = torch.empty(A, dtype=torch.float64, device=mu.device)
+        ops.dist_loss_gaussian(mu, logstd, mb["dist"][:, :A].contiguous(), mb["dist"][:, A:].contiguous(), v,
+                               mb["act"].reshape(B, A), mb["ret"], adv, dmu, dls, dv, self._scalars, **kw)
+        if direct:
+            dls32 = fl.grad_views[[id(q) for q in fl.params].index(id(param))]
+            if fused is not None:
+                fused.backward(dmu, dv, dls, dls32)
+            else:
+                fl.backward_into([p0, v_pred], [dmu, dv])
+                dls32.copy_(dls)
+        else:
+            fl.backward_into([p0, v_pred, p1], [dmu, dv, (dls / p1.detach().double()).to(p1.dtype)])
+
+    def allreduce_grads(self):
+        super().allreduce_grads()
+        if self._peer is None:             # the KL sum of the global minibatch; the coefficient adapts in stage_optimizer
+            torch.distributed.all_reduce(self._kl_glob, group=self.process_group)
+
+    def stage_optimizer(self):
+        super().stage_optimizer()
+        if self.world_size > 1 and self._peer is None:
+            ops.ppokl_kl_adapt(self._kl_glob, self._kl_coef_dev, self._kl_used, self.target_kl,
+                               self._mb_rows * self.world_size * self._kl_count)
+
+    def info(self, batch_size):
+        """Host copy of the last update's log scalars: the reference learner's keys, `actor-loss` with the coefficient
+        that update used (ppokl_learner.py:36,52-61)."""
+        s = self._scalars.cpu().numpy()
+        kl = float(s[5]) / (batch_size * self._kl_count)
+        lr = self._native_lr()
+        return {"actor-loss": -float(s[0]) / batch_size + float(self._kl_used.item()) * kl, "critic-loss": float(s[1]) / batch_size,
+                "entropy": float(s[2]) / batch_size, "learning_rate": lr, "kl": kl, "predict_value": float(s[3]) / batch_size}
 
     @property
     def kl_coef(self):

@@ -48,10 +48,11 @@ def env_step(kind, state, rng, elapsed, ep_score, actions, obs, next_obs, rew, t
 def rollout_step(kind, act_param, logstd, val, seed, counter, offset, state, rng, elapsed, ep_score, obs, next_obs, rew,
                  term, trunc, reset_obs, ep_step_out, ep_score_out, ep_stats, max_steps, x_in, act_out, logp_out, obs_row,
                  act_row, rew_row, val_row, term_row, trunc_row, logp_row, rew_std=None, rew_clip=0.0, boot_src=None,
-                 boot_row=None, trig_cache=None, stats=None):
+                 boot_row=None, trig_cache=None, stats=None, dist_row=None):
     """sample + env step + store of one vector step in one launch (see xb_rollout_step in include/xb200.h).
     `stats` (dict, optional): running statistics carried by the launch — obs_in / obs_out (normaliser states), obs_dim,
-    obs_clip, ret_state, returns, gamma, mask_terminal, partials, ticket; `rew_std` is then also rewritten for the next step."""
+    obs_clip, ret_state, returns, gamma, mask_terminal, partials, ticket; `rew_std` is then also rewritten for the next step.
+    `dist_row` (optional, f32 [N, W]): receives the parameters of the distribution each action was drawn from."""
     N = elapsed.numel()
     st = stats or {}
     _lib.call("xb_rollout_step", kind, _p(act_param, F32), _p(logstd, F32), _p(val, F32), int(seed), _p(counter, I64),
@@ -64,7 +65,7 @@ def rollout_step(kind, act_param, logstd, val, seed, counter, offset, state, rng
               int(st.get("obs_dim", 0)), float(st.get("obs_clip", 0.0)), _p(st.get("ret_state"), F64),
               _p(rew_std if st.get("returns") is not None else None, F32), _p(st.get("returns"), F64),
               float(st.get("gamma", 0.0)), int(bool(st.get("mask_terminal", True))), _p(st.get("partials"), F64),
-              _p(st.get("ticket"), I32), _p(st.get("sums_out"), F64), N, _stream())
+              _p(st.get("ticket"), I32), _p(st.get("sums_out"), F64), _p(dist_row, F32), N, _stream())
 
 
 def eval_step(kind, act_param, logstd, key, step, state, rng, elapsed, ep_score, next_obs, trig_cache, max_steps, scores, count,
@@ -184,6 +185,22 @@ def dist_loss_gaussian(mu, logstd, old_mu, old_std, v_pred, act, ret, adv, dmu, 
 
 def kl_coef_adapt(scalars, kl_coef_dev, target_kl, count):
     _lib.call("xb_kl_coef_adapt", _p(scalars, F64), _p(kl_coef_dev, F32), float(target_kl), int(count), _stream())
+
+
+def ppokl_loss_packed(idx, T, N, scal, old_dist, act_out, logstd, v_pred, adv_stats, adv_count, vf_coef, ent_coef, inv_batch,
+                      kl_coef, kl_used, target_kl, adapt, kl_count, dact, dv, dlogstd, scalars, kl_sum_out=None):
+    """PPO-KL loss forward + backward on packed minibatch rows with the adaptive coefficient (xb_ppokl_loss_packed).
+    `old_dist`: the rollout's [T, N, 2] pairs; adapt=False leaves the coefficient to xb_ppokl_kl_adapt."""
+    gaussian = logstd is not None
+    _lib.call("xb_ppokl_loss_packed", _p(idx, I64), idx.numel(), int(T), int(N), _p(scal, F32), _p(old_dist, F32),
+              _p(act_out, F32), _p(logstd, F32), int(gaussian), _p(v_pred, F32), _p(adv_stats, F64), int(adv_count),
+              float(vf_coef), float(ent_coef), float(inv_batch), _p(kl_coef, F32), _p(kl_used, F32), float(target_kl),
+              int(bool(adapt)), int(kl_count), _p(kl_sum_out, F64), _p(dact, F32), _p(dv, F32), _p(dlogstd, F64), _p(scalars, F64), _stream())
+
+
+def ppokl_kl_adapt(kl_sum, kl_coef, kl_used, target_kl, count):
+    _lib.call("xb_ppokl_kl_adapt", _p(kl_sum, F64), _p(kl_coef, F32), _p(kl_used, F32), float(target_kl), int(count),
+              _stream())
 
 
 def pack_records(b_obs, b_act, b_logp, b_adv, b_ret, rec):
