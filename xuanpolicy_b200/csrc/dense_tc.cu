@@ -16,7 +16,9 @@
 //   warp 9      MMA issuer     : one thread issues tcgen05.mma.kind::tf32 (M=128, N<=256, K=8) x3 per k-step,
 //                                tcgen05.commit releases ring slots / publishes the accumulator
 //   warps 0-3   epilogue       : tcgen05.ld the 128 x N fp32 accumulator (double-buffered in TMEM so the next
-//                                tile's MMAs overlap), bias + LeakyReLU (+ fused narrow head) / activation mask, store
+//                                tile's MMAs overlap), bias + LeakyReLU (+ fused narrow head) / activation mask, store;
+//                                TS-form forward without a stored Y: the operand warps take half of each tile's columns
+//                                (epilogue_share) once they have converted the next tile's k-blocks
 #include <stdlib.h>
 #include <string.h>
 
@@ -212,14 +214,42 @@ struct EpiCtx {
     int sign_ld;
     const uint32_t* h1_signs;   // DGRAD: nullable trunk sign words [M][4] (N = 128): the mask without the H1 tiles
     double* red;       // shared memory [4 warps][8] for the per-CTA loss sums
+    int epi_sets = 1;           // warp sets sharing each tile's columns (TS FWD without a stored Y: 1 + operand-warp sets)
+    uint32_t head_terms = 0;    // epi_sets > 1: shared memory [N/32 - kEpiOwnChunks][8][BM] float2 head terms of the other sets
 #ifdef XB_DENSE_TS
     long long* ts;
 #endif
 };
 
+// FWD, 4-column group q of an accumulator chunk: bias + LeakyReLU in place, its 4 activation sign bits into `sign_word`
+__device__ __forceinline__ void bias_leaky_group(float4& f, const float* b, float slope, int q, uint32_t& sign_word) {
+    f.x += b[0]; f.y += b[1]; f.z += b[2]; f.w += b[3];
+    sign_word |= (f.x > 0.f ? 1u : 0u) << (4 * q) | (f.y > 0.f ? 2u : 0u) << (4 * q) |
+                 (f.z > 0.f ? 4u : 0u) << (4 * q) | (f.w > 0.f ? 8u : 0u) << (4 * q);
+    f.x = f.x > 0.f ? f.x : f.x * slope;
+    f.y = f.y > 0.f ? f.y : f.y * slope;
+    f.z = f.z > 0.f ? f.z : f.z * slope;
+    f.w = f.w > 0.f ? f.w : f.w * slope;
+}
+// FWD head term of one 4-column group: both the owner warp and the operand-warp sets evaluate it through this one expression,
+// so its rounding (and the FMA contraction) is the same wherever a group is computed
+__device__ __forceinline__ float head_term(const float4& f, const float* w) {
+    return f.x * w[0] + f.y * w[1] + f.z * w[2] + f.w * w[3];
+}
+
+// Split FWD epilogue (TS kernel, no stored Y): the epilogue warp of lane quarter lq owns the first N/64 chunks of each tile,
+// the operand warps 4 + lq (set 1) and 8 + lq (set 2) take the remaining chunks alternately.  Named barriers per lane quarter:
+// kEpiBarFull + lq (the other sets' head terms of a tile are in shared memory), kEpiBarEmpty + lq (the owner has read them).
+constexpr int kEpiBarFull = 1, kEpiBarEmpty = 5;
+template <int N>
+__host__ __device__ constexpr int epi_own_chunks() { return N / 64 > 0 ? N / 64 : 1; }
+template <int N>
+__host__ __device__ constexpr int epi_sets_of() { return 1 + (N / 32 - epi_own_chunks<N>() < 2 ? N / 32 - epi_own_chunks<N>() : 2); }
+
 template <int N, int MODE>
 __device__ __forceinline__ void epilogue_warp(const EpiCtx& c, int warp, int lane) {
     constexpr int kChunks = N / 32;
+    const int own_chunks = c.epi_sets > 1 ? epi_own_chunks<N>() : kChunks;
     constexpr uint32_t kSub = 32 * 128;                               // one warp's sub-tile: 32 rows x 128 B
     const uint32_t bar_h1 = c.bar_h1w + warp * 16;                    // 2 barriers per warp
     uint32_t lt = 0, g = 0;
@@ -261,7 +291,7 @@ __device__ __forceinline__ void epilogue_warp(const EpiCtx& c, int warp, int lan
         const uint32_t taddr = c.tmem_base + ((uint32_t)(warp * 32) << 16) + acc * N;
         float h0 = 0.f, h1 = 0.f;
 #pragma unroll 1
-        for (int cc = 0; cc < kChunks; ++cc, ++g) {
+        for (int cc = 0; cc < own_chunks; ++cc, ++g) {
 #ifdef XB_DENSE_TS
             if (threadIdx.x == 0 && c.ts && blockIdx.x == 0 && lt < 64) c.ts[(3 * 64 + lt) * 8 + 1 + cc] = clock64();
 #endif
@@ -304,16 +334,10 @@ __device__ __forceinline__ void epilogue_warp(const EpiCtx& c, int warp, int lan
                                        __uint_as_float(v[4 * q + 2]), __uint_as_float(v[4 * q + 3]));
                 if (MODE == MODE_FWD) {
                     const float* b = c.sf + cc * 32 + 4 * q;
-                    f.x += b[0]; f.y += b[1]; f.z += b[2]; f.w += b[3];
-                    sign_word |= (f.x > 0.f ? 1u : 0u) << (4 * q) | (f.y > 0.f ? 2u : 0u) << (4 * q) |
-                                 (f.z > 0.f ? 4u : 0u) << (4 * q) | (f.w > 0.f ? 8u : 0u) << (4 * q);
-                    f.x = f.x > 0.f ? f.x : f.x * c.slope;
-                    f.y = f.y > 0.f ? f.y : f.y * c.slope;
-                    f.z = f.z > 0.f ? f.z : f.z * c.slope;
-                    f.w = f.w > 0.f ? f.w : f.w * c.slope;
+                    bias_leaky_group(f, b, c.slope, q, sign_word);
                     const float* w = b + N;
-                    h0 += f.x * w[0] + f.y * w[1] + f.z * w[2] + f.w * w[3];
-                    h1 += f.x * w[N] + f.y * w[N + 1] + f.z * w[N + 2] + f.w * w[N + 3];
+                    h0 += head_term(f, w);
+                    h1 += head_term(f, w + N);
                 } else if (mask_bits) {
                     f.x *= ((hx >> q) & 1u) ? 1.f : c.slope;
                     f.y *= ((hy >> q) & 1u) ? 1.f : c.slope;
@@ -338,6 +362,18 @@ __device__ __forceinline__ void epilogue_warp(const EpiCtx& c, int warp, int lan
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(c.bar_tempty + 8 * acc);
+        if (MODE == MODE_FWD && c.epi_sets > 1) {     // the other sets' head terms, added in column order after this warp's own
+            constexpr int kTerms = (kChunks - epi_own_chunks<N>()) * 8;
+            bar_sync_named(kEpiBarFull + warp, 32 * c.epi_sets);
+            const uint32_t tb = c.head_terms + (uint32_t)(warp * 32 + lane) * 8;
+#pragma unroll
+            for (int j = 0; j < kTerms; ++j) {
+                const float2 t = lds64(tb + j * (BM * 8));
+                h0 += t.x;
+                h1 += t.y;
+            }
+            if (tile + c.tile_step < c.n_tiles) bar_arrive_named(kEpiBarEmpty + warp, 32 * c.epi_sets);
+        }
 #ifdef XB_DENSE_TS
         if (threadIdx.x == 0 && c.ts && blockIdx.x == 0 && lt < 64) c.ts[(3 * 64 + lt) * 8 + 7] = clock64();
 #endif
@@ -409,6 +445,43 @@ __device__ __forceinline__ void epilogue_warp(const EpiCtx& c, int warp, int lan
             if (lane == 0) c.red[warp * 8 + k] = v;
         }
     }
+}
+
+// Split FWD epilogue, operand-warp side: set `set` (1 or 2) of lane quarter lq takes chunks epi_own_chunks + set - 1, + 2, ...
+// of tile `tile` (its lt-th): bias + LeakyReLU, sign words, and the head terms of every 4-column group into `head_terms`, where
+// the owner warp adds them to its row sums in column order.  Called after the operand warps have converted the next tile's
+// k-blocks, so the MMA stream does not wait on it.
+template <int N>
+__device__ __forceinline__ void epilogue_share(const EpiCtx& c, int set, int lq, int lane, int64_t tile, uint32_t lt) {
+    constexpr int kChunks = N / 32, kOwn = epi_own_chunks<N>();
+    const uint32_t acc = lt & 1, tph = (lt >> 1) & 1;
+    const int64_t row = tile * BM + lq * 32 + lane;
+    if (lt > 0) bar_sync_named(kEpiBarEmpty + lq, 32 * c.epi_sets);     // the owner has read the previous tile's terms
+    mbar_wait(c.bar_tfull + 8 * acc, tph);
+    tc_fence_after();
+    const uint32_t taddr = c.tmem_base + ((uint32_t)(lq * 32) << 16) + acc * N;
+#pragma unroll 1
+    for (int cc = kOwn + set - 1; cc < kChunks; cc += 2) {
+        uint32_t v[32];
+        tmem_ld_32x32(taddr + cc * 32, v);
+        const uint32_t tb = c.head_terms + ((uint32_t)((cc - kOwn) * 8 * BM) + lq * 32 + lane) * 8;
+        tmem_ld_wait();
+        uint32_t sign_word = 0u;
+#pragma unroll
+        for (int q = 0; q < 8; ++q) {
+            float4 f = make_float4(__uint_as_float(v[4 * q]), __uint_as_float(v[4 * q + 1]),
+                                   __uint_as_float(v[4 * q + 2]), __uint_as_float(v[4 * q + 3]));
+            const float* b = c.sf + cc * 32 + 4 * q;
+            bias_leaky_group(f, b, c.slope, q, sign_word);
+            const float* w = b + N;
+            sts64(tb + q * (BM * 8), head_term(f, w), head_term(f, w + N));
+        }
+        if (c.sign_out && row < c.M) c.sign_out[row * c.sign_ld + cc] = sign_word;
+    }
+    tc_fence_before();
+    __syncwarp();
+    if (lane == 0) mbar_arrive(c.bar_tempty + 8 * acc);
+    bar_arrive_named(kEpiBarFull + lq, 32 * c.epi_sets);
 }
 
 // After the CTA-wide barrier that follows the epilogue: CTA sums -> global partials -> the last CTA adds all CTAs' partials
@@ -986,6 +1059,9 @@ __global__ void __launch_bounds__(kThreads, 1)
     const float* e_head_b = sel ? p.head_b1 : p.head_b;
     const int e_n_head = sel ? p.n_head1 : p.n_head;
     float* e_head_out = sel ? p.head_out1 : p.head_out;
+    // FWD without a stored Y (rollout, rank-1 training): the operand warps take part of every tile's epilogue, with the
+    // idle staging ring holding their head terms
+    const int epi_sets = (MODE == MODE_FWD && p.Y == nullptr) ? epi_sets_of<N>() : 1;
 
     if (threadIdx.x == 0) {
         const int n_conv = p.alt_groups ? kOperandWarps / 2 : kOperandWarps;    // operand warps per k-block
@@ -1003,7 +1079,7 @@ __global__ void __launch_bounds__(kThreads, 1)
         }
         for (int a = 0; a < 2; ++a) {
             mbar_init(bar_tfull + 8 * a, 1);
-            mbar_init(bar_tempty + 8 * a, 4);
+            mbar_init(bar_tempty + 8 * a, 4 * epi_sets);
         }
         for (int a = 0; a < 8; ++a) mbar_init(bar_h1w + 8 * a, 1);
         mbar_init(bar_bfull, 1);
@@ -1046,6 +1122,27 @@ __global__ void __launch_bounds__(kThreads, 1)
         XB_STEP_STAMP(sts, 202);
         pdl_trigger();
     }
+    // epilogue context: warps 0-3, and with epi_sets > 1 the operand warps' share of it (built inside each role's branch)
+    auto epi_ctx = [&]() {
+        EpiCtx c;
+        c.tmem_base = tmem_base; c.bar_tfull = bar_tfull; c.bar_tempty = bar_tempty; c.bar_h1w = bar_h1w;
+        c.out_ring = out_ring; c.h1_ring = h1_ring; c.O = O; c.HB = HB;
+        c.tile0 = tile0; c.tile_step = tile_step; c.n_tiles = n_tiles; c.M = p.M;
+        c.map_out = map_out; c.map_h1 = map_h1; c.sf = sf; c.slope = p.slope;
+        c.n_head = e_n_head; c.head_b = e_head_b; c.head_out = e_head_out;
+        c.store_y = MODE != MODE_FWD || p.Y != nullptr;
+        c.n_off = n_off;
+        c.loss = p.loss; c.sel = sel; c.red = reinterpret_cast<double*>(misc_ptr + kLossRedOff);
+        c.sign_out = (MODE == MODE_FWD && p.sign_out) ? p.sign_out + sel * (N / 32) : nullptr;
+        c.sign_ld = p.sign_ld;
+        c.h1_signs = (MODE == MODE_DGRAD && N == 128 && p.n_split <= 1) ? p.h1_signs : nullptr;
+        c.epi_sets = epi_sets;
+        c.head_terms = out_ring;      // (unused staging when Y is not stored: [N/32 - own chunks][8][128] float2 <= kATile)
+#ifdef XB_DENSE_TS
+        c.ts = p.ts;
+#endif
+        return c;
+    };
 
     if (warp == kProducerWarp) {
         // ============================================================ TMA producer: the whole warp walks the loop, one elected
@@ -1145,6 +1242,9 @@ __global__ void __launch_bounds__(kThreads, 1)
         const bool from_bits = MODE == MODE_DGRAD && p.signs != nullptr;    // activation sign words instead of activation tiles
         const bool from_obs = (MODE == MODE_FWD && p.obs != nullptr) || from_bits;   // = no raw A ring: the operand is generated
         const bool alt = p.alt_groups != 0;     // ch is then the GROUP (k-block parity) instead of the column half
+        // epilogue set 1 + ch: its share of tile t runs once tile t + 1's k-blocks are converted (the last tile's at the end)
+        const bool epi_share = MODE == MODE_FWD && 1 + ch < epi_sets;
+        uint32_t elt = 0;
         if (!from_obs && !alt && tile0 < n_tiles) XB_TRYWAIT_ISSUE(xb_pf, bar_full + 8 * s, ph);    // first stage's phase check
         for (int64_t tile = tile0; tile < n_tiles; tile += tile_step) {
             float d00 = 0.f, d01 = 0.f, d10 = 0.f, d11 = 0.f;   // DGRAD: dL/d(head outputs) of this row
@@ -1310,26 +1410,13 @@ __global__ void __launch_bounds__(kThreads, 1)
                 if (!from_obs) { s = ns; ph = nph; }
                 if (++ta == kTA) { ta = 0; aph ^= 1; }
             }
+            if (epi_share && tile != tile0) epilogue_share<N>(epi_ctx(), 1 + ch, lq, lane, tile - tile_step, elt++);
         }
+        if (epi_share && tile0 < n_tiles) epilogue_share<N>(epi_ctx(), 1 + ch, lq, lane, tile0 + (int64_t)elt * tile_step, elt);
     } else {
         // ============================================================ epilogue warps 0-3
-        EpiCtx c;
-        c.tmem_base = tmem_base; c.bar_tfull = bar_tfull; c.bar_tempty = bar_tempty; c.bar_h1w = bar_h1w;
-        c.out_ring = out_ring; c.h1_ring = h1_ring; c.O = O; c.HB = HB;
-        c.tile0 = tile0; c.tile_step = tile_step; c.n_tiles = n_tiles; c.M = p.M;
-        c.map_out = map_out; c.map_h1 = map_h1; c.sf = sf; c.slope = p.slope;
-        c.n_head = e_n_head; c.head_b = e_head_b; c.head_out = e_head_out;
-        c.store_y = MODE != MODE_FWD || p.Y != nullptr;
-        c.n_off = n_off;
-        c.loss = p.loss; c.sel = sel; c.red = reinterpret_cast<double*>(misc_ptr + kLossRedOff);
-        c.sign_out = (MODE == MODE_FWD && p.sign_out) ? p.sign_out + sel * (N / 32) : nullptr;
-        c.sign_ld = p.sign_ld;
-        c.h1_signs = (MODE == MODE_DGRAD && N == 128 && p.n_split <= 1) ? p.h1_signs : nullptr;
-#ifdef XB_DENSE_TS
-        c.ts = p.ts;
-#endif
         if (MODE == MODE_FWD) prep_dgrad_operand(p, threadIdx.x);      // idle until the first accumulator is ready
-        epilogue_warp<N, MODE>(c, warp, lane);
+        epilogue_warp<N, MODE>(epi_ctx(), warp, lane);
     }
 
     if (threadIdx.x == 0) XB_TS(0, 63, 0);

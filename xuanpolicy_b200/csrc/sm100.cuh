@@ -223,8 +223,19 @@ __device__ __forceinline__ void sts128(uint32_t addr, float4 v) {
     // read-only tables (bias, head weights) may be scheduled across it
     asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w));
 }
+__device__ __forceinline__ float2 lds64(uint32_t addr) {
+    float2 v;
+    asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(addr));
+    return v;
+}
+__device__ __forceinline__ void sts64(uint32_t addr, float x, float y) {
+    asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(addr), "f"(x), "f"(y));
+}
 __device__ __forceinline__ void bar_sync_named(int id, int nthreads) {
     asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+}
+__device__ __forceinline__ void bar_arrive_named(int id, int nthreads) {   // signals without waiting (release ordering)
+    asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 
 }  // namespace sm100
