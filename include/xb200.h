@@ -36,6 +36,14 @@ extern "C" {
  * observation = the last 4 frames (oldest first), 8 floats = TWO float4 per row; state fp64 [8][N] = (position, velocity,
  * frame t-3, frame t-2, frame t-1); same physics, action int64 {0,1,2}, limit 200 */
 #define XB_ENV_MOUNTAINCAR_STACK4 4
+/* gym:MountainCarContinuous-v0 (gym's bare Continuous_MountainCarEnv): state (position, velocity), action float32 force
+ * (clipped to [-1, 1] for the physics; the reward's penalty takes the unclipped action), limit 999; the state is rounded to
+ * float32 at the end of every step, as gym stores it (the fp64 slots hold the rounded values) */
+#define XB_ENV_MOUNTAINCAR_CONTINUOUS 5
+/* MountainCarContinuous-v0 as the reference's make_envs builds it: the 4-frame stack of XB_ENV_MOUNTAINCAR_STACK4 (every id
+ * containing "MountainCar" gets it, gym_env.py:50-83) over XB_ENV_MOUNTAINCAR_CONTINUOUS: 8 floats = TWO float4 per row,
+ * state fp64 [8][N] in the same layout; action float32, limit 999 */
+#define XB_ENV_MOUNTAINCAR_CONTINUOUS_STACK4 6
 
 #define XB_E_BADARG (-1)
 #define XB_E_UNSUPPORTED (-2)
@@ -58,9 +66,9 @@ const char* xb_error_string(int code);
  *           Gym_Env.reset / step                xuance/environment/gym/gym_env.py:36-49
  *           gym 0.26.2 CartPoleEnv / PendulumEnv / TimeLimit / np_random (third party, restated: SURVEY.md App. A/B)
  *
- * state     fp64 [S][N] (SoA; S = 4 CartPole / Acrobot, 2 Pendulum / MountainCar, 8 MountainCar 4-frame stack)
+ * state     fp64 [S][N] (SoA; S = 4 CartPole / Acrobot, 2 Pendulum / MountainCar (both), 8 MountainCar 4-frame stacks)
  * obs       f32 [N][4] rows (one float4 per env); Acrobot-v1: [N][8] (two float4: cos t1, sin t1, cos t2, sin t2 | dt1, dt2, 0, 0);
- *           MountainCar 4-frame stack: [N][8] (p, v of frames t-3, t-2 | t-1, t)
+ *           MountainCar 4-frame stacks (discrete and continuous): [N][8] (p, v of frames t-3, t-2 | t-1, t)
  * rng       u64  [4][N] (SoA) numpy PCG64: state_hi, state_lo, inc_hi, inc_lo
  * elapsed   i32  [N]    TimeLimit._elapsed_steps == Gym_Env._episode_step
  * ep_score  fp64 [N]    Gym_Env._episode_score
@@ -72,7 +80,7 @@ int xb_env_reset(int env_kind, double* state, uint64_t* rng, int32_t* elapsed, d
                  int n_draws, int64_t N, xb_stream_t stream);
 
 /* One vector step with auto-reset.
- * actions      int64 [N] (CartPole) or float32 [N] (Pendulum)
+ * actions      int64 [N] (CartPole, MountainCar, Acrobot) or float32 [N] (Pendulum, MountainCarContinuous)
  * obs          f32 [N][4]  observation after the step: the TERMINAL observation for finished envs (buf_obs, :210)
  * next_obs     f32 [N][4]  nullable; obs with finished envs replaced by their reset observation (what the policy sees next)
  * rew          f32 [N];  term, trunc  u8 [N]
@@ -348,7 +356,8 @@ int xb_bias_act_fwd(float* y, const float* bias, float slope, int64_t B, int H, 
  * (PPOCLIP_Agent._action ppoclip_agent.py:50-57; DummyVecEnv_Gym.step_wait gym_vec_env.py:200-212;
  * DummyOnPolicyBuffer.store memory_tools.py:196-204).  CartPole-v1 / MountainCar-v0 (both forms) / Acrobot-v1: act_param = logits
  * [N][2] / [N][3] / [N][3], act_out int64 [N]; wide-row envs (Acrobot, MountainCar stack): x_in / obs / obs_row are [N][8];
- * Pendulum-v1: act_param = mu [N][1], logstd [1], act_out f32 [N].  x_in = the observations the action was computed
+ * Pendulum-v1 / MountainCarContinuous-v0 (both forms; the stack has 8-float rows): act_param = mu [N][1], logstd [1],
+ * act_out f32 [N].  x_in = the observations the action was computed
  * from (stored as the transition's obs); all other arguments as in xb_env_step / xb_store.  Physics and store are
  * bit-identical to the three separate calls; the sampled action may differ from xb_sample_* in the last ulp of the
  * transcendental functions (this translation unit is built without FMA contraction).
@@ -373,7 +382,7 @@ int xb_bias_act_fwd(float* y, const float* bias, float slope, int64_t B, int H, 
  *     n finished) are written there INSTEAD of being merged (obs_state_out / ret_state unused); exchange them across ranks
  *     (xb_peer_allreduce_merge, or xb_peer_allreduce_f64 and xb_rms_merge_sums).
  * dist_row (nullable, f32 [N][W], PPO-KL's `{"old_dist": dists}`): row t of the rollout's old-distribution array receives the
- *   parameters the action was drawn from: the W = 2 / 3 logits, or (mu, std = exp(logstd)) for Pendulum-v1 (W = 2).
+ *   parameters the action was drawn from: the W = 2 / 3 logits, or (mu, std = exp(logstd)) for the Box-action envs (W = 2).
  * ---------------------------------------------------------------------------------------------------------- */
 int xb_rollout_step(int env_kind, const float* act_param, const float* logstd, const float* val, uint64_t seed,
                     const uint64_t* counter_dev, uint64_t offset, double* state, uint64_t* rng, int32_t* elapsed,
@@ -392,7 +401,7 @@ int xb_rollout_step(int env_kind, const float* act_param, const float* logstd, c
  * ["episode_score"])` for every finished env, and the `obs_rms.update(obs)` of the next loop iteration (:126).
  *   act_param / logstd  policy outputs as in xb_rollout_step; the action is drawn with Philox keyed by *key (u64 [1]) at
  *                       counter (env, *step); the launch adds 1 to *step (u64 [1]).  act_tape (nullable): the actions are also
- *                       written to row *step of [tape_steps][N] (int64, Pendulum float32) while *step < tape_steps.
+ *                       written to row *step of [tape_steps][N] (int64; float32 for a Box action) while *step < tape_steps.
  *   state .. ep_score   env state as in xb_env_step; next_obs f32 [N][4] or [N][8] receives the observation the policy acts
  *                       on next (reset observation for finished envs); trig_cache as in xb_rollout_step.
  *   scores / count      episode queue fp64 [cap] and its length (int64 [1]): the final ep_score of every env that finished in

@@ -6,8 +6,9 @@
 Prints one JSON line per configuration (rank 0):
   * ppg_cartpole / ppg_pendulum — PPG_Agent at the ppg yaml defaults (n_steps 256, policy / value / aux epochs 4 / 8 / 8,
     use_obsnorm / use_rewnorm on) with 4096 envs on EVERY rank (weak scaling);
-  * ppo_acrobot / ppo_mountaincar — PPOCLIP_Agent at bench.py's C3 shape (65536 envs in total, split over the ranks: strong
-    scaling; horizon 256, 8 epochs x 8 minibatches, MLP 128) with both normalisers, on the 6- and 8-float observation rows;
+  * ppo_acrobot / ppo_mountaincar / ppo_mountaincar_continuous — PPOCLIP_Agent at bench.py's C3 shape (65536 envs in total,
+    split over the ranks: strong scaling; horizon 256, 8 epochs x 8 minibatches, MLP 128) with both normalisers, on the 6-
+    and 8-float observation rows (the last one with a Gaussian action);
   * ppokl_cartpole / ppo_cartpole — PPOKL_Agent and its PPO-Clip twin at the same C3 shape (no normalisers), target_kl 0.01;
   * ppokl_pendulum / ppo_pendulum — the same pair at bench.py's C2 shape (4096 envs per GPU x horizon 128, 8 x 8 minibatches,
     MLP 128, both normalisers on).
@@ -33,6 +34,7 @@ CONFIGS = {
     "ppg_pendulum": dict(agent="ppg", env_id="Pendulum-v1", envs=4096, strong=False),
     "ppo_acrobot": dict(agent="ppo", env_id="Acrobot-v1", envs=65536, strong=True),
     "ppo_mountaincar": dict(agent="ppo", env_id="MountainCar-v0", envs=65536, strong=True),
+    "ppo_mountaincar_continuous": dict(agent="ppo", env_id="MountainCarContinuous-v0", envs=65536, strong=True),
     "ppokl_cartpole": dict(agent="ppokl", env_id="CartPole-v1", envs=65536, strong=True, T=256, norm=False),
     "ppo_cartpole": dict(agent="ppo", env_id="CartPole-v1", envs=65536, strong=True, T=256, norm=False),
     "ppokl_pendulum": dict(agent="ppokl", env_id="Pendulum-v1", envs=4096, strong=False, T=128, norm=True),

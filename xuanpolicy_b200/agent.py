@@ -159,7 +159,8 @@ class DeviceEvaluator:
         self.partials, self.workspace = torch.zeros(20 * ctas, **f64), torch.zeros(2 + ctas, **i64)
         self.tape = None
         if tape_steps:                  # test hook: the sampled actions, row = evaluation step
-            self.tape = torch.zeros((tape_steps, N), dtype=torch.float32 if envs._kind == 1 else torch.int64, device=dev)
+            act_dtype = torch.float32 if ops.continuous_kind(envs._kind) else torch.int64
+            self.tape = torch.zeros((tape_steps, N), dtype=act_dtype, device=dev)
         self.local_count = self.score_step = self.record = None
         if peer is not None:
             self.local_count = torch.zeros(1, **i64)

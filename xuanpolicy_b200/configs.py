@@ -1,4 +1,4 @@
-"""Default PPO-Clip hyper-parameters for the two classic-control tasks, as a Namespace shaped like the one the
+"""Default PPO-Clip hyper-parameters for the classic-control tasks, as a Namespace shaped like the one the
 reference builds from YAML (xuance/common/common_tools.py:32-83).  Values restate
 xuance/configs/ppo/classic_control/CartPole-v1.yaml and Pendulum-v1.yaml (identical except env_id/policy);
 `use_obsnorm` / `use_rewnorm` default to False here because the BASELINE configs are measured without them (the yaml
@@ -17,9 +17,12 @@ _COMMON = dict(
 
 
 def ppo_config(env_id, **overrides):
+    """`policy`: "Gaussian_AC" for an env with a Box action (Pendulum-v1, MountainCarContinuous-v0), "Categorical_AC"
+    otherwise (ids without a device kernel included)."""
+    from .vec_env import SPECS, continuous_actions
     cfg = dict(_COMMON)
     cfg["env_id"] = env_id
-    cfg["policy"] = "Gaussian_AC" if env_id == "Pendulum-v1" else "Categorical_AC"
+    cfg["policy"] = "Gaussian_AC" if env_id in SPECS and continuous_actions(env_id) else "Categorical_AC"
     cfg.update(overrides)
     return Namespace(**cfg)
 

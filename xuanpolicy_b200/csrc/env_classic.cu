@@ -1,9 +1,11 @@
-// env_classic.cu — batched CartPole-v1 / Pendulum-v1 / MountainCar-v0 (gym's, and the reference's 4-frame wrapper) /
-// Acrobot-v1 step + auto-reset, one thread per environment.
+// env_classic.cu — batched CartPole-v1 / CartPole-v0 / Pendulum-v1 / MountainCar-v0 / MountainCarContinuous-v0 (gym's, and
+// the reference's 4-frame wrapper of each) / Acrobot-v1 step + auto-reset, one thread per environment: gym 0.26.2's six
+// classic-control ids (CartPole-v0 is the CartPole functor with a 200-step limit).
 //
 // Replaces the per-env Python loop of DummyVecEnv_Gym.step_wait (xuance/environment/gym/gym_vec_env.py:201-212)
 // over Gym_Env.step (xuance/environment/gym/gym_env.py:43-49) over gym 0.26.2's CartPoleEnv / PendulumEnv /
-// TimeLimit (third party, not vendored; equations per SURVEY.md App. A, reset stream per App. B).
+// MountainCarEnv / Continuous_MountainCarEnv / AcrobotEnv / TimeLimit (third party, not vendored; equations per SURVEY.md
+// App. A, reset stream per App. B).
 //
 // Bit-exactness contract: fp64 state lives in registers for the whole step; every fp64 operation is an
 // individually rounded __dadd_rn/__dmul_rn/__ddiv_rn (no FMA contraction — this TU is also built with
@@ -175,22 +177,64 @@ struct MountainCar {
     }
 };
 
-// MountainCar-v0 AS THE REFERENCE DEFINES IT: `make_envs` wraps every env id containing "MountainCar" in
-// xuance/environment/gym/gym_env.py:50-83 `MountainCar(Gym_Env)` (selected at xuance/environment/__init__.py:66-67): the
-// observation is the concatenation of the last FOUR frames, oldest first (`LazyFrames(list(self.frames))`, deque maxlen 4,
-// gym_env.py:227-254), shape (8,); `reset()` fills all four frames with the reset observation (:67-68).  The three previous
-// float32 frames ride in the fp64 state slots 2..7 (exact), so the generic step / reset / rollout kernels need no extra
-// argument; slots 0..1 are gym's (position, velocity) with the physics of `MountainCar` above, bit for bit.
-struct MountainCarStack {
+// gym 0.26.2 Continuous_MountainCarEnv (gym/envs/classic_control/continuous_mountain_car.py), TimeLimit 999.  Operation
+// order of step(), with the pinned numpy 1.21.6's promotion (a float32 scalar combined with a Python float or int gives
+// float64, so every operation below is fp64):
+//   force = min(max(action[0], -1.0), 1.0)
+//   velocity += force * 0.0015 - 0.0025 * math.cos(3 * position)
+//   velocity = clip(velocity, -0.07, 0.07); position += velocity; position = clip(position, -1.2, 0.6)
+//   if position == -1.2 and velocity < 0: velocity = 0
+//   terminated = position >= 0.45 and velocity >= 0            (on the fp64 values)
+//   reward = (100.0 if terminated else 0) - math.pow(action[0], 2) * 0.1      (the UNCLIPPED action)
+//   state = np.array([position, velocity], dtype=np.float32)  (obs = state)
+// reset(): state = [uniform(-0.6, -0.4), 0] as float64, obs = float32(state).  The fp64 slots hold (double)(float)x after a
+// step (exact), so the first step of an episode runs on the unrounded draw and every later one on the rounded state, like
+// gym.  pow(a, 2) of a float32 a is a*a exactly in fp64 (48 significant bits).
+struct MountainCarContinuous {
+    static constexpr int kObsVec = 1;   // float4s per observation row
+    static constexpr bool kTrigCache = false;
+    static constexpr int S = 2;
+    typedef float action_t;
+    static constexpr bool kDiscrete = false;
+    static constexpr int kActions = 1;
+    __device__ static void draw(double (&st)[2], Pcg64& g) { MountainCar::draw(st, g); }
+    __device__ static float4 observe(const double (&st)[2]) { return make_float4((float)st[0], (float)st[1], 0.0f, 0.0f); }
+    __device__ static double step(double (&st)[2], action_t action, bool& terminated) {
+        const double power = 0.0015, max_speed = 0.07, min_pos = -1.2, max_pos = 0.6, goal_pos = 0.45;
+        double position = st[0], velocity = st[1];
+        const double a = (double)action;
+        const double force = a < -1.0 ? -1.0 : (a > 1.0 ? 1.0 : a);
+        double s, c;
+        sincos_cr(__dmul_rn(3.0, position), &s, &c);
+        velocity = __dadd_rn(velocity, __dsub_rn(__dmul_rn(force, power), __dmul_rn(0.0025, c)));
+        velocity = velocity < -max_speed ? -max_speed : (velocity > max_speed ? max_speed : velocity);
+        position = __dadd_rn(position, velocity);
+        position = position < min_pos ? min_pos : (position > max_pos ? max_pos : position);
+        if (position == min_pos && velocity < 0.0) velocity = 0.0;
+        terminated = position >= goal_pos && velocity >= 0.0;
+        st[0] = (double)(float)position; st[1] = (double)(float)velocity;
+        return __dsub_rn(terminated ? 100.0 : 0.0, __dmul_rn(__dmul_rn(a, a), 0.1));
+    }
+};
+
+// The 4-frame stack the reference's `make_envs` puts around every env id containing "MountainCar": xuance/environment/gym/
+// gym_env.py:50-83 `MountainCar(Gym_Env)` (selected at xuance/environment/__init__.py:66-67): the observation is the
+// concatenation of the last FOUR frames, oldest first (`LazyFrames(list(self.frames))`, deque maxlen 4, gym_env.py:227-254),
+// shape (8,); `reset()` fills all four frames with the reset observation (:67-68).  The three previous float32 frames ride in
+// the fp64 state slots 2..7 (exact), so the generic step / reset / rollout kernels need no extra argument; slots 0..1 are the
+// bare env's (position, velocity) with its physics, bit for bit.
+template <class Base>
+struct FrameStack4 {
+    static_assert(Base::S == 2 && Base::kObsVec == 1 && !Base::kTrigCache, "a frame is the two-slot state of the bare env");
     static constexpr int kObsVec = 2;
     static constexpr bool kTrigCache = false;
     static constexpr int S = 8;
-    typedef int64_t action_t;
-    static constexpr bool kDiscrete = true;
-    static constexpr int kActions = 3;
+    typedef typename Base::action_t action_t;
+    static constexpr bool kDiscrete = Base::kDiscrete;
+    static constexpr int kActions = Base::kActions;
     __device__ static void draw(double (&st)[8], Pcg64& g) {
         double b[2];
-        MountainCar::draw(b, g);
+        Base::draw(b, g);
         st[0] = b[0]; st[1] = b[1];
 #pragma unroll
         for (int k = 0; k < 3; ++k) {           // for i in range(num_stack): frames.append(obs)
@@ -205,13 +249,16 @@ struct MountainCarStack {
     __device__ static double step(double (&st)[8], action_t action, bool& terminated) {
         double b[2] = {st[0], st[1]};
         const float fp = (float)b[0], fv = (float)b[1];       // the frame appended by the previous step / reset
-        const double r = MountainCar::step(b, action, terminated);
+        const double r = Base::step(b, action, terminated);
         st[2] = st[4]; st[3] = st[5]; st[4] = st[6]; st[5] = st[7];
         st[6] = (double)fp; st[7] = (double)fv;
         st[0] = b[0]; st[1] = b[1];
         return r;
     }
 };
+// MountainCar-v0 and MountainCarContinuous-v0 as the reference defines them (named types: the kernels' symbols stay readable)
+struct MountainCarStack : FrameStack4<MountainCar> {};
+struct MountainCarContinuousStack : FrameStack4<MountainCarContinuous> {};
 
 // gym 0.26.2 AcrobotEnv (gym/envs/classic_control/acrobot.py; xuance config xuance/configs/ppo/classic_control/Acrobot-v1.yaml),
 // "book" dynamics, TimeLimit 500, restated from the published algorithm (operation order = Python's left-to-right):
@@ -858,6 +905,12 @@ __global__ void sincos_kernel(const double* __restrict__ x, double* __restrict__
     if (i < n) sincos_cr(x[i], &s[i], &c[i]);
 }
 
+// the kinds with a Box action (float32 actions; the policy outputs mu [N][1] and a log-std)
+static inline bool continuous_kind(int env_kind) {
+    return env_kind == XB_ENV_PENDULUM || env_kind == XB_ENV_MOUNTAINCAR_CONTINUOUS ||
+           env_kind == XB_ENV_MOUNTAINCAR_CONTINUOUS_STACK4;
+}
+
 static inline int env_block(int64_t N) {
     // small batches are latency bound: spread them over more SMs with narrower CTAs
     if (N <= (int64_t)kNumSMs * 32 * 2) return 32;
@@ -889,6 +942,11 @@ extern "C" int xb_env_reset(int env_kind, double* state, uint64_t* rng, int32_t*
         env_reset_kernel<Acrobot><<<grid, block, 0, s>>>(state, rng, elapsed, ep_score, (float4*)obs, n_draws, N);
     else if (env_kind == XB_ENV_MOUNTAINCAR_STACK4)
         env_reset_kernel<MountainCarStack><<<grid, block, 0, s>>>(state, rng, elapsed, ep_score, (float4*)obs, n_draws, N);
+    else if (env_kind == XB_ENV_MOUNTAINCAR_CONTINUOUS)
+        env_reset_kernel<MountainCarContinuous><<<grid, block, 0, s>>>(state, rng, elapsed, ep_score, (float4*)obs, n_draws, N);
+    else if (env_kind == XB_ENV_MOUNTAINCAR_CONTINUOUS_STACK4)
+        env_reset_kernel<MountainCarContinuousStack><<<grid, block, 0, s>>>(state, rng, elapsed, ep_score, (float4*)obs,
+                                                                            n_draws, N);
     else
         return XB_E_UNSUPPORTED;
     XB_LAUNCH_CHECK();
@@ -929,6 +987,16 @@ extern "C" int xb_env_step(int env_kind, double* state, uint64_t* rng, int32_t* 
                                                                  (float4*)obs, (float4*)next_obs, rew, term, trunc,
                                                                  (float4*)reset_obs, ep_step_out, ep_score_out, ep_stats,
                                                                  max_episode_steps, N);
+    else if (env_kind == XB_ENV_MOUNTAINCAR_CONTINUOUS)
+        env_step_kernel<MountainCarContinuous><<<grid, block, 0, s>>>(state, rng, elapsed, ep_score, (const float*)actions,
+                                                                      (float4*)obs, (float4*)next_obs, rew, term, trunc,
+                                                                      (float4*)reset_obs, ep_step_out, ep_score_out, ep_stats,
+                                                                      max_episode_steps, N);
+    else if (env_kind == XB_ENV_MOUNTAINCAR_CONTINUOUS_STACK4)
+        env_step_kernel<MountainCarContinuousStack><<<grid, block, 0, s>>>(state, rng, elapsed, ep_score, (const float*)actions,
+                                                                           (float4*)obs, (float4*)next_obs, rew, term, trunc,
+                                                                           (float4*)reset_obs, ep_step_out, ep_score_out,
+                                                                           ep_stats, max_episode_steps, N);
     else
         return XB_E_UNSUPPORTED;
     XB_LAUNCH_CHECK();
@@ -957,7 +1025,7 @@ extern "C" int xb_rollout_step(int env_kind, const float* act_param, const float
         !reset_obs || !ep_step_out || !ep_score_out || !x_in || !act_out || !logp_out || !obs_row || !act_row ||
         !rew_row || !val_row || !term_row || !logp_row)
         return XB_E_BADARG;
-    if (env_kind == XB_ENV_PENDULUM && !logstd) return XB_E_BADARG;
+    if (continuous_kind(env_kind) && !logstd) return XB_E_BADARG;
     if ((boot_row != nullptr) != (boot_src != nullptr)) return XB_E_BADARG;
     RolloutStepArgs a{act_param, logstd, val, seed, counter_dev, offset, state, rng, elapsed, ep_score, (float4*)obs,
                       (float4*)next_obs, rew, term, trunc, (float4*)reset_obs, ep_step_out, ep_score_out, ep_stats,
@@ -984,6 +1052,10 @@ extern "C" int xb_rollout_step(int env_kind, const float* act_param, const float
     else if (env_kind == XB_ENV_MOUNTAINCAR) XB_CUDA(launch_pdl(rollout_step_kernel<MountainCar>, dim3(grid), dim3(block), 0, s, true, a));
     else if (env_kind == XB_ENV_ACROBOT) XB_CUDA(launch_pdl(rollout_step_kernel<Acrobot>, dim3(grid), dim3(block), 0, s, true, a));
     else if (env_kind == XB_ENV_MOUNTAINCAR_STACK4) XB_CUDA(launch_pdl(rollout_step_kernel<MountainCarStack>, dim3(grid), dim3(block), 0, s, true, a));
+    else if (env_kind == XB_ENV_MOUNTAINCAR_CONTINUOUS)
+        XB_CUDA(launch_pdl(rollout_step_kernel<MountainCarContinuous>, dim3(grid), dim3(block), 0, s, true, a));
+    else if (env_kind == XB_ENV_MOUNTAINCAR_CONTINUOUS_STACK4)
+        XB_CUDA(launch_pdl(rollout_step_kernel<MountainCarContinuousStack>, dim3(grid), dim3(block), 0, s, true, a));
     else return XB_E_UNSUPPORTED;
     XB_LAUNCH_CHECK();
     return 0;
@@ -998,7 +1070,7 @@ extern "C" int xb_eval_step(int env_kind, const float* act_param, const float* l
     if (N <= 0 || !act_param || !key || !step || !state || !rng || !elapsed || !ep_score || !next_obs || !scores || !count ||
         !test_episode || cap < 1 || !partials || !workspace || tape_steps < 0 || (act_tape && tape_steps == 0))
         return XB_E_BADARG;
-    if (env_kind == XB_ENV_PENDULUM && !logstd) return XB_E_BADARG;
+    if (continuous_kind(env_kind) && !logstd) return XB_E_BADARG;
     if ((local_count != nullptr) != (score_step != nullptr) || (local_count != nullptr) != (record != nullptr)) return XB_E_BADARG;
     if (obs_state && (obs_dim < 1 || obs_dim > 8)) return XB_E_BADARG;
     if (obs_state && !record && (!obs_state_cand || obs_state == obs_state_cand)) return XB_E_BADARG;     // the merge's scratch
@@ -1018,6 +1090,8 @@ extern "C" int xb_eval_step(int env_kind, const float* act_param, const float* l
     else if (env_kind == XB_ENV_MOUNTAINCAR) eval_step_kernel<MountainCar><<<grid, block, 0, s>>>(a);
     else if (env_kind == XB_ENV_ACROBOT) eval_step_kernel<Acrobot><<<grid, block, 0, s>>>(a);
     else if (env_kind == XB_ENV_MOUNTAINCAR_STACK4) eval_step_kernel<MountainCarStack><<<grid, block, 0, s>>>(a);
+    else if (env_kind == XB_ENV_MOUNTAINCAR_CONTINUOUS) eval_step_kernel<MountainCarContinuous><<<grid, block, 0, s>>>(a);
+    else if (env_kind == XB_ENV_MOUNTAINCAR_CONTINUOUS_STACK4) eval_step_kernel<MountainCarContinuousStack><<<grid, block, 0, s>>>(a);
     else return XB_E_UNSUPPORTED;
     XB_LAUNCH_CHECK();
     return 0;

@@ -7,7 +7,10 @@ import torch
 
 from . import _lib
 
-ENV_KINDS = {"CartPole-v1": 0, "Pendulum-v1": 1, "gym:MountainCar-v0": 2, "Acrobot-v1": 3, "MountainCar-v0": 4}
+ENV_KINDS = {"CartPole-v1": 0, "CartPole-v0": 0, "Pendulum-v1": 1, "gym:MountainCar-v0": 2, "Acrobot-v1": 3, "MountainCar-v0": 4,
+             "gym:MountainCarContinuous-v0": 5, "MountainCarContinuous-v0": 6}
+# env kinds with a Box action: float32 actions [N] in and out of the env kernels; every other kind takes int64 actions
+CONTINUOUS_KINDS = frozenset({1, 5, 6})
 GAE_VARIANTS = {"auto": 0, "ldg": 1, "tma": 2}
 
 
@@ -23,11 +26,20 @@ def _p(t, dtype=None):
     return t.data_ptr()
 
 
+def continuous_kind(kind):
+    """True for the env kinds whose action is one float32 per env (include/xb200.h XB_ENV_*)."""
+    return kind in CONTINUOUS_KINDS
+
+
 def _stream():
     return torch.cuda.current_stream().cuda_stream
 
 
 F32, F64, I64, I32, U8 = torch.float32, torch.float64, torch.int64, torch.int32, torch.uint8
+
+
+def _act_dtype(kind):
+    return F32 if continuous_kind(kind) else I64
 
 
 def env_reset(kind, state, rng, elapsed, ep_score, obs, n_draws):
@@ -40,7 +52,7 @@ def env_step(kind, state, rng, elapsed, ep_score, actions, obs, next_obs, rew, t
              ep_score_out, max_steps, ep_stats=None):
     N = elapsed.numel()
     _lib.call("xb_env_step", kind, _p(state, F64), _p(rng, I64), _p(elapsed, I32), _p(ep_score, F64),
-              _p(actions, F32 if kind == 1 else I64), _p(obs, F32), _p(next_obs, F32), _p(rew, F32), _p(term, U8),
+              _p(actions, _act_dtype(kind)), _p(obs, F32), _p(next_obs, F32), _p(rew, F32), _p(term, U8),
               _p(trunc, U8), _p(reset_obs, F32), _p(ep_step_out, I32), _p(ep_score_out, F64), _p(ep_stats, F64), max_steps,
               N, _stream())
 
@@ -58,7 +70,7 @@ def rollout_step(kind, act_param, logstd, val, seed, counter, offset, state, rng
     _lib.call("xb_rollout_step", kind, _p(act_param, F32), _p(logstd, F32), _p(val, F32), int(seed), _p(counter, I64),
               int(offset), _p(state, F64), _p(rng, I64), _p(elapsed, I32), _p(ep_score, F64), _p(obs, F32),
               _p(next_obs, F32), _p(rew, F32), _p(term, U8), _p(trunc, U8), _p(reset_obs, F32), _p(ep_step_out, I32),
-              _p(ep_score_out, F64), _p(ep_stats, F64), max_steps, _p(x_in, F32), _p(act_out, F32 if kind == 1 else I64),
+              _p(ep_score_out, F64), _p(ep_stats, F64), max_steps, _p(x_in, F32), _p(act_out, _act_dtype(kind)),
               _p(logp_out, F32), _p(obs_row, F32), _p(act_row, F32), _p(rew_row, F32), _p(val_row, F32),
               _p(term_row, F32), _p(trunc_row, U8), _p(logp_row, F32), _p(rew_std, F32), float(rew_clip), _p(boot_src, F32),
               _p(boot_row, F32), _p(trig_cache, F64), _p(st.get("obs_in"), F64), _p(st.get("obs_out"), F64),
@@ -78,7 +90,7 @@ def eval_step(kind, act_param, logstd, key, step, state, rng, elapsed, ep_score,
         raise _lib.XB200Error("score_step needs one entry per queue slot (%d < %d)" % (score_step.numel(), scores.numel()))
     _lib.call("xb_eval_step", kind, _p(act_param, F32), _p(logstd, F32), _p(key, I64), _p(step, I64), _p(state, F64),
               _p(rng, I64), _p(elapsed, I32), _p(ep_score, F64), _p(next_obs, F32), _p(trig_cache, F64), max_steps,
-              _p(act_tape, F32 if kind == 1 else I64), act_tape.shape[0] if act_tape is not None else 0, _p(scores, F64),
+              _p(act_tape, _act_dtype(kind)), act_tape.shape[0] if act_tape is not None else 0, _p(scores, F64),
               _p(count, I64), _p(test_episode, I64), scores.numel(), _p(obs_state, F64), _p(obs_state_cand, F64), int(obs_dim),
               _p(partials, F64), _p(workspace, I64), _p(local_count, I64), _p(score_step, I32), _p(record, F64), N, _stream())
 

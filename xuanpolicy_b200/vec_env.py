@@ -28,6 +28,11 @@ SPECS = {
     "MountainCar-v0": dict(kind=4, state_dim=8, obs_dim=8, max_steps=200),
     "gym:MountainCar-v0": dict(kind=2, state_dim=2, obs_dim=2, max_steps=200),
     "Acrobot-v1": dict(kind=3, state_dim=4, obs_dim=6, max_steps=500),
+    # CartPole with gym's v0 registration: the same env, TimeLimit 200
+    "CartPole-v0": dict(kind=0, state_dim=4, obs_dim=4, max_steps=200),
+    # the 4-frame rule of make_envs holds for every id containing "MountainCar": the continuous env too
+    "MountainCarContinuous-v0": dict(kind=6, state_dim=8, obs_dim=8, max_steps=999),
+    "gym:MountainCarContinuous-v0": dict(kind=5, state_dim=2, obs_dim=2, max_steps=999),
 }
 
 
@@ -42,7 +47,7 @@ class NotSteppingError(Exception):
 
 
 def make_spaces(env_id):
-    if env_id == "CartPole-v1":
+    if env_id in ("CartPole-v1", "CartPole-v0"):
         high = np.array([4.8, np.finfo(np.float32).max, 24 * np.pi / 360 * 2, np.finfo(np.float32).max], np.float32)
         return Box(-high, high), Discrete(2)
     if env_id == "Pendulum-v1":
@@ -55,8 +60,18 @@ def make_spaces(env_id):
     if env_id == "Acrobot-v1":
         high = np.array([1.0, 1.0, 1.0, 1.0, 4 * np.pi, 9 * np.pi], np.float32)
         return Box(-high, high), Discrete(3)
-    raise NotImplementedError("only CartPole-v1, Pendulum-v1, MountainCar-v0 and Acrobot-v1 have device kernels (got %r)"
-                              % (env_id,))
+    if env_id == "MountainCarContinuous-v0":     # the 4-frame stack of gym_env.py:50-83 over gym's continuous env
+        return (Box(np.array([-1.2, -0.07] * 4, np.float32), np.array([0.6, 0.07] * 4, np.float32)),
+                Box(-1.0, 1.0, shape=(1,)))
+    if env_id == "gym:MountainCarContinuous-v0":
+        return Box(np.array([-1.2, -0.07], np.float32), np.array([0.6, 0.07], np.float32)), Box(-1.0, 1.0, shape=(1,))
+    raise NotImplementedError("only CartPole-v1, CartPole-v0, Pendulum-v1, MountainCar-v0, MountainCarContinuous-v0 and "
+                              "Acrobot-v1 have device kernels (got %r)" % (env_id,))
+
+
+def continuous_actions(env_id):
+    """True when the env's action is a Box (one float32 per env), False for Discrete; KeyError for an unknown id."""
+    return ops.continuous_kind(SPECS[env_id]["kind"])
 
 
 class EnvFn:
@@ -153,7 +168,7 @@ class DummyVecEnv_Gym:
             self._ep_step_out = torch.zeros(N, dtype=torch.int32, device=dev)
             self._ep_score_out = torch.zeros(N, dtype=torch.float64, device=dev)
             self.ep_stats = torch.zeros(3, dtype=torch.float64, device=dev)  # finished episodes, sum score, sum length
-            act_dtype = torch.float32 if self._kind == 1 else torch.int64
+            act_dtype = torch.float32 if ops.continuous_kind(self._kind) else torch.int64
             self._act = torch.zeros(N, dtype=act_dtype, device=dev)
             ops.env_reset(self._kind, self._state, self._rng, self._elapsed, self._ep_score, self._obs, 1)
         self.buf_obs = np.zeros((N,) + self.obs_shape, dtype=np.float32)
@@ -172,7 +187,8 @@ class DummyVecEnv_Gym:
         return self._obs[:, :self._obs_dim]
 
     def step_device(self, actions):
-        """One vector step on the current stream, entirely on device (graph-capturable)."""
+        """One vector step on the current stream, entirely on device (graph-capturable).  `actions`: int64 [N], or float32
+        [N] for a Box action."""
         ops.env_step(self._kind, self._state, self._rng, self._elapsed, self._ep_score, actions, self._obs,
                      self._next_obs, self._rew, self._term, self._trunc, self._reset_obs, self._ep_step_out,
                      self._ep_score_out, self.max_episode_length, ep_stats=self.ep_stats)
